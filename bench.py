@@ -13,6 +13,11 @@ the multiplier read-back with the reference's masking, the violation norm and th
 The job is fixed (``--scenarios``, default 1024 = BASELINE config 5) and split over the GPUs: strong scaling.  At
 N = 1 the line also carries BASELINE's single-instance figures (sub-LP ms and SLP iterations/s on case13659pegase)
 under ``single_instance``.  One JSON line is printed by rank 0.
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes what the last timed step returned as ``DIR/<name>.npy`` (float64, at most 64 MB): the inputs depend
+only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +35,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 METRIC = "sub-LP scenarios/s (SLP hot path: assembly + bounds + LP solve to 1e-6 objective accuracy + read-back + merit)"
 UNIT = "scenarios/s"
@@ -57,7 +63,30 @@ def parse_args():
     ap.add_argument("--workload", default="batch", choices=["batch", "single"],
                     help="batch: scenario batch per GPU (default, the driver's metric); single: one instance "
                          "(BASELINE config 4) -- group engine at N = 1, row-partitioned over NCCL at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0's "
+                         "scenarios; full vectors for a fixed, seeded sample of them)")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 * 10**6
+
+
+def dump_sample(n_scen, row_bytes, budget=32 << 20, cap=64):
+    """Indices of a fixed, seeded sample of scenarios whose full output vectors together fit `budget` bytes."""
+    k = max(1, min(n_scen, cap, budget // max(1, row_bytes)))
+    return np.sort(np.random.default_rng(0).choice(n_scen, k, replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as out_dir/<name>.npy in float64 (integers and statuses are exact in it)."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -191,6 +220,11 @@ def run_reference(a):
             dt, res = step(a.warmup + k)
             t_total += dt
             n_ok += sum(1 for r in res if r[1] == 0)
+    if a.dump_outputs:
+        last = a.warmup + a.steps - 1
+        dump_outputs(a.dump_outputs, dict(
+            scenario_id=[1 + last * per_step + s for s in range(per_step)], status=[r[1] for r in res],
+            objective=[np.nan if r[2] is None else r[2] for r in res]))
     value = per_step * a.steps / t_total
     sample = (f"{per_step} scenarios of {a.case} per step over a {cores}-process pool (one HiGHS dual simplex per "
               f"core), host NLP evaluation included in the step")
@@ -385,6 +419,17 @@ def run_ours(a):
     infos = [dict(status=int(i.status), iterations=int(i.iterations), objective=float(i.objective),
                   pres=float(i.primal_residual), dres=float(i.dual_residual), gap=float(i.gap)) for i in info[:S]]
     loop_ms, loop_its = lp.last_solve_timing()
+    dumped = None
+    if a.dump_outputs and rank == 0:
+        # the last resident step left its results on the device: read them back outside the timed region; copies,
+        # because the end-to-end steps below reuse the host buffers
+        capi.check(lib.asm_slp_extract(lp._h, P(hout["p"]), P(hout["lam"]), P(hout["mu_u"]), P(hout["mu_l"]),
+                                       P(hout["slack"]), hstatus.ctypes.data_as(capi.c_int32_p)))
+        rows = dump_sample(S, 8 * (3 * n + 3 * m))
+        dumped = {"scenario_id": np.array(ids), "status": hstatus.copy(), "objective": [i["objective"] for i in infos],
+                  "violation": hout["viol"].copy(), "sample_scenario_id": np.array(ids)[rows], "p": hout["p"][rows],
+                  "lambda": hout["lam"][rows], "mult_x_U": hout["mu_u"][rows], "mult_x_L": hout["mu_l"][rows],
+                  "p_slack": hout["slack"][rows]}
     dev_s = max_over_ranks(dev_ms * 1e-3)
     # ---- timed, end to end through the C ABI with pinned host buffers (same number of steps)
     sync_all()
@@ -492,6 +537,8 @@ def run_ours(a):
             out["cpu_baseline"] = cpu
         if single is not None:
             out["single_instance"] = single
+        if dumped is not None:
+            dump_outputs(a.dump_outputs, dumped)
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -524,7 +571,9 @@ def run_single(a):
         def step():
             t0 = time.perf_counter()
             out = lp.sub_optimize(*args)
-            return time.perf_counter() - t0, lp.last_info[0], lp.last_solve_timing()
+            dt = time.perf_counter() - t0
+            res = dict(zip(("p", "lambda", "mult_x_U", "mult_x_L", "p_slack", "status"), out))
+            return dt, lp.last_info[0], lp.last_solve_timing(), res
     else:
         rp, ci, vals = lp.jacobian_csr()                       # device-assembled CSR of this linearisation
         x = d["x"][0]
@@ -546,16 +595,16 @@ def run_single(a):
             plp.set_col_bounds(lb, ub)
             plp.set_row_bounds(rl, ru)
             info = plp.optimize()[0]
-            plp.primal()
-            plp.row_dual()
-            return time.perf_counter() - t0, info, (0.0, info["iterations"])
+            primal = plp.primal()
+            row_dual = plp.row_dual()
+            return time.perf_counter() - t0, info, (0.0, info["iterations"]), {"primal": primal, "row_dual": row_dual}
     for _ in range(a.warmup):
         step()
     clocks = ClockSampler(local)
     clocks.start()
     tot, info, timing = 0.0, None, None
     for _ in range(a.steps):
-        dt, info, timing = step()
+        dt, info, timing, res = step()
         tot += dt
     clk = clocks.stop()
     tot = shard.max_over_ranks(tot)
@@ -574,6 +623,8 @@ def run_single(a):
                "e2e": {"value": a.steps / tot, "unit": "sub-LP/s", "h2d_bytes_per_step": 8 * (2 * n + m + nnz + 2),
                        "d2h_bytes_per_step": 8 * (3 * n + 3 * m)},
                "clocks": clk}
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {"status": info["status"], "objective": info["objective"], **res})
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.barrier()
