@@ -1634,8 +1634,8 @@ int asm_slp_ipm_timing(asm_slp *h, int32_t reps, double *factor_ms, double *solv
 // Host-only self test of the barrier engine's symbolic analysis (no device needed): orders and analyses the KKT
 // pattern of the m x n CSR matrix K, then factorises  [-diag(dx) K'; K diag(ew)]  and solves one right-hand side ON
 // THE HOST with exactly the lists and the summation order the device kernels use.  rhs_sol: n + m values, right-hand
-// side in (columns then rows), solution out.  stats[8]: nnz(L), terms, levels, factor launches, forward launches,
-// backward launches, longest chunk, chunks.
+// side in (columns then rows), solution out.  stats[8]: nnz(L), terms, levels, steps with fan-out items in the
+// factorisation / forward / backward substitution (the step-kernel launches of each), longest chunk, chunks.
 int asm_kkt_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, const int32_t *col_idx, const double *vals,
                      const double *dx, const double *ew, double *rhs_sol, int64_t *stats) {
     if (!row_ptr || n_cols <= 0 || n_rows < 0 || !dx || !rhs_sol) return fail(ASM_E_INVALID, "bad argument");
@@ -1645,8 +1645,8 @@ int asm_kkt_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, con
     for (int i = 0; i <= n_rows; ++i) rp[i] = (int)row_ptr[i];
     for (int64_t k = 0; k < nnz; ++k) ci[k] = col_idx[k];
     KktSymbolic S;
-    // supernodes as a batch handle would use them (ASM_IPM_SUPERNODE=1 turns them off)
-    if (S.build(n_cols, n_rows, rp.data(), ci.data(), 64, IpmEngine::supernode_for(32))) return fail(ASM_E_INVALID, "symbolic analysis failed");
+    // supernodes as a handle would use them (ASM_IPM_SUPERNODE=1 turns them off)
+    if (S.build(n_cols, n_rows, rp.data(), ci.data(), kkt_supernode_width())) return fail(ASM_E_INVALID, "symbolic analysis failed");
     std::vector<double> W(S.nnzL, 0.0), d0(S.N), invd;
     for (int64_t q = 0; q < nnz; ++q) W[S.kmap[q]] = vals[q];
     for (int j = 0; j < n_cols; ++j) d0[S.inv[j]] = -dx[j];
@@ -1660,9 +1660,14 @@ int asm_kkt_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, con
         stats[0] = S.nnzL;
         stats[1] = S.nterms;
         stats[2] = S.n_levels;
-        stats[3] = (int64_t)S.flaunch.size();
-        stats[4] = (int64_t)S.wlaunch.size();
-        stats[5] = (int64_t)S.blaunch.size();
+        auto fanout_steps = [&](const std::vector<int> &sb, const std::vector<int> &se, const std::vector<int> &ms) {
+            int64_t c = 0;
+            for (int l = 0; l < S.n_levels; ++l) c += se[l] > sb[l] || ms[l + 1] > ms[l];
+            return c;
+        };
+        stats[3] = fanout_steps(S.fs_beg, S.fs_end, S.fmstep);
+        stats[4] = fanout_steps(S.ws_beg, S.ws_end, S.wmstep);
+        stats[5] = fanout_steps(S.bs_beg, S.bs_end, S.bmstep);
         stats[6] = longest;
         stats[7] = S.n_fchunks;
     }

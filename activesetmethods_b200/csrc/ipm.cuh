@@ -62,20 +62,17 @@ struct IpmState {
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
+// the ranges of the launched step come as arguments, not from the step tables: one dependent load less on the critical path
 struct KktStepRange {
-    int s0, s1, m0, m1;   // single-term items [s0, s1), multi-term chunks [m0, m1) of a one-step launch
+    int s0, s1, m0, m1;   // single-term items [s0, s1), multi-term chunks [m0, m1)
 };
-constexpr int kFusedThreads = 1024;   // block size of the fused walks over runs of narrow steps
 
 struct KktDev {
     const KktTerm *terms;
-    const int *fs_beg, *fs_end, *fmstep;
     const KktRange *fmchunk;
     const KktFwdItem *fwd;
-    const int *ws_beg, *ws_end, *wmstep;
     const KktRange *wmchunk;
     const KktBwdItem *bwd;
-    const int *bs_beg, *bs_end, *bmstep;
     const KktRange *bmchunk;
     const KktPanel *panels;
     const KktPanelTask *ptasks;
@@ -111,9 +108,7 @@ __device__ __forceinline__ double ipm_slack(double d) { return fmax(d, 1e-30); }
 // (the kernel is bound by the latency of its dependent loads -- index, then operands -- not by bandwidth: ncu shows
 // 40 long-scoreboard stall cycles per issue without the pipelining).  BATCH: a warp owns a chunk and its lanes are 32
 // scenarios (index loads warp-uniform, value loads coalesced); single LP: a thread owns a chunk.  Exactly one thread
-// writes a target in a step and the terms of a chunk are added in ascending k: bit-reproducible.  FUSED: gridDim.x == 1
-// and the block walks the steps [l0, l1) with a barrier in between (W, invd and diag0 are read and written by the
-// same kernel: plain loads, no read-only path).
+// writes a target in a step and the terms of a chunk are added in ascending k: bit-reproducible.  One launch per step.
 __device__ __forceinline__ void ldl_apply(const KktDev &d, int tflag, double acc, int B, int s) {
     const int t = tflag & ~kLastBit;
     if (t >= d.nnzL) {
@@ -183,142 +178,128 @@ __device__ __forceinline__ double chunk_sum_vec(const KktDev &d, const Item *ite
     }
     return acc;
 }
-template <bool BATCH, bool FUSED>
-__global__ void __launch_bounds__(FUSED ? kFusedThreads : kThreads, FUSED ? 1 : 4) k_ldl_factor(KktDev d, int B, int l0, int l1, const ScenState *st, KktStepRange rg) {
+template <bool BATCH>
+__global__ void __launch_bounds__(kThreads, 4) k_ldl_factor(KktDev d, int B, const ScenState *st, KktStepRange rg) {
     pdl_trigger();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int s = BATCH ? blockIdx.y * 32 + lane : 0;
     const bool live = st[s].status < 0;
-    const int bw = blockDim.x >> 5;   // 8 warps per block for one-step launches, 32 for the fused walks
-    const int first = BATCH ? blockIdx.x * bw + warp : blockIdx.x * blockDim.x + threadIdx.x;
-    const int stride = BATCH ? gridDim.x * bw : gridDim.x * blockDim.x;
-    for (int l = l0; l < l1; ++l) {
-        {   // loads are never gated on the scenario's status (it would put one more dependent load on the critical path); stores are
-            // one-step launches get their ranges as arguments (one dependent load less on the critical path)
-            const int q0 = FUSED ? d.fs_beg[l] : rg.s0, q1 = FUSED ? d.fs_end[l] : rg.s1;
-            if (BATCH) {
-                if (l == l0) pdl_wait();
-                for (int q = q0 + 4 * first; q < q1; q += 4 * stride) {
-                    KktTerm u[4];
-                    double a[4], b[4], c[4];
+    const int first = BATCH ? blockIdx.x * kWarps + warp : blockIdx.x * blockDim.x + threadIdx.x;
+    const int stride = BATCH ? gridDim.x * kWarps : gridDim.x * blockDim.x;
+    // loads are never gated on the scenario's status (it would put one more dependent load on the critical path); stores are
+    const int q0 = rg.s0, q1 = rg.s1;
+    pdl_wait();
+    if (BATCH) {
+        for (int q = q0 + 4 * first; q < q1; q += 4 * stride) {
+            KktTerm u[4];
+            double a[4], b[4], c[4];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) u[i] = d.terms[q + i < q1 ? q + i : q];
+            for (int i = 0; i < 4; ++i) u[i] = d.terms[q + i < q1 ? q + i : q];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        a[i] = d.W[(int64_t)u[i].a * B + s];
-                        b[i] = d.W[(int64_t)u[i].b * B + s];
-                        c[i] = d.invd[(int64_t)u[i].k * B + s];
-                    }
-                    double tv[4];
-                    int64_t te[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int t = u[i].t & ~kLastBit;
-                        const bool piv = t >= d.nnzL;
-                        te[i] = (int64_t)(piv ? t - d.nnzL : t) * B + s;
-                        tv[i] = piv ? d.diag0[te[i]] : d.W[te[i]];
-                    }
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        if (q + i >= q1 || !live) break;
-                        const double r = tv[i] - a[i] * b[i] * c[i];
-                        if ((u[i].t & ~kLastBit) >= d.nnzL) {
-                            d.diag0[te[i]] = r;
-                            if (u[i].t & kLastBit) d.invd[te[i]] = 1.0 / r;
-                        } else {
-                            d.W[te[i]] = r;
-                        }
-                    }
-                }
-            } else {
-                if (l == l0) pdl_wait();
-                for (int q = q0 + first; q < q1; q += stride) {
-                    const KktTerm u = d.terms[q];
-                    if (live) ldl_apply(d, u.t, d.W[u.a] * d.W[u.b] * d.invd[u.k], 1, 0);
-                }
+            for (int i = 0; i < 4; ++i) {
+                a[i] = d.W[(int64_t)u[i].a * B + s];
+                b[i] = d.W[(int64_t)u[i].b * B + s];
+                c[i] = d.invd[(int64_t)u[i].k * B + s];
             }
-            const int c0 = FUSED ? d.fmstep[l] : rg.m0, c1 = FUSED ? d.fmstep[l + 1] : rg.m1;
-            for (int c = c0 + first; c < c1; c += stride) {
-                const KktRange r = d.fmchunk[c];
-                int tflag;
-                double tv;
-                const double acc = chunk_sum(d, r.begin, r.end, B, s, tflag, tv);
-                if (live) {
-                    const int t = tflag & ~kLastBit;
-                    const double r2 = tv - acc;
-                    if (t >= d.nnzL) {
-                        const int64_t e = (int64_t)(t - d.nnzL) * B + s;
-                        d.diag0[e] = r2;
-                        if (tflag & kLastBit) d.invd[e] = 1.0 / r2;
-                    } else {
-                        d.W[(int64_t)t * B + s] = r2;
-                    }
+            double tv[4];
+            int64_t te[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const int t = u[i].t & ~kLastBit;
+                const bool piv = t >= d.nnzL;
+                te[i] = (int64_t)(piv ? t - d.nnzL : t) * B + s;
+                tv[i] = piv ? d.diag0[te[i]] : d.W[te[i]];
+            }
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                if (q + i >= q1 || !live) break;
+                const double r = tv[i] - a[i] * b[i] * c[i];
+                if ((u[i].t & ~kLastBit) >= d.nnzL) {
+                    d.diag0[te[i]] = r;
+                    if (u[i].t & kLastBit) d.invd[te[i]] = 1.0 / r;
+                } else {
+                    d.W[te[i]] = r;
                 }
             }
         }
-        if (FUSED) __syncthreads();
+    } else {
+        for (int q = q0 + first; q < q1; q += stride) {
+            const KktTerm u = d.terms[q];
+            if (live) ldl_apply(d, u.t, d.W[u.a] * d.W[u.b] * d.invd[u.k], 1, 0);
+        }
+    }
+    for (int c = rg.m0 + first; c < rg.m1; c += stride) {
+        const KktRange r = d.fmchunk[c];
+        int tflag;
+        double tv;
+        const double acc = chunk_sum(d, r.begin, r.end, B, s, tflag, tv);
+        if (live) {
+            const int t = tflag & ~kLastBit;
+            const double r2 = tv - acc;
+            if (t >= d.nnzL) {
+                const int64_t e = (int64_t)(t - d.nnzL) * B + s;
+                d.diag0[e] = r2;
+                if (tflag & kLastBit) d.invd[e] = 1.0 / r2;
+            } else {
+                d.W[(int64_t)t * B + s] = r2;
+            }
+        }
     }
 }
 
 // forward substitution  v <- L^-1 v  (fan-out, laid out like the factorisation; v indexed by node id, in place)
-template <bool BATCH, bool FUSED>
-__global__ void __launch_bounds__(FUSED ? kFusedThreads : kThreads, FUSED ? 1 : 4) k_ldl_fwd(KktDev d, double *v, int B, int l0, int l1, const ScenState *st, KktStepRange rg) {
+template <bool BATCH>
+__global__ void __launch_bounds__(kThreads, 4) k_ldl_fwd(KktDev d, double *v, int B, const ScenState *st, KktStepRange rg) {
     pdl_trigger();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int s = BATCH ? blockIdx.y * 32 + lane : 0;
     const bool live = st[s].status < 0;
-    const int bw = blockDim.x >> 5;   // 8 warps per block for one-step launches, 32 for the fused walks
-    const int first = BATCH ? blockIdx.x * bw + warp : blockIdx.x * blockDim.x + threadIdx.x;
-    const int stride = BATCH ? gridDim.x * bw : gridDim.x * blockDim.x;
-    for (int l = l0; l < l1; ++l) {
-        {   // loads are never gated on the scenario's status (it would put one more dependent load on the critical path); stores are
-            const int q0 = FUSED ? d.ws_beg[l] : rg.s0, q1 = FUSED ? d.ws_end[l] : rg.s1;
-            if (BATCH) {
-                int q = q0 + 4 * first;
-                KktFwdItem u[4];
-                if (q < q1) {
+    const int first = BATCH ? blockIdx.x * kWarps + warp : blockIdx.x * blockDim.x + threadIdx.x;
+    const int stride = BATCH ? gridDim.x * kWarps : gridDim.x * blockDim.x;
+    // loads are never gated on the scenario's status (it would put one more dependent load on the critical path); stores are
+    const int q0 = rg.s0, q1 = rg.s1;
+    if (BATCH) {
+        int q = q0 + 4 * first;
+        KktFwdItem u[4];
+        if (q < q1) {
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) u[i] = d.fwd[q + i < q1 ? q + i : q];
-                }
-                if (l == l0) pdl_wait();
-                while (q < q1) {
-                    double a[4], x[4], c[4], t[4];
-                    int dst[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        a[i] = d.W[(int64_t)u[i].pos * B + s];
-                        x[i] = v[(int64_t)u[i].src * B + s];
-                        c[i] = d.invd[(int64_t)u[i].k * B + s];
-                        t[i] = v[(int64_t)u[i].dst * B + s];
-                        dst[i] = u[i].dst;
-                    }
-                    const int qn = q + 4 * stride;
-                    if (qn < q1) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) u[i] = d.fwd[qn + i < q1 ? qn + i : qn];
-                    }
-#pragma unroll
-                    for (int i = 0; i < 4; ++i)
-                        if (q + i < q1 && live) v[(int64_t)dst[i] * B + s] = t[i] - a[i] * x[i] * c[i];
-                    q = qn;
-                }
-            } else {
-                if (l == l0) pdl_wait();
-                for (int q = q0 + first; q < q1; q += stride) {
-                    const KktFwdItem u = d.fwd[q];
-                    if (live) v[u.dst] -= d.W[u.pos] * v[u.src] * d.invd[u.k];
-                }
-            }
-            const int c0 = FUSED ? d.wmstep[l] : rg.m0, c1 = FUSED ? d.wmstep[l + 1] : rg.m1;
-            for (int c = c0 + first; c < c1; c += stride) {
-                const KktRange r = d.wmchunk[c];
-                int dst;
-                double tv;
-                const double acc = chunk_sum_vec(d, d.fwd, v, r.begin, r.end, B, s, dst, tv);
-                if (live) v[(int64_t)dst * B + s] = tv - acc;
-            }
+            for (int i = 0; i < 4; ++i) u[i] = d.fwd[q + i < q1 ? q + i : q];
         }
-        if (FUSED) __syncthreads();
+        pdl_wait();
+        while (q < q1) {
+            double a[4], x[4], c[4], t[4];
+            int dst[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                a[i] = d.W[(int64_t)u[i].pos * B + s];
+                x[i] = v[(int64_t)u[i].src * B + s];
+                c[i] = d.invd[(int64_t)u[i].k * B + s];
+                t[i] = v[(int64_t)u[i].dst * B + s];
+                dst[i] = u[i].dst;
+            }
+            const int qn = q + 4 * stride;
+            if (qn < q1) {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) u[i] = d.fwd[qn + i < q1 ? qn + i : qn];
+            }
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+                if (q + i < q1 && live) v[(int64_t)dst[i] * B + s] = t[i] - a[i] * x[i] * c[i];
+            q = qn;
+        }
+    } else {
+        pdl_wait();
+        for (int q = q0 + first; q < q1; q += stride) {
+            const KktFwdItem u = d.fwd[q];
+            if (live) v[u.dst] -= d.W[u.pos] * v[u.src] * d.invd[u.k];
+        }
+    }
+    for (int c = rg.m0 + first; c < rg.m1; c += stride) {
+        const KktRange r = d.wmchunk[c];
+        int dst;
+        double tv;
+        const double acc = chunk_sum_vec(d, d.fwd, v, r.begin, r.end, B, s, dst, tv);
+        if (live) v[(int64_t)dst * B + s] = tv - acc;
     }
 }
 // v <- D^-1 v
@@ -330,65 +311,59 @@ __global__ void __launch_bounds__(kThreads) k_ldl_diag(KktDev d, double *v, int 
 }
 // backward substitution  v <- L'^-1 v : the rows of a column are its ancestors in the elimination tree; without
 // supernodes they sit on distinct levels and every item of a step has its own target, with supernodes a column can have
-// several rows in one step (a chunk).  Steps are walked downwards
-template <bool BATCH, bool FUSED>
-__global__ void __launch_bounds__(FUSED ? kFusedThreads : kThreads, FUSED ? 1 : 4) k_ldl_bwd(KktDev d, double *v, int B, int l0, int l1, const ScenState *st, KktStepRange rg) {
+// several rows in one step (a chunk).  Steps are launched downwards
+template <bool BATCH>
+__global__ void __launch_bounds__(kThreads, 4) k_ldl_bwd(KktDev d, double *v, int B, const ScenState *st, KktStepRange rg) {
     pdl_trigger();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int s = BATCH ? blockIdx.y * 32 + lane : 0;
     const bool live = st[s].status < 0;
-    const int bw = blockDim.x >> 5;   // 8 warps per block for one-step launches, 32 for the fused walks
-    const int first = BATCH ? blockIdx.x * bw + warp : blockIdx.x * blockDim.x + threadIdx.x;
-    const int stride = BATCH ? gridDim.x * bw : gridDim.x * blockDim.x;
-    for (int l = l1 - 1; l >= l0; --l) {
-        const int q0 = FUSED ? d.bs_beg[l] : rg.s0, q1 = FUSED ? d.bs_end[l] : rg.s1;
-        {   // loads are never gated on the scenario's status (it would put one more dependent load on the critical path); stores are
-            if (BATCH) {
-                int q = q0 + 4 * first;
-                KktBwdItem u[4];
-                if (q < q1) {
+    const int first = BATCH ? blockIdx.x * kWarps + warp : blockIdx.x * blockDim.x + threadIdx.x;
+    const int stride = BATCH ? gridDim.x * kWarps : gridDim.x * blockDim.x;
+    // loads are never gated on the scenario's status (it would put one more dependent load on the critical path); stores are
+    const int q0 = rg.s0, q1 = rg.s1;
+    if (BATCH) {
+        int q = q0 + 4 * first;
+        KktBwdItem u[4];
+        if (q < q1) {
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) u[i] = d.bwd[q + i < q1 ? q + i : q];
-                }
-                if (l == l1 - 1) pdl_wait();
-                while (q < q1) {
-                    double a[4], x[4], c[4], t[4];
-                    int dst[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        a[i] = d.W[(int64_t)u[i].pos * B + s];
-                        x[i] = v[(int64_t)u[i].src * B + s];
-                        c[i] = d.invd[(int64_t)u[i].k * B + s];
-                        t[i] = v[(int64_t)u[i].dst * B + s];
-                        dst[i] = u[i].dst;
-                    }
-                    const int qn = q + 4 * stride;
-                    if (qn < q1) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) u[i] = d.bwd[qn + i < q1 ? qn + i : qn];
-                    }
-#pragma unroll
-                    for (int i = 0; i < 4; ++i)
-                        if (q + i < q1 && live) v[(int64_t)dst[i] * B + s] = t[i] - c[i] * a[i] * x[i];
-                    q = qn;
-                }
-            } else {
-                if (l == l1 - 1) pdl_wait();
-                for (int q = q0 + first; q < q1; q += stride) {
-                    const KktBwdItem u = d.bwd[q];
-                    if (live) v[u.dst] -= d.invd[u.k] * d.W[u.pos] * v[u.src];
-                }
-            }
-            const int c0 = FUSED ? d.bmstep[l] : rg.m0, c1 = FUSED ? d.bmstep[l + 1] : rg.m1;
-            for (int c = c0 + first; c < c1; c += stride) {
-                const KktRange r = d.bmchunk[c];
-                int dst;
-                double tv;
-                const double acc = chunk_sum_vec(d, d.bwd, v, r.begin, r.end, B, s, dst, tv);
-                if (live) v[(int64_t)dst * B + s] = tv - acc;
-            }
+            for (int i = 0; i < 4; ++i) u[i] = d.bwd[q + i < q1 ? q + i : q];
         }
-        if (FUSED) __syncthreads();
+        pdl_wait();
+        while (q < q1) {
+            double a[4], x[4], c[4], t[4];
+            int dst[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                a[i] = d.W[(int64_t)u[i].pos * B + s];
+                x[i] = v[(int64_t)u[i].src * B + s];
+                c[i] = d.invd[(int64_t)u[i].k * B + s];
+                t[i] = v[(int64_t)u[i].dst * B + s];
+                dst[i] = u[i].dst;
+            }
+            const int qn = q + 4 * stride;
+            if (qn < q1) {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) u[i] = d.bwd[qn + i < q1 ? qn + i : qn];
+            }
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+                if (q + i < q1 && live) v[(int64_t)dst[i] * B + s] = t[i] - c[i] * a[i] * x[i];
+            q = qn;
+        }
+    } else {
+        pdl_wait();
+        for (int q = q0 + first; q < q1; q += stride) {
+            const KktBwdItem u = d.bwd[q];
+            if (live) v[u.dst] -= d.invd[u.k] * d.W[u.pos] * v[u.src];
+        }
+    }
+    for (int c = rg.m0 + first; c < rg.m1; c += stride) {
+        const KktRange r = d.bmchunk[c];
+        int dst;
+        double tv;
+        const double acc = chunk_sum_vec(d, d.bwd, v, r.begin, r.end, B, s, dst, tv);
+        if (live) v[(int64_t)dst * B + s] = tv - acc;
     }
 }
 
@@ -1366,7 +1341,7 @@ struct IpmEngine {
     KktSymbolic sym;
     bool ready = false;
     int B = 0;
-    DBuf<int> fs_beg, fs_end, fmstep, ws_beg, ws_end, wmstep, bs_beg, bs_end, bmstep, perm, inv, kmap;
+    DBuf<int> perm, inv, kmap;
     DBuf<KktRange> fmchunk, wmchunk, bmchunk;
     DBuf<KktPanel> panels;
     DBuf<KktPanelTask> ptasks;
@@ -1390,20 +1365,6 @@ struct IpmEngine {
         if (g_solve_work) cudaGraphExecDestroy(g_solve_work);
     }
 
-    // steps with at most this many items are walked by one 1024-thread block per 32 scenarios instead of getting a
-    // launch of their own: a launch costs ~4-5 us on the critical path, a pass of the block ~1.5 us
-    static int narrow_for(int B) {
-        const char *e = getenv("ASM_IPM_NARROW");
-        if (e) return atoi(e);
-        return B == 1 ? 2048 : 64;
-    }
-    // widest supernode (1 = none)
-    static int supernode_for(int B) {
-        const char *e = getenv(B == 1 ? "ASM_IPM_SUPERNODE_SINGLE" : "ASM_IPM_SUPERNODE");
-        if (e) return std::max(1, std::min(atoi(e), kSnMax));
-        return kSnMax;
-    }
-    bool supernodal() const { return !sym.panels.empty(); }
     template <class T>
     static int up(DBuf<T> &dst, const std::vector<T> &src) {
         ASM_TRY(dst.alloc(std::max<size_t>(src.size(), 1)));
@@ -1420,23 +1381,14 @@ struct IpmEngine {
                 return fail(ASM_E_INVALID, "duplicate (row, column) entries in the pattern: the barrier engine needs a deduplicated CSR");
         }
         const auto t0 = std::chrono::steady_clock::now();
-        if (sym.build(n, m, row_ptr.data(), col_idx.data(), narrow_for(B), supernode_for(B)))
+        if (sym.build(n, m, row_ptr.data(), col_idx.data(), kkt_supernode_width()))
             return fail(ASM_E_INVALID, "KKT symbolic analysis failed (index out of range or more than 2^31 update terms)");
         symbolic_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         ASM_TRY(up(terms, sym.terms));
-        ASM_TRY(up(fs_beg, sym.fs_beg));
-        ASM_TRY(up(fs_end, sym.fs_end));
-        ASM_TRY(up(fmstep, sym.fmstep));
         ASM_TRY(up(fmchunk, sym.fmchunk));
         ASM_TRY(up(fwd, sym.fwd));
-        ASM_TRY(up(ws_beg, sym.ws_beg));
-        ASM_TRY(up(ws_end, sym.ws_end));
-        ASM_TRY(up(wmstep, sym.wmstep));
         ASM_TRY(up(wmchunk, sym.wmchunk));
         ASM_TRY(up(bwd, sym.bwd));
-        ASM_TRY(up(bs_beg, sym.bs_beg));
-        ASM_TRY(up(bs_end, sym.bs_end));
-        ASM_TRY(up(bmstep, sym.bmstep));
         ASM_TRY(up(bmchunk, sym.bmchunk));
         ASM_TRY(up(panels, sym.panels));
         ASM_TRY(up(ptasks, sym.ptasks));
@@ -1467,19 +1419,10 @@ struct IpmEngine {
     KktDev dev() const {
         KktDev d;
         d.terms = terms.p;
-        d.fs_beg = fs_beg.p;
-        d.fs_end = fs_end.p;
-        d.fmstep = fmstep.p;
         d.fmchunk = fmchunk.p;
         d.fwd = fwd.p;
-        d.ws_beg = ws_beg.p;
-        d.ws_end = ws_end.p;
-        d.wmstep = wmstep.p;
         d.wmchunk = wmchunk.p;
         d.bwd = bwd.p;
-        d.bs_beg = bs_beg.p;
-        d.bs_end = bs_end.p;
-        d.bmstep = bmstep.p;
         d.bmchunk = bmchunk.p;
         d.panels = panels.p;
         d.ptasks = ptasks.p;
@@ -1531,17 +1474,13 @@ struct IpmEngine {
         cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
     }
     // grid of a step kernel.  Batch: a warp per item, scenarios over blockIdx.y; single LP: a thread per item
-    dim3 level_grid(const KktLaunch &L, int64_t multi = 0) const {
-        unsigned gx = 1;
+    dim3 level_grid(int items, int multi) const {
         const int per_block = B == 1 ? kThreads : kWarps;
-        if (!L.fused) {
-            const int gy = B == 1 ? 1 : B / 32;
-            int64_t cap = std::max<int64_t>(1, (int64_t)kMaxBlocksX * 4 / gy);
-            // batch: four single-term chunks per warp pass, one multi-term chunk per warp pass
-            const int64_t units = B == 1 ? L.items : (L.items - multi + 3) / 4 + multi + 1;
-            gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>((units + per_block - 1) / per_block, cap));
-        }
-        return dim3(gx, B == 1 ? 1 : B / 32);
+        const int gy = B == 1 ? 1 : B / 32;
+        const int64_t cap = std::max<int64_t>(1, (int64_t)kMaxBlocksX * 4 / gy);
+        // batch: four single-term chunks per warp pass, one multi-term chunk per warp pass
+        const int64_t units = B == 1 ? items : (items - multi + 3) / 4 + multi + 1;
+        return dim3((unsigned)std::max<int64_t>(1, std::min<int64_t>((units + per_block - 1) / per_block, cap)), gy);
     }
     void enqueue_factor(LpView &v, cudaStream_t st, int64_t &count) {
         KktDev d = dev();
@@ -1555,140 +1494,65 @@ struct IpmEngine {
                 k_kkt_scatter<false><<<gz.grid, gz.block, 0, st>>>(v, d, nz);
         }
         count += 2;
-        if (supernodal()) {   // per step: the panels of its supernodes, then the updates that leave them
-            const int gy = (B + 31) / 32;
-            for (int l = 0; l < sym.n_levels; ++l) {
-                // wide tasks (rows of the wide panels) come first in the step's task range, then the narrow tasks
-                const int np = sym.pstep[l + 1] - sym.pstep[l], npw = sym.pwide[l];
-                const int nt = sym.ptstep[l + 1] - sym.ptstep[l], ntw = sym.ptwide[l];
-                if (np > 0) {
-                    const int per = kPanelThreads / 32;
-                    launch_step(k_sn_diag, dim3(npw + (nt - ntw + per - 1) / per, gy), kPanelThreads, st, d, B, sym.pstep[l], npw,
-                                sym.ptstep[l] + ntw, nt - ntw, v.state);
-                    ++count;
-                }
-                if (ntw > 0) {
-                    launch_step(k_sn_rows, dim3(ntw, gy), kPanelThreads, st, d, B, sym.ptstep[l], v.state);
-                    ++count;
-                }
-                const KktStepRange rg = {sym.fs_beg[l], sym.fs_end[l], sym.fmstep[l], sym.fmstep[l + 1]};
-                const int multi = rg.m1 - rg.m0, items = rg.s1 - rg.s0 + multi;
-                if (items > 0) {
-                    const dim3 grid = level_grid(KktLaunch{l, l + 1, 0, items}, multi);
-                    if (B > 1)
-                        launch_step(k_ldl_factor<true, false>, grid, kThreads, st, d, B, l, l + 1, v.state, rg);
-                    else
-                        launch_step(k_ldl_factor<false, false>, grid, kThreads, st, d, B, l, l + 1, v.state, rg);
-                    ++count;
-                }
+        const int gy = (B + 31) / 32;
+        for (int l = 0; l < sym.n_levels; ++l) {   // per step: the panels of its supernodes, then the updates that leave them
+            // wide tasks (rows of the wide panels) come first in the step's task range, then the narrow tasks
+            const int np = sym.pstep[l + 1] - sym.pstep[l], npw = sym.pwide[l];
+            const int nt = sym.ptstep[l + 1] - sym.ptstep[l], ntw = sym.ptwide[l];
+            if (np > 0) {
+                const int per = kPanelThreads / 32;
+                launch_step(k_sn_diag, dim3(npw + (nt - ntw + per - 1) / per, gy), kPanelThreads, st, d, B, sym.pstep[l], npw,
+                            sym.ptstep[l] + ntw, nt - ntw, v.state);
+                ++count;
             }
-            return;
-        }
-        for (const KktLaunch &L : sym.flaunch) {
-            const dim3 grid = level_grid(L);
-            const KktStepRange rg = {sym.fs_beg[L.l0], sym.fs_end[L.l0], sym.fmstep[L.l0], sym.fmstep[L.l0 + 1]};
-            if (B > 1) {
-                if (L.fused)
-                    launch_step(k_ldl_factor<true, true>, grid, kFusedThreads, st, d, B, L.l0, L.l1, v.state, rg);
-                else
-                    launch_step(k_ldl_factor<true, false>, grid, kThreads, st, d, B, L.l0, L.l1, v.state, rg);
-            } else {
-                if (L.fused)
-                    launch_step(k_ldl_factor<false, true>, grid, kFusedThreads, st, d, B, L.l0, L.l1, v.state, rg);
-                else
-                    launch_step(k_ldl_factor<false, false>, grid, kThreads, st, d, B, L.l0, L.l1, v.state, rg);
+            if (ntw > 0) {
+                launch_step(k_sn_rows, dim3(ntw, gy), kPanelThreads, st, d, B, sym.ptstep[l], v.state);
+                ++count;
             }
-            ++count;
+            const KktStepRange rg = {sym.fs_beg[l], sym.fs_end[l], sym.fmstep[l], sym.fmstep[l + 1]};
+            const int multi = rg.m1 - rg.m0, items = rg.s1 - rg.s0 + multi;
+            if (items > 0) {
+                launch_step(B > 1 ? k_ldl_factor<true> : k_ldl_factor<false>, level_grid(items, multi), kThreads, st, d, B, v.state, rg);
+                ++count;
+            }
         }
     }
     void enqueue_solve(LpView &v, double *vec, cudaStream_t st, int64_t &count) {
         KktDev d = dev();
-        if (supernodal()) {
-            const int gy = (B + 31) / 32;
-            for (int l = 0; l < sym.n_levels; ++l) {
-                const int np = sym.pstep[l + 1] - sym.pstep[l], nwide = sym.pwide[l];
-                if (np > 0) {
-                    const int per = kPanelSolveThreads / 32;
-                    launch_step(k_sn_solve<true>, dim3(nwide + (np - nwide + per - 1) / per, gy), kPanelSolveThreads, st, d, vec, B, sym.pstep[l], nwide, np, v.state);
-                    ++count;
-                }
-                const KktStepRange rg = {sym.ws_beg[l], sym.ws_end[l], sym.wmstep[l], sym.wmstep[l + 1]};
-                const int multi = rg.m1 - rg.m0, items = rg.s1 - rg.s0 + multi;
-                if (items > 0) {
-                    const dim3 grid = level_grid(KktLaunch{l, l + 1, 0, items}, multi);
-                    if (B > 1)
-                        launch_step(k_ldl_fwd<true, false>, grid, kThreads, st, d, vec, B, l, l + 1, v.state, rg);
-                    else
-                        launch_step(k_ldl_fwd<false, false>, grid, kThreads, st, d, vec, B, l, l + 1, v.state, rg);
-                    ++count;
-                }
+        const int gy = (B + 31) / 32;
+        for (int l = 0; l < sym.n_levels; ++l) {
+            const int np = sym.pstep[l + 1] - sym.pstep[l], nwide = sym.pwide[l];
+            if (np > 0) {
+                const int per = kPanelSolveThreads / 32;
+                launch_step(k_sn_solve<true>, dim3(nwide + (np - nwide + per - 1) / per, gy), kPanelSolveThreads, st, d, vec, B, sym.pstep[l], nwide, np, v.state);
+                ++count;
             }
-            const Geo gN = geo_for(sym.N, B);
-            if (B > 1)
-                k_ldl_diag<true><<<gN.grid, gN.block, 0, st>>>(d, vec, B, v.state);
-            else
-                k_ldl_diag<false><<<gN.grid, gN.block, 0, st>>>(d, vec, B, v.state);
-            ++count;
-            for (int l = sym.n_levels - 1; l >= 0; --l) {
-                const int np = sym.pstep[l + 1] - sym.pstep[l], nwide = sym.pwide[l];
-                if (np > 0) {
-                    const int per = kPanelSolveThreads / 32;
-                    launch_step(k_sn_solve<false>, dim3(nwide + (np - nwide + per - 1) / per, gy), kPanelSolveThreads, st, d, vec, B, sym.pstep[l], nwide, np, v.state);
-                    ++count;
-                }
-                const KktStepRange rg = {sym.bs_beg[l], sym.bs_end[l], sym.bmstep[l], sym.bmstep[l + 1]};
-                const int multi = rg.m1 - rg.m0, items = rg.s1 - rg.s0 + multi;
-                if (items > 0) {
-                    const dim3 grid = level_grid(KktLaunch{l, l + 1, 0, items}, multi);
-                    if (B > 1)
-                        launch_step(k_ldl_bwd<true, false>, grid, kThreads, st, d, vec, B, l, l + 1, v.state, rg);
-                    else
-                        launch_step(k_ldl_bwd<false, false>, grid, kThreads, st, d, vec, B, l, l + 1, v.state, rg);
-                    ++count;
-                }
+            const KktStepRange rg = {sym.ws_beg[l], sym.ws_end[l], sym.wmstep[l], sym.wmstep[l + 1]};
+            const int multi = rg.m1 - rg.m0, items = rg.s1 - rg.s0 + multi;
+            if (items > 0) {
+                launch_step(B > 1 ? k_ldl_fwd<true> : k_ldl_fwd<false>, level_grid(items, multi), kThreads, st, d, vec, B, v.state, rg);
+                ++count;
             }
-            return;
         }
-        for (const KktLaunch &L : sym.wlaunch) {
-            const dim3 grid = level_grid(L);
-            const KktStepRange rg = {sym.ws_beg[L.l0], sym.ws_end[L.l0], sym.wmstep[L.l0], sym.wmstep[L.l0 + 1]};
-            if (B > 1) {
-                if (L.fused)
-                    launch_step(k_ldl_fwd<true, true>, grid, kFusedThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
-                else
-                    launch_step(k_ldl_fwd<true, false>, grid, kThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
-            } else {
-                if (L.fused)
-                    launch_step(k_ldl_fwd<false, true>, grid, kFusedThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
-                else
-                    launch_step(k_ldl_fwd<false, false>, grid, kThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
+        const Geo gN = geo_for(sym.N, B);
+        if (B > 1)
+            k_ldl_diag<true><<<gN.grid, gN.block, 0, st>>>(d, vec, B, v.state);
+        else
+            k_ldl_diag<false><<<gN.grid, gN.block, 0, st>>>(d, vec, B, v.state);
+        ++count;
+        for (int l = sym.n_levels - 1; l >= 0; --l) {
+            const int np = sym.pstep[l + 1] - sym.pstep[l], nwide = sym.pwide[l];
+            if (np > 0) {
+                const int per = kPanelSolveThreads / 32;
+                launch_step(k_sn_solve<false>, dim3(nwide + (np - nwide + per - 1) / per, gy), kPanelSolveThreads, st, d, vec, B, sym.pstep[l], nwide, np, v.state);
+                ++count;
             }
-            ++count;
-        }
-        {
-            const Geo gN = geo_for(sym.N, B);
-            if (B > 1)
-                k_ldl_diag<true><<<gN.grid, gN.block, 0, st>>>(d, vec, B, v.state);
-            else
-                k_ldl_diag<false><<<gN.grid, gN.block, 0, st>>>(d, vec, B, v.state);
-            ++count;
-        }
-        for (auto it = sym.blaunch.rbegin(); it != sym.blaunch.rend(); ++it) {
-            const KktLaunch &L = *it;
-            const dim3 grid = level_grid(L);
-            const KktStepRange rg = {sym.bs_beg[L.l0], sym.bs_end[L.l0], sym.bmstep[L.l0], sym.bmstep[L.l0 + 1]};
-            if (B > 1) {
-                if (L.fused)
-                    launch_step(k_ldl_bwd<true, true>, grid, kFusedThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
-                else
-                    launch_step(k_ldl_bwd<true, false>, grid, kThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
-            } else {
-                if (L.fused)
-                    launch_step(k_ldl_bwd<false, true>, grid, kFusedThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
-                else
-                    launch_step(k_ldl_bwd<false, false>, grid, kThreads, st, d, vec, B, L.l0, L.l1, v.state, rg);
+            const KktStepRange rg = {sym.bs_beg[l], sym.bs_end[l], sym.bmstep[l], sym.bmstep[l + 1]};
+            const int multi = rg.m1 - rg.m0, items = rg.s1 - rg.s0 + multi;
+            if (items > 0) {
+                launch_step(B > 1 ? k_ldl_bwd<true> : k_ldl_bwd<false>, level_grid(items, multi), kThreads, st, d, vec, B, v.state, rg);
+                ++count;
             }
-            ++count;
         }
     }
     // the level sequences never change for a handle: captured once, replayed every Newton step

@@ -21,8 +21,6 @@
 //     that the kernel can keep four of them in flight per warp,
 //   * the same chunked fan-out lists for the forward substitution; the backward substitution needs no chunks
 //     (the rows of a column are its ancestors, which sit on distinct levels),
-//   * the launch plan (wide steps: one launch each; runs of narrow steps: one launch of a single block per 32
-//     scenarios that walks them with __syncthreads()),
 //   * optionally (sn > 1) SUPERNODES: chains c_0 -> c_1 -> ... of at most sn columns along the elimination tree whose
 //     patterns nest exactly (pattern(c_i) = {c_i+1} + pattern(c_i+1)), the separators of the network.  All columns
 //     of a supernode share one step; the updates inside a supernode (its dense diagonal block and the rows below
@@ -69,11 +67,6 @@ struct KktBwdItem {
 };
 struct KktRange {
     int begin, end;
-};
-struct KktLaunch {
-    int l0, l1;  // steps [l0, l1)
-    int fused;   // 1: one block walks the steps; 0: l1 == l0 + 1, grid over the items of the step
-    int items;   // largest step of the launch
 };
 constexpr int kLastBit = 1 << 30;  // in KktTerm::t of the first term of a chunk: last update of this pivot -> invert it
 constexpr int kSnMax = 16;         // widest supernode
@@ -123,6 +116,14 @@ inline void kkt_parallel_for(int n, int chunk, F f) {
     for (std::thread &x : th) x.join();
 }
 
+// widest supernode, the one parameter of the schedule: ASM_IPM_SUPERNODE, default kSnMax; 1 = no supernodes, one step
+// per level of the elimination tree
+inline int kkt_supernode_width() {
+    const char *e = getenv("ASM_IPM_SUPERNODE");
+    if (e) return std::max(1, std::min(atoi(e), kSnMax));
+    return kSnMax;
+}
+
 struct KktSymbolic {
     int n = 0, m = 0, N = 0;
     int64_t nnzL = 0, nterms = 0;
@@ -152,7 +153,6 @@ struct KktSymbolic {
     std::vector<KktBwdItem> bwd;
     std::vector<int> bs_beg, bs_end, bmstep;
     std::vector<KktRange> bmchunk;
-    std::vector<KktLaunch> flaunch, wlaunch, blaunch;
     // supernodes (empty when built with sn <= 1): panels sorted by step, pstep[l] .. pstep[l+1]; the row tasks of the
     // factorisation likewise in ptstep
     int sn_width = 1;
@@ -165,7 +165,7 @@ struct KktSymbolic {
     int64_t panel_slots = 0;       // size of the buffer of factorised diagonal blocks (entries per LP)
 
     // K: m x n CSR pattern (0-based).  Returns 0, or -1 when an index is out of range / the term count overflows.
-    int build(int n_, int m_, const int *row_ptr, const int *col_idx, int narrow = 64, int sn = 1) {
+    int build(int n_, int m_, const int *row_ptr, const int *col_idx, int sn) {
         sn_width = std::max(1, std::min(sn, kSnMax));
         n_intra = 0;
         n = n_;
@@ -412,11 +412,6 @@ struct KktSymbolic {
         regroup(bwd, [&](const KktBwdItem &u) { return level[inv[u.src]]; }, [](const KktBwdItem &u) { return u.dst; },
                 bs_beg, bs_end, bmstep, bmchunk);
         KKT_PHASE("substitution lists");
-        auto work = [&](const std::vector<int> &sb, const std::vector<int> &se, const std::vector<int> &ms) {
-            std::vector<int> w(n_levels + 1, 0);
-            for (int l = 0; l < n_levels; ++l) w[l + 1] = w[l] + (se[l] - sb[l]) + (ms[l + 1] - ms[l]);
-            return w;
-        };
         {   // compulsory traffic per step (see f_distinct_reads)
             std::vector<int> stampW(nnzL + 1, -1), stampD(N, -1), stampV(N, -1), stampT(nnzL + N + 1, -1);
             size_t q = 0;
@@ -464,9 +459,6 @@ struct KktSymbolic {
             }
         }
         KKT_PHASE("traffic statistics");
-        plan(work(fs_beg, fs_end, fmstep), narrow, flaunch);
-        plan(work(ws_beg, ws_end, wmstep), narrow, wlaunch);
-        plan(work(bs_beg, bs_end, bmstep), narrow, blaunch);
         return 0;
     }
 
@@ -614,30 +606,6 @@ struct KktSymbolic {
             longest_chunk = std::max(longest_chunk, longest[l]);
         }
         return n_chunks;
-    }
-
-    void plan(const std::vector<int> &sptr, int narrow, std::vector<KktLaunch> &out) const {
-        out.clear();
-        int l = 0;
-        while (l < n_levels) {
-            const int items = sptr[l + 1] - sptr[l];
-            if (items == 0) {
-                ++l;
-                continue;
-            }
-            if (items > narrow) {
-                out.push_back(KktLaunch{l, l + 1, 0, items});
-                ++l;
-                continue;
-            }
-            int e = l, mx = 0;
-            while (e < n_levels && sptr[e + 1] - sptr[e] <= narrow) {
-                mx = std::max(mx, sptr[e + 1] - sptr[e]);
-                ++e;
-            }
-            out.push_back(KktLaunch{l, e, e - l > 1 ? 1 : 0, std::max(mx, 1)});
-            l = e;
-        }
     }
 
     // ---- host reference of the device numerics (same lists, same order): used by the CPU self test ------------

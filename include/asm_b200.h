@@ -254,18 +254,17 @@ int asm_plan_check(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, const
  * pairs of the last solve, distinct f64 operands read / targets updated per factorisation and per substitution pair
  * (summed over the levels: the compulsory HBM traffic of a batch larger than L2, DESIGN.md 4.4); times[4]: symbolic analysis
  * ms, Newton steps of the last solve, factor / solve ms of the traced step (ASM_TRACE=1).  Either pointer may be NULL.
- * Environment switches read when a handle builds its engine: ASM_IPM_SUPERNODE / ASM_IPM_SUPERNODE_SINGLE = widest
- * supernode for batches / single LPs (default 16, 1 = one column per level), ASM_IPM_NARROW = items below which runs of
- * levels are fused into one block (level schedule only), ASM_NO_PDL = plain stream-ordered launches */
+ * Environment switches read when a handle builds its engine: ASM_IPM_SUPERNODE = widest supernode (default 16, 1 = one
+ * column per level), ASM_NO_PDL = plain stream-ordered launches */
 int asm_slp_ipm_info(asm_slp *h, int64_t *stats, double *times);
 /* average device time (CUDA events on the handle's stream) of one numeric factorisation and one substitution pair of
  * the whole batch, `reps` launches each, on the data of the last solve */
 int asm_slp_ipm_timing(asm_slp *h, int32_t reps, double *factor_ms, double *solve_ms);
 /* host-only self test of the barrier engine's symbolic analysis (no device needed): factorises
  * [-diag(dx) K'; K diag(ew)] and solves one right-hand side on the host with the lists and the summation order of the
- * device kernels (supernodes as a batch handle would use them).  rhs_sol[n_cols + n_rows]: right-hand side in,
- * solution out.  stats[8]: nnz(L), terms, steps, factor / forward / backward launches of the level plan, longest chunk,
- * chunks */
+ * device kernels (supernodes as a handle would use them).  rhs_sol[n_cols + n_rows]: right-hand side in, solution out.
+ * stats[8]: nnz(L), terms, steps, steps with fan-out items in the factorisation / forward / backward substitution (the
+ * step-kernel launches of each), longest chunk, chunks */
 int asm_kkt_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, const int32_t *col_idx, const double *vals,
                      const double *dx, const double *ew, double *rhs_sol, int64_t *stats);
 

@@ -1,7 +1,8 @@
 """The barrier engine's two schedules -- supernodal (default) and one column per level of the elimination tree
-(ASM_IPM_SUPERNODE=1 / ASM_IPM_SUPERNODE_SINGLE=1, read when a handle builds its engine) -- factorise the same matrices
-with different kernels (dense panels + chunked updates vs single-term updates) and must return the same LP solutions.
-Both are also run through test_gpu_lp_conformance.py / test_gpu_sublp.py by setting the variables for the whole run."""
+(ASM_IPM_SUPERNODE=1, read when a handle builds its engine, for batches and single LPs alike) -- factorise the same
+matrices with different kernels (dense panels + chunked updates vs single-term updates) and must return the same LP
+solutions.  Both are also run through test_gpu_lp_conformance.py / test_gpu_sublp.py by setting the variable for the
+whole run."""
 import numpy as np
 import pytest
 
@@ -31,7 +32,6 @@ def test_schedules_agree(gpu, monkeypatch, B, fr):
     res = {}
     for name, width in (("supernodal", "16"), ("levels", "1")):
         monkeypatch.setenv("ASM_IPM_SUPERNODE", width)
-        monkeypatch.setenv("ASM_IPM_SUPERNODE_SINGLE", width)
         lp = SubLp(m0.n, m0.m, m0.j_str, sq(d["xL"]), sq(d["xU"]), sq(d["gL"]), sq(d["gU"]), batch=B, engine=4)
         out = lp.sub_optimize(sq(d["x"]), sq(d["f"]), sq(d["df"]), sq(d["E"]), sq(d["dE"]), 1000.0, fr)
         res[name] = dict(status=np.atleast_1d(out[5]).astype(int),

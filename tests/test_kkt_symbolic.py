@@ -27,7 +27,7 @@ def _selftest(lib, K, dx, ew, rhs):
                               capi.dptr(np.ascontiguousarray(ew, dtype=np.float64)), capi.dptr(sol),
                               stats.ctypes.data_as(capi.c_int64_p))
     capi.check(rc)
-    return sol, dict(zip(("nnz_L", "terms", "levels", "f_launch", "w_launch", "b_launch", "longest_chunk", "chunks"),
+    return sol, dict(zip(("nnz_L", "terms", "levels", "f_steps", "w_steps", "b_steps", "longest_chunk", "chunks"),
                          (int(v) for v in stats)))
 
 
