@@ -65,8 +65,9 @@ class Parameters:
     # engine options forwarded to asm_lp_params (not in the reference)
     lp_options: dict = field(default_factory=dict)
     device: int = 0
-    # line search on an examples.acopf.AcopfModel with the B200 engine: evaluate f, g, the Jacobian and the
-    # backtracking trials with the device-side ACOPF evaluator instead of the host callbacks (SURVEY.md 8(f)-1)
+    # either algorithm on an examples.acopf.AcopfModel with the B200 engine: evaluate f, g, the Jacobian and the
+    # merit at trial points (backtracking / step quality) with the device-side ACOPF evaluator instead of the host
+    # callbacks (SURVEY.md 8(f)-1)
     device_evaluator: bool = False
 
 
@@ -370,7 +371,11 @@ class SlpTR(_Slp):
 
     def compute_nu(self):                                                   # slp.jl:54-66
         if self.iter == 1:
-            norm_df = 1.0 if self.feasibility_restoration else float(np.linalg.norm(self.df))
+            if self.feasibility_restoration:
+                norm_df = 1.0
+            else:
+                df = self.optimizer.get_eval_df() if self.options.device_evaluator else self.df
+                norm_df = float(np.linalg.norm(df))
             rn = self.optimizer.row_norms()
             self.nu = np.maximum(1.0, norm_df / np.maximum(1.0, rn))
         else:
@@ -409,12 +414,25 @@ class SlpTR(_Slp):
         self.start_time = time.time()
         self.clip_start()
         self.iter = 1
+        dev_eval = bool(o.device_evaluator)
+        if dev_eval:
+            if self.optimizer is None:
+                self.optimizer = self._instantiate()
+            self.optimizer.attach_acopf(self.problem.source)
         while True:
-            self.eval_functions()
-            self.p, self.lam, self.mult_x_U, self.mult_x_L, self.p_slack, status = self.sub_optimize(self.delta)
+            if dev_eval:
+                self.optimizer.eval_acopf(self.x, self.delta, self.feasibility_restoration)
+                self.f = float(np.atleast_1d(self.optimizer.get_eval_f())[0])
+                out = self.sub_optimize(self.delta, True)
+            else:
+                self.eval_functions()
+                out = self.sub_optimize(self.delta)
+            self.p, self.lam, self.mult_x_U, self.mult_x_L, self.p_slack, status = out
             if status not in (LP_OPTIMAL, LP_INFEASIBLE):
                 self.ret = -3                      # same deviation as in SlpLS.run (slp_trust_region.jl:131)
-                if self.optimizer.norm_violations(pr.eval_g(self.x, np.zeros(pr.m)), self.x, 1) <= o.tol_infeas:
+                # g(x) of this iteration: on the device with the device evaluator (E = None), else from the callback
+                E = None if dev_eval else pr.eval_g(self.x, np.zeros(pr.m))
+                if self.optimizer.norm_violations(E, self.x, 1) <= o.tol_infeas:
                     self.ret = 6
                 break
             elif status == LP_INFEASIBLE:
@@ -460,17 +478,13 @@ class SlpTR(_Slp):
         return self
 
 
-class SlpLSBatch:
-    """B independent line-search SLP solves that share one Jacobian pattern (load scenarios of one network,
-    BASELINE config 5), advanced in lock-step so that every round is **one** batched call of the device hot path:
-    one `update`, the KKT reductions, one sub-LP batch solve (two when some scenarios are in feasibility
-    restoration), and one batched merit evaluation per backtracking round.  Per scenario the control flow is
-    exactly ``SlpLS.run`` (reference ``slp_line_search.jl:78-215``) — a scenario that terminates simply stops
-    moving while the others go on.  ``problems`` are objects with the ``Model.from_problem`` interface.
+class _SlpBatch:
+    """B independent SLP solves that share one Jacobian pattern (load scenarios of one network, BASELINE config 5),
+    advanced in lock-step so that every round is one batched call of each operation of the device hot path.
+    ``problems`` are objects with the ``Model.from_problem`` interface.  Subclasses give the round (``run``) and
+    ``warm_start``, the engine's warm-start flag (see ``_Slp._instantiate``)."""
 
-    ``device_evaluator=True`` (ACOPF scenarios of one network, B200 engine): the NLP callbacks are not called at all —
-    f, g and the Jacobian are evaluated by the device-side ACOPF evaluator (``SubLp.eval_acopf``) and every
-    backtracking trial is one ``SubLp.acopf_trial`` call for the whole batch."""
+    warm_start = 1
 
     def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
         self.device_evaluator = bool(device_evaluator)
@@ -479,8 +493,8 @@ class SlpLSBatch:
         p0 = self.problems[0]
         self.B, self.n, self.m = len(self.problems), p0.n, p0.m
         for pr in self.problems:
-            assert pr.n == self.n and pr.m == self.m and np.array_equal(pr.j_str, p0.j_str), \
-                "batched scenarios must share the Jacobian pattern"
+            if pr.n != self.n or pr.m != self.m or not np.array_equal(pr.j_str, p0.j_str):
+                raise ValueError("batched scenarios must share the Jacobian pattern")
         B, n, m = self.B, self.n, self.m
         self.x = np.array([np.array(pr.x0, dtype=float) for pr in self.problems])
         self.f = np.zeros(B)
@@ -496,12 +510,13 @@ class SlpLSBatch:
         self.ret = np.full(B, -5, dtype=np.int64)
         self.running = np.ones(B, dtype=bool)
         self.fr = np.zeros(B, dtype=bool)
-        self.alpha = np.zeros(B)
         self.prim_infeas = np.full(B, INF)
         self.dual_infeas = np.full(B, INF)
         self.compl = np.full(B, INF)
         self.obj_val = np.zeros(B)
         self.rounds = 0
+        self.two_phase_rounds = 0       # rounds with scenarios in both phases: two sub-LP batch solves
+        self.lp_solves = np.zeros(B, dtype=np.int64)
         self.lp_iterations = 0
         self.optimizer = None
 
@@ -511,7 +526,7 @@ class SlpLSBatch:
         arr = lambda name: np.array([np.asarray(getattr(pr, name), dtype=float) for pr in prs])  # noqa: E731
         if o.external_optimizer == "B200LP":
             opt = SubLp(self.n, self.m, prs[0].j_str, arr("x_L"), arr("x_U"), arr("g_L"), arr("g_U"), batch=self.B,
-                        device=o.device, **{"warm_start": 1, **o.lp_options})
+                        device=o.device, **{"warm_start": self.warm_start, **o.lp_options})
             opt._squeeze = False
             if self.device_evaluator:
                 # the device evaluator holds ONE network: every scenario must share everything but its loads (which
@@ -531,6 +546,13 @@ class SlpLSBatch:
         return o.external_optimizer(self.n, self.m, prs[0].j_str, arr("x_L"), arr("x_U"), arr("g_L"), arr("g_U"),
                                     batch=self.B)
 
+    def _clip_starts(self):
+        for s, pr in enumerate(self.problems):                              # slp_line_search.jl:96-105
+            lo = pr.x_L > -INF
+            self.x[s][lo] = np.maximum(self.x[s][lo], pr.x_L[lo])
+            up = pr.x_U > -INF
+            self.x[s][up] = np.minimum(self.x[s][up], pr.x_U[up])
+
     def _eval(self, s):
         pr = self.problems[s]
         self.f[s] = pr.eval_f(self.x[s])
@@ -538,31 +560,46 @@ class SlpLSBatch:
         pr.eval_g(self.x[s], self.E[s])
         pr.eval_jac_g(self.x[s], "eval", None, None, self.dE[s])
 
-    def _solve_phase(self, fr, sel=None):
-        """Sub-LP batch of one phase; returns the extract tuple plus phi(0) and the directional derivative computed
-        while the device still holds this phase's step and slacks.  ``sel``: the scenarios that are running in this
-        phase -- the others (terminated, or in the other phase, whose normal LP is infeasible by construction) are
-        masked out of the solve instead of being re-solved every round."""
+    def _solve_phase(self, fr, sel, delta):
+        """Sub-LP batch of one phase (``delta``: the trust-region radius, scalar or per scenario).  ``sel``: the
+        scenarios that are running in this phase -- the others (terminated, or in the other phase, whose normal LP is
+        infeasible by construction) are masked out of the solve instead of being re-solved every round."""
         opt = self.optimizer
-        if sel is not None and hasattr(opt, "set_active"):
+        if hasattr(opt, "set_active"):
             opt.set_active(sel)
         if fr and self.device_evaluator:
-            opt.eval_acopf(self.x, 1000.0, True)
-        elif fr:                    # the normal-phase data push was done for the KKT metrics of this round
-            opt.update(self.x, self.f, self.df, self.E, self.dE, 1000.0, True)
+            opt.eval_acopf(self.x, delta, True)
+        elif fr:                    # the normal-phase data push was done at the start of this round
+            opt.update(self.x, self.f, self.df, self.E, self.dE, delta, True)
         p, lam, mu_u, mu_l, slack, status = opt.solve_extract()
+        self.lp_solves[sel] += 1
         info = getattr(opt, "last_info", None) or []
         self.lp_iterations += int(sum(i.get("iterations") or 0 for i in info))
         return [np.atleast_2d(a) if np.ndim(a) < 2 else a for a in (p, lam, mu_u, mu_l)] + [slack, np.atleast_1d(status)]
 
+    def _finish(self):
+        for s, pr in enumerate(self.problems):
+            self.obj_val[s] = pr.eval_f(self.x[s])
+
+
+class SlpLSBatch(_SlpBatch):
+    """B independent line-search SLP solves in lock-step (see ``_SlpBatch``): every round is one `update`, the KKT
+    reductions, one sub-LP batch solve (two when some scenarios are in feasibility restoration), and one batched merit
+    evaluation per backtracking round.  Per scenario the control flow is exactly ``SlpLS.run`` (reference
+    ``slp_line_search.jl:78-215``) — a scenario that terminates simply stops moving while the others go on.
+
+    ``device_evaluator=True`` (ACOPF scenarios of one network, B200 engine): the NLP callbacks are not called at all —
+    f, g and the Jacobian are evaluated by the device-side ACOPF evaluator (``SubLp.eval_acopf``) and every
+    backtracking trial is one ``SubLp.acopf_trial`` call for the whole batch."""
+
+    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
+        super().__init__(problems, parameters, device_evaluator)
+        self.alpha = np.zeros(self.B)
+
     def run(self):
         o = self.options
         B = self.B
-        for s, pr in enumerate(self.problems):                              # slp_line_search.jl:96-105
-            lo = pr.x_L > -INF
-            self.x[s][lo] = np.maximum(self.x[s][lo], pr.x_L[lo])
-            up = pr.x_U > -INF
-            self.x[s][up] = np.minimum(self.x[s][up], pr.x_U[up])
+        self._clip_starts()
         if self.optimizer is None:
             self.optimizer = self._instantiate()
         opt = self.optimizer
@@ -581,6 +618,7 @@ class SlpLSBatch:
             self.dual_infeas[run] = np.atleast_1d(opt.kt_residuals(self.lam, self.mult_x_U, self.mult_x_L))[run]
             self.compl[run] = np.atleast_1d(opt.norm_complementarity(self.lam))[run]
             need = {False: self.running & ~self.fr, True: self.running & self.fr}
+            self.two_phase_rounds += int(need[False].any() and need[True].any())
             status = np.zeros(B, dtype=np.int64)
             phi0 = np.zeros(B)
             deriv = np.zeros(B)
@@ -588,7 +626,7 @@ class SlpLSBatch:
                 sel = need[fr]
                 if not sel.any():
                     continue
-                p, lam, mu_u, mu_l, slack, st = self._solve_phase(fr, sel)
+                p, lam, mu_u, mu_l, slack, st = self._solve_phase(fr, sel, 1000.0)
                 idx = np.nonzero(sel)[0]
                 self.p[idx], self.lam[idx], self.mult_x_U[idx], self.mult_x_L[idx] = p[idx], lam[idx], mu_u[idx], mu_l[idx]
                 status[idx] = st[idx]
@@ -640,8 +678,7 @@ class SlpLSBatch:
                     continue
                 self.x[s] = self.x[s] + self.alpha[s] * self.p[s]
                 self.iter[s] += 1
-        for s, pr in enumerate(self.problems):
-            self.obj_val[s] = pr.eval_f(self.x[s])
+        self._finish()
         return self
 
     def _line_search(self, fr, idx, phi0, deriv):
@@ -680,3 +717,159 @@ class SlpLSBatch:
                         self.alpha[s] *= o.tau
                 else:
                     searching[s] = False
+
+
+class SlpTRBatch(_SlpBatch):
+    """B independent trust-region SLP solves in lock-step (see ``_SlpBatch``).  Per scenario the control flow is
+    exactly ``SlpTR.run`` (reference ``slp_trust_region.jl:87-206``) — a scenario that terminates simply stops moving
+    while the others go on.  Each scenario has its own radius ``delta[s]``, which also bounds its restoration LPs
+    (``sub_optimize!(slp, Δ)`` passes Δ in both phases).
+
+    A round is one evaluation + `update`, then for each phase that has running scenarios: one masked sub-LP batch
+    solve, ν, the KKT metrics with the new multipliers, and one batched ϕ(x + p), ϕ(x) and predicted reduction for
+    ``step_quality``.  All of a phase runs before the next phase's push, which overwrites the step and slacks on the
+    device that the merit calls read.
+
+    ``device_evaluator=True``: as for ``SlpLSBatch``; ϕ(x + p) is one ``SubLp.acopf_trial`` call for the batch."""
+
+    warm_start = 0      # as SlpTR._instantiate, so that a scenario's trajectory is the one of its single run
+
+    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
+        super().__init__(problems, parameters, device_evaluator)
+        self.delta = np.full(self.B, float(self.options.tr_size))           # slp_trust_region.jl:62-65
+        self.delta_max = 2.0
+        self.alpha1 = 0.1
+        self.alpha2 = 0.25
+
+    def run(self):                                                          # :87-206
+        self._clip_starts()
+        if self.optimizer is None:
+            self.optimizer = self._instantiate()
+        opt = self.optimizer
+        while self.running.any():
+            self.rounds += 1
+            if self.device_evaluator:
+                opt.eval_acopf(self.x, self.delta, False)
+                self.f[:] = opt.get_eval_f()
+            else:
+                for s in np.nonzero(self.running)[0]:
+                    self._eval(s)
+                opt.update(self.x, self.f, self.df, self.E, self.dE, self.delta, False)
+            need = {False: self.running & ~self.fr, True: self.running & self.fr}
+            self.two_phase_rounds += int(need[False].any() and need[True].any())
+            for fr in (False, True):
+                if need[fr].any():
+                    self._phase(fr, need[fr])
+        self._finish()
+        return self
+
+    def _phase(self, fr, sel):
+        """One iteration of ``SlpTR.run`` for the scenarios ``sel``, all in phase ``fr``."""
+        o = self.options
+        opt = self.optimizer
+        p, lam, mu_u, mu_l, _, status = self._solve_phase(fr, sel, self.delta)
+        idx = np.nonzero(sel)[0]
+        self.p[idx], self.lam[idx], self.mult_x_U[idx], self.mult_x_L[idx] = p[idx], lam[idx], mu_u[idx], mu_l[idx]
+        ok = idx[status[idx] == LP_OPTIMAL]
+        if len(ok):
+            self._compute_nu(fr, ok)
+            self.prim_infeas[ok] = np.atleast_1d(opt.norm_violations(None, None, INF))[ok]
+            self.dual_infeas[ok] = np.atleast_1d(opt.kt_residuals(self.lam, self.mult_x_U, self.mult_x_L))[ok]
+            self.compl[ok] = np.atleast_1d(opt.norm_complementarity(self.lam))[ok]
+        viol1 = None
+        quality = []
+        for s in idx:
+            st = status[s]
+            if st not in (LP_OPTIMAL, LP_INFEASIBLE):
+                if viol1 is None:   # 1-norm at x: E and x of this phase's push are g(x) and x
+                    viol1 = np.atleast_1d(opt.norm_violations(None, None, 1))
+                self.ret[s] = 6 if viol1[s] <= o.tol_infeas else -3           # see SlpTR.run
+                self.running[s] = False
+                continue
+            if st == LP_INFEASIBLE:
+                if fr:
+                    self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else 2
+                    self.running[s] = False
+                else:
+                    self.fr[s] = True                                       # re-solved next round, iter unchanged
+                continue
+            if self.prim_infeas[s] <= o.tol_infeas and self.compl[s] <= o.tol_residual and \
+                    float(np.max(np.abs(self.p[s]))) <= o.tol_direction:
+                if fr:
+                    self.fr[s] = False
+                    self.iter[s] += 1
+                    if self.iter[s] >= o.max_iter:                          # see SlpTR.run
+                        self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else -1
+                        self.running[s] = False
+                    continue
+                if self.dual_infeas[s] <= o.tol_residual:
+                    self.ret[s] = 0
+                    self.running[s] = False
+                    continue
+            if self.iter[s] >= o.max_iter:
+                self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else -1
+                self.running[s] = False
+                continue
+            quality.append(s)
+        if quality:
+            self._step_quality(fr, np.array(quality))
+
+    def _compute_nu(self, fr, ok):                                          # slp.jl:54-66
+        first = ok[self.iter[ok] == 1]
+        later = ok[self.iter[ok] != 1]
+        if len(first):
+            rn = np.atleast_2d(self.optimizer.row_norms())
+            df = None
+            if not fr:
+                df = self.optimizer.get_eval_df() if self.device_evaluator else self.df
+            for s in first:
+                norm_df = 1.0 if fr else float(np.linalg.norm(df[s]))
+                self.nu[s] = np.maximum(1.0, norm_df / np.maximum(1.0, rn[s]))
+        self.nu[later] = np.maximum(self.nu[later], np.abs(self.lam[later]))
+
+    def _step_quality(self, fr, idx):                                       # :213-251
+        """step_quality for the scenarios ``idx`` of phase ``fr``, then the step acceptance of run! (:195-204)."""
+        o = self.options
+        opt = self.optimizer
+        B = self.B
+        base = self.prim_infeas if fr else self.f
+        if self.device_evaluator:
+            phi1 = np.atleast_1d(opt.acopf_trial(np.ones(B), self.nu, self.prim_infeas if fr else None, fr))
+        else:
+            base1 = base.copy()
+            Et = self.E.copy()
+            for s in idx:
+                pr = self.problems[s]
+                xt = self.x[s] + self.p[s]
+                pr.eval_g(xt, Et[s])
+                if not fr:
+                    base1[s] = pr.eval_f(xt)
+            phi1 = np.atleast_1d(opt.merit_phi(base1, Et, self.nu, np.ones(B), fr))
+        phi0 = np.atleast_1d(opt.merit_phi(base, None, self.nu, np.zeros(B), fr))
+        phi_pre = np.atleast_1d(opt.merit_derivative(self.nu, fr))
+        for s in idx:
+            phi = phi1[s] - phi0[s]
+            if abs(phi_pre[s]) > 0.0:
+                rho = phi / phi_pre[s]
+                if rho <= 0:
+                    self.delta[s] *= self.alpha1
+                elif rho <= 0.25:
+                    self.delta[s] *= self.alpha2
+                elif rho > 0.75:
+                    self.delta[s] = min(2 * self.delta[s], self.delta_max)
+            else:
+                rho = -phi
+                if abs(phi) < 1.0e-8:
+                    if fr:
+                        self.fr[s] = False
+                    elif self.prim_infeas[s] <= o.tol_infeas:
+                        ok = self.dual_infeas[s] <= o.tol_residual and self.compl[s] <= o.tol_residual
+                        self.ret[s] = 0 if ok else 6
+                    else:
+                        self.ret[s] = 2
+            if self.ret[s] in (0, 2, 6):
+                self.running[s] = False
+                continue
+            if rho >= 0:
+                self.x[s] = self.x[s] + self.p[s]
+            self.iter[s] += 1

@@ -295,6 +295,13 @@ class SubLp:
         capi.check(self._lib.asm_slp_get_eval(self._h, capi.dptr(f), None, None, None))
         return f
 
+    def get_eval_df(self):
+        """df[batch, n] of the last evaluation (squeezed when ``batch == 1``): the gradient norm of the trust
+        region's first penalty (slp.jl:54-66)."""
+        df = np.empty((self.batch, self.n))
+        capi.check(self._lib.asm_slp_get_eval(self._h, None, capi.dptr(df), None, None))
+        return df[0] if self.batch == 1 and self._squeeze else df
+
     def get_eval(self):
         """(f, df, E, dE) of the last evaluation, ``[batch, ...]`` (squeezed when ``batch == 1``)."""
         B = self.batch
