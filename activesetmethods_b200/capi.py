@@ -116,6 +116,9 @@ SIGNATURES = {
     "asm_slp_ipm_timing": (C.c_int, [_VP, C.c_int32, c_double_p, c_double_p]),
     "asm_kkt_selftest": (C.c_int, [C.c_int32, C.c_int32, c_int64_p, c_int32_p, c_double_p, c_double_p, c_double_p,
                                    c_double_p, c_int64_p]),
+    "asm_kkt_device_selftest": (C.c_int, [C.c_int32, C.c_int32, c_int64_p, c_int32_p, C.c_int32, c_double_p,
+                                          c_double_p, c_double_p, c_int32_p, c_double_p, c_double_p, C.c_int32,
+                                          c_int64_p]),
 }
 
 _lib = None

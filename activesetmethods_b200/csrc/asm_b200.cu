@@ -13,6 +13,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <limits>
 #include <memory>
 #include <numeric>
 
@@ -1670,6 +1671,125 @@ int asm_kkt_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, con
         stats[5] = fanout_steps(S.bs_beg, S.bs_end, S.bmstep);
         stats[6] = longest;
         stats[7] = S.n_fchunks;
+    }
+    return ASM_OK;
+}
+
+// Device counterpart of asm_kkt_selftest: the same matrix, factorised and solved for a batch of scenarios by the
+// barrier engine's own symbolic analysis (IpmEngine::init), launch sequences and captured graphs, as LpSolver::solve_ipm
+// runs them.  Only the inputs differ: the pivots come straight from dx / ew (no regularisation) instead of k_ipm_diag.
+int asm_kkt_device_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, const int32_t *col_idx,
+                            int32_t batch, const double *vals, const double *dx, const double *ew,
+                            const int32_t *active, double *rhs_sol, double *inv_pivots, int32_t device,
+                            int64_t *stats) {
+    if (!row_ptr || n_cols <= 0 || n_rows < 0 || batch < 1 || !dx || (n_rows > 0 && !ew) || !rhs_sol)
+        return fail(ASM_E_INVALID, "bad argument");
+    if (row_ptr[0] != 0) return fail(ASM_E_INVALID, "row_ptr[0] != 0");
+    for (int i = 0; i < n_rows; ++i)
+        if (row_ptr[i + 1] < row_ptr[i]) return fail(ASM_E_INVALID, "row_ptr is not non-decreasing");
+    const int64_t nnz = row_ptr[n_rows];
+    if (nnz > INT32_MAX) return fail(ASM_E_INVALID, "more than 2^31 - 1 entries");
+    if (nnz > 0 && (!col_idx || !vals)) return fail(ASM_E_INVALID, "null matrix");
+    for (int64_t q = 0; q < nnz; ++q)
+        if (col_idx[q] < 0 || col_idx[q] >= n_cols) return fail(ASM_E_INVALID, "column index out of range");
+    const int ndev = asm_device_count();
+    if (ndev == 0) return fail(ASM_E_CUDA, "no CUDA device: this library has no CPU fallback");
+    if (device < 0 || device >= ndev) return fail(ASM_E_INVALID, "device index out of range");
+    ASM_CK(cudaSetDevice(device));
+
+    struct Stream {   // destroyed after the engine, which is declared below it
+        cudaStream_t s = nullptr;
+        ~Stream() {
+            if (s) cudaStreamDestroy(s);
+        }
+    } stream;
+    ASM_CK(cudaStreamCreateWithFlags(&stream.s, cudaStreamNonBlocking));
+    const cudaStream_t st = stream.s;
+    const int n = n_cols, m = n_rows, B = pad_batch(batch);
+    std::vector<int> rp(m + 1), ci(nnz);
+    for (int i = 0; i <= m; ++i) rp[i] = (int)row_ptr[i];
+    for (int64_t q = 0; q < nnz; ++q) ci[q] = col_idx[q];
+    IpmEngine E;
+    ASM_TRY(E.init(n, m, rp, ci, B));
+    const int N = E.sym.N;
+    const std::vector<int> &inv = E.sym.inv;
+
+    // element-major device layout v[i * B + s].  Padding lanes carry NaN: a kernel that mixes lanes spreads it
+    const double nan = std::numeric_limits<double>::quiet_NaN();
+    std::vector<double> hA((size_t)std::max<int64_t>(nnz, 1) * B, nan), hd((size_t)N * B, nan), hv((size_t)N * B, nan);
+    std::vector<ScenState> hst(B);
+    for (int s = 0; s < B; ++s) hst[s].status = s >= batch ? ASM_LP_OPTIMAL : (active && !active[s] ? ASM_LP_SKIPPED : -1);
+    for (int s = 0; s < batch; ++s) {
+        for (int64_t q = 0; q < nnz; ++q) hA[q * B + s] = vals[(int64_t)s * nnz + q];
+        for (int j = 0; j < n; ++j) hd[(size_t)inv[j] * B + s] = -dx[(int64_t)s * n + j];
+        for (int i = 0; i < m; ++i) hd[(size_t)inv[n + i] * B + s] = ew[(int64_t)s * m + i];
+        for (int k = 0; k < N; ++k) hv[(size_t)k * B + s] = rhs_sol[(int64_t)s * N + k];
+    }
+    std::vector<double> hi(hd.size());
+    for (size_t e = 0; e < hd.size(); ++e) hi[e] = 1.0 / hd[e];
+    DBuf<double> A;
+    DBuf<ScenState> state;
+    ASM_TRY(A.alloc(hA.size()));
+    ASM_TRY(state.alloc(B));
+    double *vec = E.kktv[1].p;
+    ASM_CK(cudaMemcpyAsync(A.p, hA.data(), hA.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    ASM_CK(cudaMemcpyAsync(state.p, hst.data(), hst.size() * sizeof(ScenState), cudaMemcpyHostToDevice, st));
+    ASM_CK(cudaMemcpyAsync(E.diag0.p, hd.data(), hd.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    ASM_CK(cudaMemcpyAsync(E.invd.p, hi.data(), hi.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+    ASM_CK(cudaMemcpyAsync(vec, hv.data(), hv.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+
+    LpView v = {};   // what k_kkt_scatter and the step kernels read
+    v.n = n;
+    v.m = m;
+    v.B = B;
+    v.A = A.p;
+    v.state = state.p;
+    ASM_TRY(E.capture(st, &E.g_factor, E.launches_factor, [&](int64_t &c) { E.enqueue_factor(v, st, c); }));
+    ASM_TRY(E.capture(st, &E.g_solve_sol, E.launches_solve, [&](int64_t &c) { E.enqueue_solve(v, vec, st, c); }));
+    ASM_CK(cudaGraphLaunch(E.g_factor, st));
+    ASM_CK(cudaGraphLaunch(E.g_solve_sol, st));
+    ASM_CK(cudaMemcpyAsync(hv.data(), vec, hv.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    ASM_CK(cudaMemcpyAsync(hi.data(), E.invd.p, hi.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    const int nfm = E.sym.fmstep[E.sym.n_levels];
+    std::vector<KktRange> fm(nfm);
+    if (nfm) ASM_CK(cudaMemcpyAsync(fm.data(), E.fmchunk.p, nfm * sizeof(KktRange), cudaMemcpyDeviceToHost, st));
+    ASM_CK(cudaStreamSynchronize(st));
+    ASM_CK(cudaGetLastError());
+    for (int s = 0; s < batch; ++s)
+        for (int k = 0; k < N; ++k) {
+            rhs_sol[(int64_t)s * N + k] = hv[(size_t)k * B + s];
+            if (inv_pivots) inv_pivots[(int64_t)s * N + k] = hi[(size_t)inv[k] * B + s];
+        }
+    if (stats) {
+        const KktSymbolic &S = E.sym;
+        int64_t narrow = 0, wide = 0, narrow_split = 0, wide_multi = 0, longest = 0, capped = 0;
+        for (const KktPanel &P : S.panels) {
+            if (P.w > kSnSmall) {
+                ++wide;
+                wide_multi += P.nr > kPanelRowsWide;
+            } else {
+                ++narrow;
+            }
+        }
+        for (const KktPanelTask &t : S.ptasks) narrow_split += S.panels[t.panel].w <= kSnSmall && t.r0 > 0;
+        for (int l = 0; l < S.n_levels; ++l) longest = std::max<int64_t>(longest, S.fs_end[l] > S.fs_beg[l]);
+        for (const KktRange &r : fm) longest = std::max<int64_t>(longest, r.end - r.begin);
+        // launches whose grid-stride loops take a second pass: the capped grid has fewer threads (batch: warps) than
+        // single-term units (batch: four terms each) or multi-term chunks
+        auto count_capped = [&](const std::vector<int> &sb, const std::vector<int> &se, const std::vector<int> &ms) {
+            for (int l = 0; l < S.n_levels; ++l) {
+                const int multi = ms[l + 1] - ms[l], singles = se[l] - sb[l];
+                if (singles + multi == 0) continue;
+                const int64_t threads = (int64_t)E.level_grid(singles + multi, multi).x * (B == 1 ? kThreads : kWarps);
+                capped += std::max<int64_t>(B == 1 ? singles : (singles + 3) / 4, multi) > threads;
+            }
+        };
+        count_capped(S.fs_beg, S.fs_end, S.fmstep);
+        count_capped(S.ws_beg, S.ws_end, S.wmstep);
+        count_capped(S.bs_beg, S.bs_end, S.bmstep);
+        const int64_t out[10] = {S.nnzL, S.n_levels, narrow, wide, narrow_split, wide_multi, longest, capped,
+                                 E.launches_factor, E.launches_solve};
+        std::copy(out, out + 10, stats);
     }
     return ASM_OK;
 }

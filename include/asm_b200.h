@@ -267,6 +267,20 @@ int asm_slp_ipm_timing(asm_slp *h, int32_t reps, double *factor_ms, double *solv
  * step-kernel launches of each), longest chunk, chunks */
 int asm_kkt_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, const int32_t *col_idx, const double *vals,
                      const double *dx, const double *ew, double *rhs_sol, int64_t *stats);
+/* device self test of the barrier engine's numeric kernels: factorises, for each of `batch` scenarios sharing the
+ * m x n CSR pattern, [-diag(dx_s) K_s'; K_s diag(ew_s)] with the engine's captured factor graph and solves
+ * rhs_sol[s] with its captured substitution graph.  vals[batch][nnz], dx[batch][n_cols], ew[batch][n_rows],
+ * rhs_sol[batch][n_cols + n_rows] (node order: columns then rows; right-hand side in, solution out).
+ * active[batch] (NULL = all): masked scenarios are not live and their rhs_sol comes back unchanged.
+ * inv_pivots[batch][n_cols + n_rows] (may be NULL): 1/d of every node after the factorisation.
+ * stats[10] (may be NULL): nnz(L), steps, narrow panels (2 <= w <= 4), wide panels (w > 4), narrow row tasks that
+ * start below the first row (r0 > 0), wide panels with more than one row task, longest factor chunk, step launches
+ * whose grid-stride loops take a second pass (capped grid), launches per factorisation, per substitution pair.
+ * Reads ASM_IPM_SUPERNODE and ASM_NO_PDL like a handle.  ASM_E_CUDA without a device: there is no host fallback */
+int asm_kkt_device_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_ptr, const int32_t *col_idx,
+                            int32_t batch, const double *vals, const double *dx, const double *ew,
+                            const int32_t *active, double *rhs_sol, double *inv_pivots, int32_t device,
+                            int64_t *stats);
 
 /* Restrict the following solves of a batch to the scenarios with active[s] != 0 (active[batch]; NULL = all again).
  * A lock-step batch of SLP runs calls this every round: scenarios that have terminated, or that are in the other

@@ -43,6 +43,34 @@ def test_no_cpu_fallback(built_lib):
     assert e.value.code == capi.E_CUDA
 
 
+def test_kkt_device_selftest_arguments(built_lib):
+    """The device self test rejects bad arguments before it looks for a device, and without one it fails with
+    ASM_E_CUDA: its host twin is asm_kkt_selftest, not a fallback."""
+    import numpy as np
+    i64, i32, d = capi.c_int64_p, capi.c_int32_p, capi.dptr
+    rp = np.array([0, 2, 3], dtype=np.int64)
+    ci = np.array([0, 2, 1], dtype=np.int32)
+    vals, dx, ew = np.ones(3), np.ones(3), np.ones(2)
+    sol, stats = np.zeros(5), np.zeros(10, dtype=np.int64)
+
+    def call(n=3, m=2, rp=rp, ci=ci, batch=1, vals=vals, dx=dx, ew=ew, sol=sol, device=0):
+        return built_lib.asm_kkt_device_selftest(
+            n, m, None if rp is None else rp.ctypes.data_as(i64), None if ci is None else ci.ctypes.data_as(i32),
+            batch, d(vals), d(dx), d(ew), None, d(sol), None, device, stats.ctypes.data_as(i64))
+
+    bad = [dict(n=0), dict(m=-1), dict(batch=0), dict(rp=None), dict(ci=None), dict(vals=None), dict(dx=None),
+           dict(ew=None), dict(sol=None), dict(rp=np.array([1, 2, 3], dtype=np.int64)),
+           dict(rp=np.array([0, 3, 2], dtype=np.int64)), dict(ci=np.array([0, 3, 1], dtype=np.int32)),
+           dict(ci=np.array([0, -1, 1], dtype=np.int32))]
+    for kw in bad:
+        assert call(**kw) == capi.E_INVALID, kw
+    if built_lib.asm_device_count() > 0:
+        assert call(device=-1) == capi.E_INVALID
+    else:
+        assert call() == capi.E_CUDA
+        assert call(device=-1) == capi.E_CUDA
+
+
 def test_product_does_not_import_oracle():
     """Only tests/, smoke() and bench.py's cpu_baseline may touch oracle/."""
     pkg = os.path.join(ROOT, "activesetmethods_b200")
