@@ -6,21 +6,26 @@ here                              reference (relative to /root/reference)
 ================================  ==========================================================================
 ``Parameters``                    ``src/parameters.jl:1-29``
 ``Model`` / ``optimize``          ``src/model.jl:1-80`` (problem container, algorithm dispatch)
-``SlpLS``                         ``src/algorithms/slp_line_search.jl:4-261``
-``SlpTR``                         ``src/algorithms/slp_trust_region.jl:10-251``, ``src/algorithms/slp.jl:54-66``
+``SlpLSBatch``                    ``src/algorithms/slp_line_search.jl:78-261``
+``SlpTRBatch``                    ``src/algorithms/slp_trust_region.jl:62-251``, ``src/algorithms/slp.jl:54-66``
+``SlpLS`` / ``SlpTR``             ``SlpLS`` / ``SlpTR`` ``(model)``, ``run!``, the write-back into ``Model``
+                                  (``slp_line_search.jl:207-214``): the one-scenario batch
 ``STATUS``                        ``src/status.jl:2-22``
 ================================  ==========================================================================
 
-The NLP callbacks (``eval_f``, ``eval_grad_f``, ``eval_g``, ``eval_jac_g``) stay on the host exactly like the
-JuMP ``NLPEvaluator`` of the reference (``src/MOI_wrapper.jl:1047-1069``).  Per iteration the driver hands
-``x, f, df, E, dE`` to ``SubLp.sub_optimize`` (one H2D hand-over, assembly + bounds + PDHG on the device,
-one D2H read-back) and asks the device for the merit / KKT reductions.
+Each algorithm has one driver, the lock-step batch (``SlpLSBatch``, ``SlpTRBatch``); a single solve is its
+one-scenario case.  The NLP callbacks (``eval_f``, ``eval_grad_f``, ``eval_g``, ``eval_jac_g``) stay on the host
+exactly like the JuMP ``NLPEvaluator`` of the reference (``src/MOI_wrapper.jl:1047-1069``), unless the device-side
+ACOPF evaluator replaces them.  Per round the driver hands ``x, f, df, E, dE`` to ``SubLp.update`` (one H2D
+hand-over, assembly + bounds on the device), solves the sub-LPs with ``solve_extract`` and asks the device for the
+merit / KKT reductions.
 """
 from __future__ import annotations
 
 import math
 import time
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, replace
+from functools import partial
 
 import numpy as np
 
@@ -122,368 +127,21 @@ def optimize(model: Model):
     return model
 
 
-class _Slp:
-    def __init__(self, model: Model):
-        self.problem = model
-        self.options = model.parameters
-        n, m = model.n, model.m
-        self.x = model.x.copy()
-        self.p = np.zeros(n)
-        self.p_slack = np.zeros((m, 2))
-        self.lam = np.zeros(m)
-        self.mult_x_L = np.zeros(n)
-        self.mult_x_U = np.zeros(n)
-        self.f = 0.0
-        self.df = np.zeros(n)
-        self.E = np.zeros(m)
-        self.dE = np.zeros(len(model.j_str))
-        self.phi = INF
-        self.nu = np.zeros(m)
-        self.alpha = 1.0
-        self.directional_derivative = 0.0
-        self.prim_infeas = INF
-        self.dual_infeas = INF
-        self.compl = INF
-        self.feasibility_restoration = False
-        self.iter = 1
-        self.ret = -5
-        self.optimizer = None
-        self.lp_log = []        # (status, objective, restoration flag, PDHG iterations) per sub-LP
-        self.lp_time = 0.0
-        self.start_time = 0.0
-        self.record = None      # optional callable(slp, dict) invoked before every sub-LP (tests / benchmarks)
-
-    # slp.jl:186-191
-    def eval_functions(self):
-        pr = self.problem
-        self.f = pr.eval_f(self.x)
-        pr.eval_grad_f(self.x, self.df)
-        pr.eval_g(self.x, self.E)
-        pr.eval_jac_g(self.x, "eval", None, None, self.dE)
-
-    def _instantiate(self):
-        """slp.jl:24-37: lazy creation of the external optimizer with the problem skeleton."""
-        pr, o = self.problem, self.options
-        factory = o.external_optimizer
-        if factory == "B200LP":
-            # Line search: every sub-LP starts from the previous one's (p, lambda) -- the analogue of GLPK keeping
-            # its basis (one glp_prob per SLP run, slp.jl:24); it halves the PDHG work (case118: 1.03 M -> 0.51 M
-            # iterations for the same 14 SLP iterations).  Trust region: cold starts; there a warm start changes
-            # which minimiser of the (degenerate) restoration LPs is returned and the runs measured so far ended
-            # further from the optimum.  ``lp_options={"warm_start": ...}`` overrides either.
-            warm = 1 if o.algorithm == "Line Search" else 0
-            return SubLp(pr.n, pr.m, pr.j_str, pr.x_L, pr.x_U, pr.g_L, pr.g_U, batch=1, device=o.device,
-                         **{"warm_start": warm, **o.lp_options})
-        return factory(pr.n, pr.m, pr.j_str, pr.x_L, pr.x_U, pr.g_L, pr.g_U)
-
-    # slp.jl:23-47
-    def sub_optimize(self, delta=1000.0, updated=False):
-        """``updated``: the data push for this iterate has already been done by ``optimizer.update``."""
-        if self.optimizer is None:
-            self.optimizer = self._instantiate()
-        if self.record is not None:
-            self.record(self, dict(x=self.x.copy(), f=self.f, df=self.df.copy(), E=self.E.copy(),
-                                   dE=self.dE.copy(), delta=delta, fr=self.feasibility_restoration))
-        t0 = time.time()
-        if updated:
-            out = self.optimizer.solve_extract()
-        else:
-            out = self.optimizer.sub_optimize(self.x, self.f, self.df, self.E, self.dE, delta,
-                                              self.feasibility_restoration)
-        self.lp_time = time.time() - t0
-        info = self.optimizer.last_info[0] if getattr(self.optimizer, "last_info", None) else {}
-        self.lp_log.append((out[5], info.get("objective"), self.feasibility_restoration, info.get("iterations")))
-        return out
-
-    def clip_start(self):
-        pr = self.problem                                                   # slp_line_search.jl:96-105
-        lo = pr.x_L > -INF
-        self.x[lo] = np.maximum(self.x[lo], pr.x_L[lo])
-        up = pr.x_U > -INF                                                  # sic (SURVEY App. C-5)
-        self.x[up] = np.minimum(self.x[up], pr.x_U[up])
-
-    # slp.jl:79-115 — f / g at the trial point on the host (NLP evaluator), the m-length reduction on the GPU
-    def compute_phi(self, x, alpha, p):
-        pr = self.problem
-        if self.options.device_evaluator and alpha != 0.0:      # f and g at the trial point on the device
-            return self.optimizer.acopf_trial(alpha, self.nu, self.prim_infeas if self.feasibility_restoration else None,
-                                              self.feasibility_restoration)
-        xp = x + alpha * p
-        E = None if alpha == 0.0 else pr.eval_g(xp, np.zeros(pr.m))
-        if self.feasibility_restoration:
-            return self.optimizer.merit_phi(self.prim_infeas, E, self.nu, alpha, True)
-        base = self.f if (self.options.device_evaluator and alpha == 0.0) else pr.eval_f(xp)
-        return self.optimizer.merit_phi(base, E, self.nu, alpha, False)
-
-    # slp.jl:122-147
-    def compute_derivative(self):
-        return self.optimizer.merit_derivative(self.nu, self.feasibility_restoration)
-
-    def norm_violations(self, p=1):                                         # slp.jl:174-178
-        return self.optimizer.norm_violations(None, self.x, p) if self.optimizer is not None else \
-            _host_violations(self.problem, self.E, self.x, p)
-
-    def kt_residuals(self):                                                 # slp.jl:154
-        if self.optimizer is None:                                          # before the first LP: lambda = 0
-            return float(np.linalg.norm(self.df - self.mult_x_U - self.mult_x_L) /
-                         max(1.0, np.linalg.norm(self.df)))
-        return self.optimizer.kt_residuals(self.lam, self.mult_x_U, self.mult_x_L)
-
-    def norm_complementarity(self):                                         # slp.jl:161-166
-        if self.optimizer is None:
-            return 0.0
-        return self.optimizer.norm_complementarity(self.lam)
-
-    def finish(self):                                                       # slp_line_search.jl:207-214
-        pr = self.problem
-        pr.obj_val = pr.eval_f(self.x)
-        pr.status = int(self.ret)
-        pr.x[:] = self.x
-        if self.options.device_evaluator:      # the loop kept g on the device: one host evaluation for the write-back
-            pr.eval_g(self.x, self.E)
-        pr.g[:] = self.E
-        pr.mult_g[:] = self.lam
-        pr.mult_x_U[:] = self.mult_x_U
-        pr.mult_x_L[:] = self.mult_x_L
-        self.obj_val = pr.obj_val
-        self.status = pr.status
-
-    def _print(self, extra=""):
-        if self.options.OutputFlag:
-            print(f"{self.iter:6d}  {self.f: .8e}  {self.phi: .8e}  {self.directional_derivative: .4e}  "
-                  f"{float(np.max(np.abs(self.p))):.4e}  {self.alpha:.4e}  {self.prim_infeas:.4e}  "
-                  f"{self.dual_infeas:.4e}  {self.compl:.4e}  {self.lp_time:7.2f}{extra}")
-
-
-def _host_violations(pr, E, x, p):
-    viol = np.concatenate([
-        np.where(E > pr.g_U, E - pr.g_U, np.where(E < pr.g_L, pr.g_L - E, 0.0)),
-        np.where(x > pr.x_U, x - pr.x_U, np.where(x < pr.x_L, pr.x_L - x, 0.0))])
-    if len(viol) == 0:
-        return 0.0
-    return float(np.max(np.abs(viol))) if p == INF else float(np.linalg.norm(viol, p))
-
-
-class SlpLS(_Slp):
-    """Line-search SLP (slp_line_search.jl)."""
-
-    def compute_nu(self):                                                   # :251-261
-        if self.iter == 1:
-            self.nu = np.abs(self.lam)
-        else:
-            self.nu = np.maximum(self.nu, np.abs(self.lam))
-
-    def compute_alpha(self):                                                # :222-244
-        o = self.options
-        is_valid = True
-        self.alpha = 1.0
-        phi_x_p = self.compute_phi(self.x, self.alpha, self.p)
-        while phi_x_p > self.phi + o.eta * self.alpha * self.directional_derivative:
-            if self.alpha < o.min_alpha:
-                if self.feasibility_restoration:
-                    self.ret = -3
-                is_valid = False
-                break
-            self.alpha *= o.tau
-            phi_x_p = self.compute_phi(self.x, self.alpha, self.p)
-        return is_valid
-
-    def run(self):                                                          # :78-215
-        o = self.options
-        self.start_time = time.time()
-        self.clip_start()
-        self.iter = 1
-        if self.optimizer is None:
-            self.optimizer = self._instantiate()
-        dev_eval = bool(o.device_evaluator)
-        if dev_eval:
-            self.optimizer.attach_acopf(self.problem.source)
-        while True:
-            self.alpha = 0.0
-            # KKT metrics with the multipliers of the previous iteration (App. C-7); they need the
-            # Jacobian of *this* iterate on the device, which the update below provides
-            if dev_eval:
-                self.optimizer.eval_acopf(self.x, 1000.0, self.feasibility_restoration)
-                self.f = float(np.atleast_1d(self.optimizer.get_eval_f())[0])
-            else:
-                self.eval_functions()
-                self.optimizer.update(self.x, self.f, self.df, self.E, self.dE, 1000.0, self.feasibility_restoration)
-            self.prim_infeas = self.optimizer.norm_violations(None, None, INF)
-            self.dual_infeas = self.kt_residuals()
-            self.compl = self.norm_complementarity()
-            self.p, self.lam, self.mult_x_U, self.mult_x_L, self.p_slack, status = self.sub_optimize(1000.0, True)
-            if status not in (LP_OPTIMAL, LP_INFEASIBLE):
-                # Deviation from slp_line_search.jl:129, whose `slp.ret == -3` is a comparison, not an assignment: the
-                # run would end as -5 "Optimize_not_called" after a full solve.  -3 (Error_In_Step_Computation) is the
-                # evident intent.
-                self.ret = -3
-                if self.prim_infeas <= o.tol_infeas:
-                    self.ret = 6
-                break
-            elif status == LP_INFEASIBLE:
-                if self.feasibility_restoration:
-                    self.ret = 6 if self.prim_infeas <= o.tol_infeas else 2
-                    break
-                self.feasibility_restoration = True
-                continue
-            self.compute_nu()
-            self.phi = self.compute_phi(self.x, 0.0, self.p)
-            self.directional_derivative = self.compute_derivative()
-            is_valid_step = self.compute_alpha()
-            self._print()
-            if self.iter >= o.max_iter:
-                self.ret = -1
-                if self.prim_infeas <= o.tol_infeas:
-                    self.ret = 6
-                break
-            if (self.prim_infeas <= o.tol_infeas and self.compl <= o.tol_residual) or \
-                    float(np.max(np.abs(self.p))) <= o.tol_direction:
-                if self.feasibility_restoration:
-                    self.feasibility_restoration = False
-                    self.iter += 1
-                    continue
-                elif self.dual_infeas <= o.tol_residual:
-                    self.ret = 0
-                    break
-            if not is_valid_step:
-                if self.ret == -3:
-                    self.ret = 6 if self.prim_infeas <= o.tol_infeas else 2
-                    break
-                else:
-                    self.feasibility_restoration = True
-                self.iter += 1
-                continue
-            self.x = self.x + self.alpha * self.p
-            self.iter += 1
-        self.finish()
-        return self
-
-
-class SlpTR(_Slp):
-    """Trust-region SLP (slp_trust_region.jl)."""
-
-    def __init__(self, model):
-        super().__init__(model)
-        self.delta = self.options.tr_size                                   # :62-65
-        self.delta_max = 2.0
-        self.alpha1 = 0.1
-        self.alpha2 = 0.25
-
-    def compute_nu(self):                                                   # slp.jl:54-66
-        if self.iter == 1:
-            if self.feasibility_restoration:
-                norm_df = 1.0
-            else:
-                df = self.optimizer.get_eval_df() if self.options.device_evaluator else self.df
-                norm_df = float(np.linalg.norm(df))
-            rn = self.optimizer.row_norms()
-            self.nu = np.maximum(1.0, norm_df / np.maximum(1.0, rn))
-        else:
-            self.nu = np.maximum(self.nu, np.abs(self.lam))
-
-    def step_quality(self):                                                 # :213-251
-        o = self.options
-        self.phi = self.compute_phi(self.x, 1.0, self.p) - self.compute_phi(self.x, 0.0, self.p)
-        phi_pre = self.compute_derivative()
-        if abs(phi_pre) > 0.0:
-            rho = self.phi / phi_pre
-            if rho <= 0:
-                self.delta *= self.alpha1
-            elif rho <= 0.25:
-                self.delta *= self.alpha2
-            elif rho > 0.75:
-                self.delta = min(2 * self.delta, self.delta_max)
-        else:
-            rho = -self.phi
-            if abs(self.phi) < 1.0e-8:
-                if self.feasibility_restoration:
-                    self.feasibility_restoration = False
-                else:
-                    if self.prim_infeas <= o.tol_infeas:
-                        if self.dual_infeas <= o.tol_residual and self.compl <= o.tol_residual:
-                            self.ret = 0
-                        else:
-                            self.ret = 6
-                    else:
-                        self.ret = 2
-        return rho
-
-    def run(self):                                                          # :87-206
-        o = self.options
-        pr = self.problem
-        self.start_time = time.time()
-        self.clip_start()
-        self.iter = 1
-        dev_eval = bool(o.device_evaluator)
-        if dev_eval:
-            if self.optimizer is None:
-                self.optimizer = self._instantiate()
-            self.optimizer.attach_acopf(self.problem.source)
-        while True:
-            if dev_eval:
-                self.optimizer.eval_acopf(self.x, self.delta, self.feasibility_restoration)
-                self.f = float(np.atleast_1d(self.optimizer.get_eval_f())[0])
-                out = self.sub_optimize(self.delta, True)
-            else:
-                self.eval_functions()
-                out = self.sub_optimize(self.delta)
-            self.p, self.lam, self.mult_x_U, self.mult_x_L, self.p_slack, status = out
-            if status not in (LP_OPTIMAL, LP_INFEASIBLE):
-                self.ret = -3                      # same deviation as in SlpLS.run (slp_trust_region.jl:131)
-                # g(x) of this iteration: on the device with the device evaluator (E = None), else from the callback
-                E = None if dev_eval else pr.eval_g(self.x, np.zeros(pr.m))
-                if self.optimizer.norm_violations(E, self.x, 1) <= o.tol_infeas:
-                    self.ret = 6
-                break
-            elif status == LP_INFEASIBLE:
-                if self.feasibility_restoration:
-                    self.ret = 6 if self.prim_infeas <= o.tol_infeas else 2
-                    break
-                self.feasibility_restoration = True
-                continue
-            self.compute_nu()
-            self.prim_infeas = self.optimizer.norm_violations(None, None, INF)
-            self.dual_infeas = self.kt_residuals()
-            self.compl = self.norm_complementarity()
-            if self.prim_infeas <= o.tol_infeas and self.compl <= o.tol_residual and \
-                    float(np.max(np.abs(self.p))) <= o.tol_direction:
-                if self.feasibility_restoration:
-                    self.feasibility_restoration = False
-                    self.iter += 1
-                    # Deviation from slp_trust_region.jl:163-170, which `continue`s here without ever reaching
-                    # its max_iter test: once the trust region has collapsed (delta ~ 1e-7) at a point that is
-                    # feasible to tolerance but whose linearisation is infeasible inside the tiny box, the
-                    # reference alternates normal LP (INFEASIBLE) / restoration LP forever.  Stop as its own
-                    # max_iter branch (:177-183) would.
-                    if self.iter >= o.max_iter:
-                        self.ret = 6 if self.prim_infeas <= o.tol_infeas else -1
-                        break
-                    continue
-                elif self.dual_infeas <= o.tol_residual:
-                    self.ret = 0
-                    break
-            if self.iter >= o.max_iter:
-                self.ret = -1
-                if self.prim_infeas <= o.tol_infeas:
-                    self.ret = 6
-                break
-            rho = self.step_quality()
-            self._print(f"  rho {rho: .3e} delta {self.delta:.3e}")
-            if self.ret in (0, 2, 6):
-                break
-            if rho >= 0:
-                self.x = self.x + self.p
-            self.iter += 1
-        self.finish()
-        return self
-
-
 class _SlpBatch:
     """B independent SLP solves that share one Jacobian pattern (load scenarios of one network, BASELINE config 5),
     advanced in lock-step so that every round is one batched call of each operation of the device hot path.
-    ``problems`` are objects with the ``Model.from_problem`` interface.  Subclasses give the round (``run``) and
-    ``warm_start``, the engine's warm-start flag (see ``_Slp._instantiate``)."""
+    ``problems`` are objects with the ``Model.from_problem`` interface, or ``Model`` s (which start from ``model.x``).
+    Subclasses give the round (``run``) and ``warm_start``, the B200 engine's warm-start flag.
 
+    ``record``: optional ``callable(driver, dict)``, called before every sub-LP solve for each scenario solved, with
+    that scenario's linearisation (``x, f, df, E, dE, delta, fr``).  ``lp_log[s]`` lists (status, objective,
+    restoration flag, iterations) of every sub-LP solved for scenario ``s``."""
+
+    # Line search: every sub-LP starts from the previous one's (p, lambda) -- the analogue of GLPK keeping its basis
+    # (one glp_prob per SLP run, slp.jl:24); it halves the PDHG work (case118: 1.03 M -> 0.51 M iterations for the
+    # same 14 SLP iterations).  Trust region: cold starts; there a warm start changes which minimiser of the
+    # (degenerate) restoration LPs is returned and the runs measured so far ended further from the optimum.
+    # ``lp_options={"warm_start": ...}`` overrides either.
     warm_start = 1
 
     def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
@@ -496,7 +154,7 @@ class _SlpBatch:
             if pr.n != self.n or pr.m != self.m or not np.array_equal(pr.j_str, p0.j_str):
                 raise ValueError("batched scenarios must share the Jacobian pattern")
         B, n, m = self.B, self.n, self.m
-        self.x = np.array([np.array(pr.x0, dtype=float) for pr in self.problems])
+        self.x = np.array([np.array(pr.x if isinstance(pr, Model) else pr.x0, dtype=float) for pr in self.problems])
         self.f = np.zeros(B)
         self.df = np.zeros((B, n))
         self.E = np.zeros((B, m))
@@ -517,8 +175,11 @@ class _SlpBatch:
         self.rounds = 0
         self.two_phase_rounds = 0       # rounds with scenarios in both phases: two sub-LP batch solves
         self.lp_solves = np.zeros(B, dtype=np.int64)
+        self.lp_log = [[] for _ in range(B)]
         self.lp_iterations = 0
+        self.lp_time = 0.0
         self.optimizer = None
+        self.record = None
 
     def _instantiate(self):
         o = self.options
@@ -530,16 +191,17 @@ class _SlpBatch:
             opt._squeeze = False
             if self.device_evaluator:
                 # the device evaluator holds ONE network: every scenario must share everything but its loads (which
-                # only enter g_L / g_U)
-                n0 = prs[0].net
-                for k, pr in enumerate(prs[1:], 1):
+                # only enter g_L / g_U).  A Model hands over the problem it was built from.
+                acopf = [pr.source if isinstance(pr, Model) else pr for pr in prs]
+                n0 = acopf[0].net
+                for k, pr in enumerate(acopf[1:], 1):
                     for name in ("f_bus", "t_bus", "br_r", "br_x", "br_b", "tap", "shift", "gs", "bs", "cost2", "cost1",
                                  "cost0", "gen_bus", "dc_loss1"):
                         if not np.array_equal(getattr(pr.net, name), getattr(n0, name)):
                             raise ValueError(f"device_evaluator: scenario {k} differs from scenario 0 in network.{name}")
                     if pr.net.ref_bus != n0.ref_bus:
                         raise ValueError(f"device_evaluator: scenario {k} has another reference bus")
-                opt.attach_acopf(prs[0])
+                opt.attach_acopf(acopf[0])
             return opt
         if self.device_evaluator:
             raise ValueError("device_evaluator needs the B200 engine")
@@ -571,11 +233,28 @@ class _SlpBatch:
             opt.eval_acopf(self.x, delta, True)
         elif fr:                    # the normal-phase data push was done at the start of this round
             opt.update(self.x, self.f, self.df, self.E, self.dE, delta, True)
+        idx = np.nonzero(sel)[0]
+        if self.record is not None:
+            radius = np.broadcast_to(delta, (self.B,))
+            for s in idx:
+                self.record(self, dict(x=self.x[s].copy(), f=float(self.f[s]), df=self.df[s].copy(),
+                                       E=self.E[s].copy(), dE=self.dE[s].copy(), delta=float(radius[s]), fr=fr))
+        t0 = time.time()
         p, lam, mu_u, mu_l, slack, status = opt.solve_extract()
+        self.lp_time = time.time() - t0
+        status = np.atleast_1d(status)
         self.lp_solves[sel] += 1
-        info = getattr(opt, "last_info", None) or []
+        info = getattr(opt, "last_info", None) or [{}] * self.B
         self.lp_iterations += int(sum(i.get("iterations") or 0 for i in info))
-        return [np.atleast_2d(a) if np.ndim(a) < 2 else a for a in (p, lam, mu_u, mu_l)] + [slack, np.atleast_1d(status)]
+        for s in idx:
+            self.lp_log[s].append((int(status[s]), info[s].get("objective"), fr, info[s].get("iterations")))
+        return [np.atleast_2d(a) if np.ndim(a) < 2 else a for a in (p, lam, mu_u, mu_l)] + [slack, status]
+
+    def _print(self, s, phi, derivative, alpha, extra=""):
+        if self.options.OutputFlag:
+            print(f"{s:4d}  {self.iter[s]:6d}  {self.f[s]: .8e}  {phi: .8e}  {derivative: .4e}  "
+                  f"{float(np.max(np.abs(self.p[s]))):.4e}  {alpha:.4e}  {self.prim_infeas[s]:.4e}  "
+                  f"{self.dual_infeas[s]:.4e}  {self.compl[s]:.4e}  {self.lp_time:7.2f}{extra}")
 
     def _finish(self):
         for s, pr in enumerate(self.problems):
@@ -585,8 +264,9 @@ class _SlpBatch:
 class SlpLSBatch(_SlpBatch):
     """B independent line-search SLP solves in lock-step (see ``_SlpBatch``): every round is one `update`, the KKT
     reductions, one sub-LP batch solve (two when some scenarios are in feasibility restoration), and one batched merit
-    evaluation per backtracking round.  Per scenario the control flow is exactly ``SlpLS.run`` (reference
-    ``slp_line_search.jl:78-215``) — a scenario that terminates simply stops moving while the others go on.
+    evaluation per backtracking round.  Per scenario the control flow is exactly ``run!`` of the reference
+    (``slp_line_search.jl:78-215``) — a scenario that terminates simply stops moving while the others go on.  A
+    single solve (``SlpLS``) is the one-scenario batch.
 
     ``device_evaluator=True`` (ACOPF scenarios of one network, B200 engine): the NLP callbacks are not called at all —
     f, g and the Jacobian are evaluated by the device-side ACOPF evaluator (``SubLp.eval_acopf``) and every
@@ -644,7 +324,10 @@ class SlpLSBatch(_SlpBatch):
             for s in run:
                 st = status[s]
                 if st not in (LP_OPTIMAL, LP_INFEASIBLE):
-                    self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else -3   # see SlpLS.run
+                    # Deviation from slp_line_search.jl:129, whose `slp.ret == -3` is a comparison, not an assignment:
+                    # the run would end as -5 "Optimize_not_called" after a full solve.  -3 (Error_In_Step_Computation)
+                    # is the evident intent.
+                    self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else -3
                     self.running[s] = False
                     continue
                 if st == LP_INFEASIBLE:
@@ -654,6 +337,7 @@ class SlpLSBatch(_SlpBatch):
                     else:
                         self.fr[s] = True                                   # re-solved next round, iter unchanged
                     continue
+                self._print(s, phi0[s], deriv[s], self.alpha[s])
                 if self.iter[s] >= o.max_iter:
                     self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else -1
                     self.running[s] = False
@@ -721,9 +405,9 @@ class SlpLSBatch(_SlpBatch):
 
 class SlpTRBatch(_SlpBatch):
     """B independent trust-region SLP solves in lock-step (see ``_SlpBatch``).  Per scenario the control flow is
-    exactly ``SlpTR.run`` (reference ``slp_trust_region.jl:87-206``) — a scenario that terminates simply stops moving
-    while the others go on.  Each scenario has its own radius ``delta[s]``, which also bounds its restoration LPs
-    (``sub_optimize!(slp, Δ)`` passes Δ in both phases).
+    exactly ``run!`` of the reference (``slp_trust_region.jl:87-206``) — a scenario that terminates simply stops moving
+    while the others go on.  A single solve (``SlpTR``) is the one-scenario batch.  Each scenario has its own radius
+    ``delta[s]``, which also bounds its restoration LPs (``sub_optimize!(slp, Δ)`` passes Δ in both phases).
 
     A round is one evaluation + `update`, then for each phase that has running scenarios: one masked sub-LP batch
     solve, ν, the KKT metrics with the new multipliers, and one batched ϕ(x + p), ϕ(x) and predicted reduction for
@@ -732,7 +416,7 @@ class SlpTRBatch(_SlpBatch):
 
     ``device_evaluator=True``: as for ``SlpLSBatch``; ϕ(x + p) is one ``SubLp.acopf_trial`` call for the batch."""
 
-    warm_start = 0      # as SlpTR._instantiate, so that a scenario's trajectory is the one of its single run
+    warm_start = 0      # see _SlpBatch.warm_start
 
     def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
         super().__init__(problems, parameters, device_evaluator)
@@ -764,7 +448,7 @@ class SlpTRBatch(_SlpBatch):
         return self
 
     def _phase(self, fr, sel):
-        """One iteration of ``SlpTR.run`` for the scenarios ``sel``, all in phase ``fr``."""
+        """One iteration of ``run!`` (:117-205) for the scenarios ``sel``, all in phase ``fr``."""
         o = self.options
         opt = self.optimizer
         p, lam, mu_u, mu_l, _, status = self._solve_phase(fr, sel, self.delta)
@@ -783,7 +467,7 @@ class SlpTRBatch(_SlpBatch):
             if st not in (LP_OPTIMAL, LP_INFEASIBLE):
                 if viol1 is None:   # 1-norm at x: E and x of this phase's push are g(x) and x
                     viol1 = np.atleast_1d(opt.norm_violations(None, None, 1))
-                self.ret[s] = 6 if viol1[s] <= o.tol_infeas else -3           # see SlpTR.run
+                self.ret[s] = 6 if viol1[s] <= o.tol_infeas else -3           # see SlpLSBatch.run (:131)
                 self.running[s] = False
                 continue
             if st == LP_INFEASIBLE:
@@ -798,7 +482,12 @@ class SlpTRBatch(_SlpBatch):
                 if fr:
                     self.fr[s] = False
                     self.iter[s] += 1
-                    if self.iter[s] >= o.max_iter:                          # see SlpTR.run
+                    # Deviation from slp_trust_region.jl:163-170, which `continue`s here without ever reaching its
+                    # max_iter test: once the trust region has collapsed (delta ~ 1e-7) at a point that is feasible to
+                    # tolerance but whose linearisation is infeasible inside the tiny box, the reference alternates
+                    # normal LP (INFEASIBLE) / restoration LP forever.  Stop as its own max_iter branch (:177-183)
+                    # would.
+                    if self.iter[s] >= o.max_iter:
                         self.ret[s] = 6 if self.prim_infeas[s] <= o.tol_infeas else -1
                         self.running[s] = False
                     continue
@@ -867,9 +556,112 @@ class SlpTRBatch(_SlpBatch):
                         self.ret[s] = 0 if ok else 6
                     else:
                         self.ret[s] = 2
+            self._print(s, phi, phi_pre[s], 1.0, f"  rho {rho: .3e} delta {self.delta[s]:.3e}")
             if self.ret[s] in (0, 2, 6):
                 self.running[s] = False
                 continue
             if rho >= 0:
                 self.x[s] = self.x[s] + self.p[s]
             self.iter[s] += 1
+
+
+class _OneLp:
+    """A single-LP ``external_optimizer`` -- the reference's one-LP optimizer: ``factory(n, m, j_str, x_L, x_U, g_L,
+    g_U)`` with 1-D bounds, scalar results and 1-D arrays -- presented to the batch drivers as a batch of one: every
+    argument loses its leading axis and every result gains one.  It has no ``set_active``: there is nothing to mask."""
+
+    def __init__(self, factory, n, m, j_str, x_L, x_U, g_L, g_U, batch):
+        self.lp = factory(n, m, j_str, x_L[0], x_U[0], g_L[0], g_U[0])
+
+    @property
+    def last_info(self):
+        return self.lp.last_info
+
+    def _call(self, name, *args):
+        return getattr(self.lp, name)(*(a[0] if np.ndim(a) else a for a in args))
+
+    def _batched(self, name, *args):
+        return np.asarray(self._call(name, *args))[None]
+
+    def update(self, *args):
+        self._call("update", *args)
+
+    def solve_extract(self):
+        return tuple(np.asarray(a)[None] for a in self.lp.solve_extract())
+
+    def norm_violations(self, *args):
+        return self._batched("norm_violations", *args)
+
+    def kt_residuals(self, *args):
+        return self._batched("kt_residuals", *args)
+
+    def norm_complementarity(self, *args):
+        return self._batched("norm_complementarity", *args)
+
+    def row_norms(self):
+        return self._batched("row_norms")
+
+    def merit_phi(self, *args):
+        return self._batched("merit_phi", *args)
+
+    def merit_derivative(self, *args):
+        return self._batched("merit_derivative", *args)
+
+
+class _Slp:
+    """A single SLP solve of ``model`` (``SlpLS(model)`` / ``SlpTR(model)``, slp_line_search.jl:4-71,
+    slp_trust_region.jl:10-80): ``run`` solves it as the one-scenario batch of ``_batch``, copies scenario 0 back
+    into this object (scalars and 1-D arrays) and writes the result into the model (slp_line_search.jl:207-214).
+    ``record`` (see ``_SlpBatch``) and the ``_inputs`` may be set between construction and ``run``."""
+
+    _inputs = ("x",)
+
+    def __init__(self, model: Model):
+        self.problem = model
+        self.options = model.parameters
+        self.x = model.x.copy()
+        self.record = None
+        self.optimizer = None
+
+    def run(self):
+        pr, o = self.problem, self.options
+        if o.external_optimizer != "B200LP":
+            o = replace(o, external_optimizer=partial(_OneLp, o.external_optimizer))
+        b = self._batch([pr], o, device_evaluator=o.device_evaluator)
+        for name in self._inputs:
+            getattr(b, name)[0] = getattr(self, name)
+        b.record = self.record
+        b.run()
+        for name in self._inputs + ("p", "lam", "mult_x_U", "mult_x_L", "nu", "ret", "iter", "f", "prim_infeas",
+                                    "dual_infeas", "compl", "obj_val"):
+            v = getattr(b, name)[0]
+            setattr(self, name, v.item() if v.ndim == 0 else v)
+        self.feasibility_restoration = bool(b.fr[0])
+        self.lp_log = b.lp_log[0]
+        self.optimizer = b.optimizer
+        pr.obj_val = self.obj_val
+        pr.status = self.status = self.ret
+        pr.x[:] = self.x
+        pr.eval_g(self.x, pr.g)
+        pr.mult_g[:] = self.lam
+        pr.mult_x_U[:] = self.mult_x_U
+        pr.mult_x_L[:] = self.mult_x_L
+        return self
+
+
+class SlpLS(_Slp):
+    """Line-search SLP (slp_line_search.jl) on one model: the one-scenario ``SlpLSBatch``."""
+
+    _batch = SlpLSBatch
+
+
+class SlpTR(_Slp):
+    """Trust-region SLP (slp_trust_region.jl) on one model: the one-scenario ``SlpTRBatch``, with the radius
+    ``delta`` as a second input."""
+
+    _batch = SlpTRBatch
+    _inputs = ("x", "delta")
+
+    def __init__(self, model: Model):
+        super().__init__(model)
+        self.delta = self.options.tr_size                                   # :62-65

@@ -124,21 +124,23 @@ def test_trust_region_on_device_evaluator(gpu):
     """SlpTR on case9 with the device-side evaluator: every ϕ(x + p) checked against the host callbacks as above; the
     same status and iteration count as the host-callback run, and the objective within the reference's suite
     tolerance of it and of the public optimum 5296.69 (the trajectories part as described for the batch)."""
-    from activesetmethods_b200.slp import Model, SlpTR
+    from activesetmethods_b200.slp import Model, SlpTR, SlpTRBatch
+    checked = []
+
+    class CheckedBatch(SlpTRBatch):
+        def _step_quality(self, fr, idx):
+            _check_trial(checked, self.optimizer, self.problems, self.x, self.p, self.nu, self.prim_infeas, fr, idx)
+            super()._step_quality(fr, idx)
 
     class Checked(SlpTR):
-        def step_quality(self):
-            _check_trial(self.checked, self.optimizer, [self.problem], self.x[None], self.p[None], self.nu[None],
-                         np.array([self.prim_infeas]), self.feasibility_restoration, [0])
-            return super().step_quality()
+        _batch = CheckedBatch
 
     host = SlpTR(Model.from_problem(acopf.AcopfModel(acopf.case9()), _params())).run()
     dev = Checked(Model.from_problem(acopf.AcopfModel(acopf.case9()), _params(device_evaluator=True)))
-    dev.checked = []
     dev.run()
     print(f"case9 TR: host ret {host.ret} iter {host.iter} obj {host.obj_val:.10f}; "
           f"device ret {dev.ret} iter {dev.iter} obj {dev.obj_val:.10f}")
-    _assert_trials(dev.checked)
+    _assert_trials(checked)
     assert dev.ret == host.ret and dev.iter == host.iter
     assert abs(dev.obj_val - host.obj_val) <= 1e-2 * abs(host.obj_val)
     assert abs(dev.obj_val - 5296.69) <= 1e-2 * 5296.69

@@ -20,10 +20,12 @@ slp = (SlpLS if alg == "Line Search" else SlpTR)(mdl)
 t0 = time.time()
 
 
-def progress(s_, d):
-    if s_.lp_log:
-        print(f"  [{time.time() - t0:7.1f}s] SLP it {s_.iter} last LP {s_.lp_log[-1]} prim_infeas {s_.prim_infeas:.3e} "
-              f"f {s_.f:.6f} alpha {s_.alpha:.3g}", flush=True)
+def progress(b, d):
+    """``b`` is the one-scenario batch driver behind ``slp``: its state is scenario 0 of each array."""
+    if b.lp_log[0]:
+        alpha = b.alpha[0] if hasattr(b, "alpha") else 1.0
+        print(f"  [{time.time() - t0:7.1f}s] SLP it {b.iter[0]} last LP {b.lp_log[0][-1]} prim_infeas "
+              f"{b.prim_infeas[0]:.3e} f {b.f[0]:.6f} alpha {alpha:.3g}", flush=True)
 
 
 slp.record = progress
