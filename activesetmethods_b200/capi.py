@@ -84,6 +84,9 @@ SIGNATURES = {
     "asm_slp_destroy": (None, [_VP]),
     "asm_slp_sizes": (C.c_int, [_VP, c_int64_p, c_int32_p, c_int32_p]),
     "asm_slp_get_csr": (C.c_int, [_VP, C.c_int32, c_int64_p, c_int32_p, c_double_p]),
+    "asm_slp_get_lp": (C.c_int, [_VP, C.c_int32, c_int32_p, c_int32_p, c_int64_p, c_int64_p, c_int32_p, c_double_p,
+                                 c_double_p, c_double_p, c_double_p, c_double_p, c_double_p, c_double_p, c_double_p,
+                                 c_double_p, c_double_p, c_double_p, c_int32_p]),
     "asm_slp_update": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, c_double_p, c_double_p, c_double_p,
                                  C.c_int32]),
     "asm_slp_solve": (C.c_int, [_VP, C.POINTER(LpParams), C.POINTER(LpInfo)]),

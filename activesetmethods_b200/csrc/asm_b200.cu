@@ -1108,6 +1108,46 @@ int asm_slp_get_csr(asm_slp *hh, int32_t s, int64_t *row_ptr, int32_t *col_idx, 
     }
     return ASM_OK;
 }
+int asm_slp_get_lp(asm_slp *hh, int32_t s, int32_t *cols, int32_t *rows, int64_t *nnz, int64_t *row_ptr,
+                   int32_t *col_idx, double *vals, double *c, double *c0, double *lb, double *ub, double *rl,
+                   double *ru, double *x, double *y, double *dual_lb, double *dual_ub, int32_t *status) {
+    if (!hh) return fail(ASM_E_INVALID, "null handle");
+    SlpHandle &h = hh->h;
+    if (s < 0 || s >= h.Buser) return fail(ASM_E_INVALID, "scenario out of range");
+    if (h.phase < 0) return fail(ASM_E_STATE, "no update yet");
+    if ((x || y || dual_lb || dual_ub || status) && !h.solved) return fail(ASM_E_STATE, "no solve since the last update");
+    LpSolver &lp = *h.cur();
+    if (cols) *cols = lp.n;
+    if (rows) *rows = lp.m;
+    if (nnz) *nnz = lp.nnz;
+    if (row_ptr)
+        for (int i = 0; i <= lp.m; ++i) row_ptr[i] = lp.h_row_ptr[i];
+    if (col_idx) std::copy(lp.h_col_idx.begin(), lp.h_col_idx.begin() + lp.nnz, col_idx);
+    ASM_CK(cudaSetDevice(h.device));
+    // one lane of an element-major [len][B] array
+    auto lane = [&](double *dst, const DBuf<double> &src, int64_t len) -> int {
+        if (dst && len)
+            ASM_CK(cudaMemcpy2DAsync(dst, sizeof(double), src.p + s, sizeof(double) * h.B, sizeof(double), len,
+                                     cudaMemcpyDeviceToHost, h.stream));
+        return ASM_OK;
+    };
+    ASM_TRY(lane(vals, lp.vals, lp.nnz));
+    ASM_TRY(lane(c, lp.c, lp.n));
+    ASM_TRY(lane(c0, lp.c0, 1));
+    ASM_TRY(lane(lb, lp.lb, lp.n));
+    ASM_TRY(lane(ub, lp.ub, lp.n));
+    ASM_TRY(lane(rl, lp.rl, lp.m));
+    ASM_TRY(lane(ru, lp.ru, lp.m));
+    ASM_TRY(lane(x, lp.xo, lp.n));
+    ASM_TRY(lane(y, lp.yo, lp.m));
+    ASM_TRY(lane(dual_lb, lp.dlo, lp.n));
+    ASM_TRY(lane(dual_ub, lp.dup, lp.n));
+    ScenState st;
+    if (status) ASM_CK(cudaMemcpyAsync(&st, lp.state.p + s, sizeof st, cudaMemcpyDeviceToHost, h.stream));
+    ASM_CK(cudaStreamSynchronize(h.stream));
+    if (status) *status = st.status;
+    return ASM_OK;
+}
 int asm_slp_update(asm_slp *h, const double *x_k, const double *f, const double *df, const double *E,
                    const double *dE, const double *delta, int32_t feasibility) {
     if (!h) return fail(ASM_E_INVALID, "null handle");

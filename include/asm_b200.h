@@ -165,6 +165,16 @@ int asm_slp_sizes(asm_slp *h, int64_t *nnz_csr, int32_t *lp_cols, int32_t *lp_ro
  * (bit-exact restatement of common.jl:12-20; duplicates summed in j_str order from 0.0).
  * row_ptr[m+1], col_idx[nnz_csr] 0-based, vals[nnz_csr]; any pointer may be NULL */
 int asm_slp_get_csr(asm_slp *h, int32_t s, int64_t *row_ptr, int32_t *col_idx, double *vals);
+/* the sub-LP of the last update as the engine holds it, for scenario s.  Normal phase: n columns, m rows (range rows
+ * two-sided), the Jacobian CSR; restoration: the reference layout of asm_slp_sizes (n + slacks, m + |adj|).
+ * cols, rows, nnz, row_ptr[rows+1], col_idx[nnz], vals[nnz], c[cols], c0, lb/ub[cols], rl/ru[rows];
+ * after a solve also the LP's own solution, before the read-back of subproblem.jl:500-536:
+ * x[cols], y[rows], dual_lb/dual_ub[cols] and the raw status of the scenario's solve (-1: still running when the
+ * solve stopped).  Any pointer may be NULL.  ASM_E_STATE before an update, and for the solution outputs before a
+ * solve; the handle's state is left as it is (no solve, no read-back). */
+int asm_slp_get_lp(asm_slp *h, int32_t s, int32_t *cols, int32_t *rows, int64_t *nnz, int64_t *row_ptr,
+                   int32_t *col_idx, double *vals, double *c, double *c0, double *lb, double *ub, double *rl,
+                   double *ru, double *x, double *y, double *dual_lb, double *dual_ub, int32_t *status);
 
 /* eval_functions! hand-over (slp.jl:186-191) + the data push of sub_optimize! (subproblem.jl:248-484):
  * x_k[batch][n], f[batch], df[batch][n], E[batch][m], dE[batch][nnz_coo] (j_str order), delta[batch],

@@ -71,6 +71,36 @@ def test_kkt_device_selftest_arguments(built_lib):
         assert call(device=-1) == capi.E_CUDA
 
 
+def test_slp_get_lp_arguments(built_lib):
+    """asm_slp_get_lp rejects a null handle without touching a device; with a device, a scenario outside [0, batch),
+    a read before the first update and a read of the solution before a solve are refused too."""
+    import numpy as np
+    i32, i64 = capi.c_int32_p, capi.c_int64_p
+    cols, rows, st = np.zeros(1, np.int32), np.zeros(1, np.int32), np.zeros(1, np.int32)
+    nnz = np.zeros(1, np.int64)
+    buf = np.zeros(64)
+
+    def call(h, s, x=None, status=None):
+        return built_lib.asm_slp_get_lp(h, s, cols.ctypes.data_as(i32), rows.ctypes.data_as(i32),
+                                        nnz.ctypes.data_as(i64), None, None, None, None, None, None, None, None, None,
+                                        capi.dptr(x), None, None, None, None if status is None else status.ctypes.data_as(i32))
+
+    for s in (-1, 0, 1):
+        assert call(None, s) == capi.E_INVALID
+        assert call(None, s, x=buf, status=st) == capi.E_INVALID
+    if built_lib.asm_device_count() == 0:
+        return
+    from activesetmethods_b200.sublp import SubLp
+    lp = SubLp(2, 1, np.array([[1, 1], [1, 2]]), [-1, -1], [1, 1], [0.0], [1.0], batch=3)
+    for s in (-1, 3, 64):
+        assert call(lp._h, s) == capi.E_INVALID
+    assert call(lp._h, 0) == capi.E_STATE
+    lp.update(np.zeros((3, 2)), np.zeros(3), np.ones((3, 2)), np.zeros((3, 1)), np.ones((3, 2)), 1.0)
+    assert call(lp._h, 2) == capi.OK and (cols[0], rows[0], nnz[0]) == (2, 1, 2)
+    assert call(lp._h, 2, x=buf) == capi.E_STATE and call(lp._h, 2, status=st) == capi.E_STATE
+    lp.close()
+
+
 def test_product_does_not_import_oracle():
     """Only tests/, smoke() and bench.py's cpu_baseline may touch oracle/."""
     pkg = os.path.join(ROOT, "activesetmethods_b200")
