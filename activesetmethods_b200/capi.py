@@ -101,6 +101,7 @@ SIGNATURES = {
     "asm_slp_merit_phi": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, c_double_p, C.c_int32, c_double_p]),
     "asm_slp_merit_derivative": (C.c_int, [_VP, c_double_p, C.c_int32, c_double_p]),
     "asm_slp_attach_acopf": (C.c_int, [_VP, C.POINTER(AcopfDesc)]),
+    "asm_slp_acopf_branch_coef": (C.c_int, [_VP, c_double_p]),
     "asm_slp_eval_acopf": (C.c_int, [_VP, c_double_p, c_double_p, C.c_int32]),
     "asm_slp_get_eval": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, c_double_p]),
     "asm_slp_acopf_trial": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, C.c_int32, c_double_p]),

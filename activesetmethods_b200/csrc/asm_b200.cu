@@ -327,6 +327,9 @@ struct AcopfDev {
     int k_angmax, k_angmin, k_ref, k_dc, k_thermal, k_bal, k_ohm;
     const int *f_bus, *t_bus, *bal_ptr, *bal_col;
     const double *coef, *gs, *bs, *cost2, *cost1, *cost0, *dc_loss1, *bal_coef;
+    // coefficient t of branch l for scenario s is coef[(t * nl + l) * coef_ld + s * coef_ls]: (1, 0) when the batch
+    // shares one [12][nl] array (asm_slp_attach_acopf), (B, 1) for per-scenario [12 nl][B] (asm_slp_acopf_branch_coef)
+    int64_t coef_ld = 1, coef_ls = 0;
 };
 struct AcopfIo {
     const double *xk, *p, *alpha;   // evaluation point x = xk (+ alpha p when TRIAL)
@@ -355,7 +358,7 @@ __global__ void __launch_bounds__(kThreads) k_acopf_branch(AcopfDev a, AcopfIo i
         const double vv = vf * vt;
         double c[12];
 #pragma unroll
-        for (int t = 0; t < 12; ++t) c[t] = a.coef[(int64_t)t * nl + l];
+        for (int t = 0; t < 12; ++t) c[t] = a.coef[((int64_t)t * nl + l) * a.coef_ld + s * a.coef_ls];
         auto E = [&](int row) -> double & { return io.E[(int64_t)row * B + s]; };
         E(a.r_angmax + (int)l) = d;
         E(a.r_angmin + (int)l) = d;
@@ -523,6 +526,7 @@ struct SlpHandle {
     AcopfDev acopf;
     DBuf<int> ac_f, ac_t, ac_bal_ptr, ac_bal_col;
     DBuf<double> ac_coef, ac_gs, ac_bs, ac_c2, ac_c1, ac_c0, ac_loss1, ac_bal_coef, ac_ftrial;
+    DBuf<double> ac_coef_scen;   // per-scenario branch coefficients [12 nl][B] (asm_slp_acopf_branch_coef)
 
     ~SlpHandle() {
         normal.reset();
@@ -1398,8 +1402,28 @@ int asm_slp_attach_acopf(asm_slp *hh, const asm_acopf_desc *d) {
     a.f_bus = h.ac_f.p; a.t_bus = h.ac_t.p; a.bal_ptr = h.ac_bal_ptr.p; a.bal_col = h.ac_bal_col.p;
     a.coef = h.ac_coef.p; a.gs = h.ac_gs.p; a.bs = h.ac_bs.p; a.cost2 = h.ac_c2.p; a.cost1 = h.ac_c1.p;
     a.cost0 = h.ac_c0.p; a.dc_loss1 = h.ac_loss1.p; a.bal_coef = h.ac_bal_coef.p;
+    h.ac_coef_scen.release();   // back to the shared coefficients
     h.acopf = a;
     h.has_acopf = true;
+    return ASM_OK;
+}
+
+// per-scenario branch coefficients coef[batch][12][nl] (contingencies, tap or impedance changes): the evaluator reads
+// them instead of the shared coef of the attach until the next asm_slp_attach_acopf
+int asm_slp_acopf_branch_coef(asm_slp *hh, const double *coef) {
+    SLP_GUARD();
+    if (!h.has_acopf) return fail(ASM_E_STATE, "asm_slp_attach_acopf first");
+    if (!coef) return fail(ASM_E_INVALID, "null argument");
+    const int64_t len = 12 * (int64_t)h.acopf.nl;
+    for (int64_t k = 0; k < len * h.Buser; ++k)
+        if (!std::isfinite(coef[k])) return fail(ASM_E_INVALID, "non-finite branch coefficient");
+    const size_t cnt = (size_t)std::max<int64_t>(len * B, 1);
+    if (h.ac_coef_scen.n < cnt) ASM_TRY(h.ac_coef_scen.alloc(cnt));
+    ASM_TRY(h.put(coef, len, h.Buser, h.ac_coef_scen.p));
+    ASM_CK(cudaGetLastError());
+    h.acopf.coef = h.ac_coef_scen.p;
+    h.acopf.coef_ld = B;
+    h.acopf.coef_ls = 1;
     return ASM_OK;
 }
 

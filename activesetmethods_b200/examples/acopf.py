@@ -15,6 +15,8 @@ Contents
   * ``CASE3_M`` / ``case9``     – the two small public networks (case3 is read from text, see tests)
   * ``synthetic_network``       – seeded generator matching the (bus, gen, branch) counts of the pegase cases
   * ``perturb_loads``           – load scenarios  pd,qd * (1 + 0.1 N(0,1)) clipped to +-30 %
+  * ``branch_contingencies``    – N-1 scenarios: one network per non-islanding single-branch outage
+  * ``generator_contingencies`` – one network per single-generator outage
   * ``AcopfModel``              – the NLP: sizes, bounds, ``j_str`` (1-based like the reference), callbacks
 
 Variable order (PowerModels creation order): va[nb], vm[nb], pg[ng], qg[ng], p[2nl arcs], q[2nl arcs],
@@ -33,7 +35,7 @@ import numpy as np
 
 __all__ = [
     "Network", "parse_matpower", "case9", "synthetic_network", "perturb_loads", "AcopfModel",
-    "PEGASE_SHAPES",
+    "PEGASE_SHAPES", "branch_contingencies", "generator_contingencies",
 ]
 
 # (buses, gens, branches) of the named configs in BASELINE.json (SURVEY.md App. D)
@@ -47,7 +49,13 @@ PEGASE_SHAPES = {
 
 @dataclass
 class Network:
-    """Per-unit network data (already divided by baseMVA, angles in radians, only in-service elements)."""
+    """Per-unit network data (already divided by baseMVA, angles in radians).
+
+    ``br_status[nl]`` and ``gen_status[ng]`` are 0/1 like MATPOWER's BR_STATUS / GEN_STATUS and default to all in
+    service.  ``parse_matpower`` drops the elements a file marks out of service, so the base network has only
+    in-service elements; a status set to 0 afterwards (a contingency) keeps the element in the arrays, and
+    ``AcopfModel`` keeps its variables, rows and Jacobian entries and takes it out of service by values and bounds
+    only, so that every contingency of a network shares the base case's Jacobian pattern."""
     baseMVA: float
     # buses
     bus_id: np.ndarray
@@ -91,6 +99,15 @@ class Network:
     dc_qmaxt: np.ndarray = field(default_factory=lambda: np.zeros(0))
     dc_loss0: np.ndarray = field(default_factory=lambda: np.zeros(0))
     dc_loss1: np.ndarray = field(default_factory=lambda: np.zeros(0))
+    # in-service flags (None: all in service)
+    br_status: np.ndarray = None
+    gen_status: np.ndarray = None
+
+    def __post_init__(self):
+        if self.br_status is None:
+            self.br_status = np.ones(len(self.f_bus), dtype=np.int64)
+        if self.gen_status is None:
+            self.gen_status = np.ones(len(self.gen_bus), dtype=np.int64)
 
     @property
     def nb(self):
@@ -343,13 +360,96 @@ def perturb_loads(net: Network, scenario: int, sigma: float = 0.1, clip: float =
     return out
 
 
+def _islands(net: Network, status: np.ndarray) -> bool:
+    """True if the branches with ``status`` != 0 leave the network in more pieces than the base network's in-service
+    branches do."""
+    from scipy.sparse import coo_matrix
+    from scipy.sparse.csgraph import connected_components
+
+    def pieces(on):
+        G = coo_matrix((np.ones(int(on.sum())), (net.f_bus[on], net.t_bus[on])), shape=(net.nb, net.nb))
+        return connected_components(G, directed=False)[0]
+    return pieces(status != 0) > pieces(net.br_status != 0)
+
+
+def branch_contingencies(net: Network, count: int | None = None) -> list:
+    """N-1 branch scenarios: one network per in-service branch whose outage does not island the network (the branch
+    set out of service with ``br_status``), in branch order; the first ``count`` of them if given.  Copies ``net``
+    like ``perturb_loads``; every scenario shares the base case's Jacobian pattern."""
+    import copy
+    out = []
+    for l in np.nonzero(net.br_status != 0)[0]:
+        if count is not None and len(out) == count:
+            break
+        status = net.br_status.copy()
+        status[l] = 0
+        if _islands(net, status):
+            continue
+        c = copy.copy(net)
+        c.br_status = status
+        out.append(c)
+    return out
+
+
+def generator_contingencies(net: Network) -> list:
+    """One network per in-service generator with that generator out of service (``gen_status``), in generator order.
+    Copies ``net`` like ``perturb_loads``."""
+    import copy
+    out = []
+    for k in np.nonzero(net.gen_status != 0)[0]:
+        c = copy.copy(net)
+        c.gen_status = net.gen_status.copy()
+        c.gen_status[k] = 0
+        out.append(c)
+    return out
+
+
+def _angle_paths(net: Network, lines: np.ndarray) -> np.ndarray:
+    """For each branch in ``lines``: the shortest path from its from-bus to its to-bus over the in-service branches,
+    each weighted by the widest angle difference its rows allow, max(angmax, -angmin).  Summed along any in-service
+    path, the angle-difference rows bound |va_f - va_t| by that length, so it is a bound the in-service network
+    already implies.  Raises ValueError if the terminals are not connected: the outage islands the network."""
+    from scipy.sparse import coo_matrix
+    from scipy.sparse.csgraph import dijkstra
+    on = net.br_status != 0
+    a = np.minimum(net.f_bus, net.t_bus)[on]
+    b = np.maximum(net.f_bus, net.t_bus)[on]
+    w = np.maximum(net.angmax, -net.angmin)[on]
+    # parallel branches: the smallest weight of each bus pair (a sparse matrix would add duplicates up)
+    order = np.lexsort((w, b, a))
+    a, b, w = a[order], b[order], w[order]
+    first = np.ones(len(a), dtype=bool)
+    first[1:] = (a[1:] != a[:-1]) | (b[1:] != b[:-1])
+    G = coo_matrix((w[first], (a[first], b[first])), shape=(net.nb, net.nb)).tocsr()
+    src = np.unique(net.f_bus[lines])
+    dist = dijkstra(G, directed=False, indices=src)
+    d = dist[np.searchsorted(src, net.f_bus[lines]), net.t_bus[lines]]
+    cut = ~np.isfinite(d)
+    if cut.any():
+        l = int(lines[np.argmax(cut)])
+        raise ValueError(f"the outage of branch {l} (buses {net.bus_id[net.f_bus[l]]}-{net.bus_id[net.t_bus[l]]}) "
+                         "islands the network: islanding contingencies are not supported")
+    return d
+
+
 # ----------------------------------------------------------------------------------------------------------
 # The NLP
 # ----------------------------------------------------------------------------------------------------------
 class AcopfModel:
     """ACP-polar OPF as (n, m, bounds, j_str, callbacks) — the tuple ``Model(...)`` receives at
     reference ``src/MOI_wrapper.jl:1093-1099``.  ``j_str`` is an (nnz, 2) int64 array of **1-based**
-    (row, col) pairs, like the reference's ``Vector{Tuple{Int64,Int64}}`` (``src/model.jl:10``)."""
+    (row, col) pairs, like the reference's ``Vector{Tuple{Int64,Int64}}`` (``src/model.jl:10``).
+
+    Out-of-service elements (``Network.br_status`` / ``gen_status`` = 0) change values and bounds only: ``n``, ``m``
+    and ``j_str`` are those of the all-in-service network.
+      * branch: its 12 admittance coefficients are 0, so its Ohm rows read p = 0, q = 0 on both arcs and the arcs drop
+        out of the balance rows by value.  Its thermal rows and flow bounds stay (inactive at zero flow).  Its angle-
+        difference rows are relaxed to +- the shortest in-service path between its terminals (``_angle_paths``): a
+        bound the rest of the network implies, so the feasible set is that of the network without the branch, and the
+        rows stay bounded (a free row is not accepted by the sub-LP builder).  An outage that islands the network
+        raises ValueError.
+      * generator: pmin = pmax = qmin = qmax = 0.  Its ``cost0`` stays in the objective as a constant (costs are
+        shared by a batch), so compare objectives with the network without it after subtracting that constant."""
 
     def __init__(self, net: Network, start: str = "midpoint"):
         self.net = net
@@ -385,20 +485,23 @@ class AcopfModel:
         ti = net.tap * np.sin(net.shift)
         tm2 = net.tap ** 2
         half_b = net.br_b / 2.0
-        self._cf = dict(
+        on = net.br_status != 0
+        cf = dict(
             a_pf=(g + 0.0) / tm2, b_pf=(-g * tr + b * ti) / tm2, c_pf=(-b * tr - g * ti) / tm2,
             a_qf=-(b + half_b) / tm2, b_qf=-(-b * tr - g * ti) / tm2, c_qf=(-g * tr + b * ti) / tm2,
             a_pt=(g + 0.0), b_pt=(-g * tr - b * ti) / tm2, c_pt=(-b * tr + g * ti) / tm2,
             a_qt=-(b + half_b), b_qt=-(-b * tr + g * ti) / tm2, c_qt=(-g * tr - b * ti) / tm2,
         )
+        self._cf = {k: np.where(on, v, 0.0) for k, v in cf.items()}
 
         # bounds
         inf = np.inf
         xl = np.full(self.n, -inf)
         xu = np.full(self.n, inf)
         xl[self.o_vm:self.o_vm + nb] = net.vmin; xu[self.o_vm:self.o_vm + nb] = net.vmax
-        xl[self.o_pg:self.o_pg + ng] = net.pmin; xu[self.o_pg:self.o_pg + ng] = net.pmax
-        xl[self.o_qg:self.o_qg + ng] = net.qmin; xu[self.o_qg:self.o_qg + ng] = net.qmax
+        gon = net.gen_status != 0
+        xl[self.o_pg:self.o_pg + ng] = np.where(gon, net.pmin, 0.0); xu[self.o_pg:self.o_pg + ng] = np.where(gon, net.pmax, 0.0)
+        xl[self.o_qg:self.o_qg + ng] = np.where(gon, net.qmin, 0.0); xu[self.o_qg:self.o_qg + ng] = np.where(gon, net.qmax, 0.0)
         ra2 = np.r_[net.rate_a, net.rate_a]
         xl[self.o_p:self.o_p + 2 * nl] = -ra2; xu[self.o_p:self.o_p + 2 * nl] = ra2
         xl[self.o_q:self.o_q + 2 * nl] = -ra2; xu[self.o_q:self.o_q + 2 * nl] = ra2
@@ -413,6 +516,11 @@ class AcopfModel:
         gu = np.full(self.m, inf)
         gu[self.r_angmax:self.r_angmax + nl] = net.angmax
         gl[self.r_angmin:self.r_angmin + nl] = net.angmin
+        out = np.nonzero(~on)[0]
+        if len(out):
+            d = _angle_paths(net, out)
+            gu[self.r_angmax + out] = d
+            gl[self.r_angmin + out] = -d
         gl[self.r_ref] = gu[self.r_ref] = 0.0
         if nd:
             gl[self.r_dc:self.r_dc + nd] = gu[self.r_dc:self.r_dc + nd] = net.dc_loss0

@@ -190,18 +190,18 @@ class _SlpBatch:
                         device=o.device, **{"warm_start": self.warm_start, **o.lp_options})
             opt._squeeze = False
             if self.device_evaluator:
-                # the device evaluator holds ONE network: every scenario must share everything but its loads (which
-                # only enter g_L / g_U).  A Model hands over the problem it was built from.
+                # the device evaluator holds one topology, shunts, costs, dc-line losses and reference bus for the
+                # batch; branch data (impedances, taps, shifts, outages) may differ per scenario, and loads, generator
+                # outages and relaxed angle rows only enter the bounds.  A Model hands over the problem it was built from.
                 acopf = [pr.source if isinstance(pr, Model) else pr for pr in prs]
                 n0 = acopf[0].net
                 for k, pr in enumerate(acopf[1:], 1):
-                    for name in ("f_bus", "t_bus", "br_r", "br_x", "br_b", "tap", "shift", "gs", "bs", "cost2", "cost1",
-                                 "cost0", "gen_bus", "dc_loss1"):
+                    for name in ("f_bus", "t_bus", "gs", "bs", "cost2", "cost1", "cost0", "gen_bus", "dc_loss1"):
                         if not np.array_equal(getattr(pr.net, name), getattr(n0, name)):
                             raise ValueError(f"device_evaluator: scenario {k} differs from scenario 0 in network.{name}")
                     if pr.net.ref_bus != n0.ref_bus:
                         raise ValueError(f"device_evaluator: scenario {k} has another reference bus")
-                opt.attach_acopf(acopf[0])
+                opt.attach_acopf(acopf)
             return opt
         if self.device_evaluator:
             raise ValueError("device_evaluator needs the B200 engine")

@@ -261,28 +261,54 @@ class SubLp:
         return dict(engine=e.value, group_size=g.value, groups=k.value)
 
     # -- device-side ACOPF evaluator (SURVEY.md 8(f)-1) ----------------------------------------------------------
-    def attach_acopf(self, model):
-        """Hand the network of an ``examples.acopf.AcopfModel`` to the device so that ``eval_acopf`` /
-        ``acopf_trial`` replace the host callbacks (``src/MOI_wrapper.jl:1047-1069``).  All scenarios of the batch
-        share the network; loads only enter the row bounds given at construction."""
+    _COEF_KEYS = ("a_pf", "b_pf", "c_pf", "a_qf", "b_qf", "c_qf", "a_pt", "b_pt", "c_pt", "a_qt", "b_qt", "c_qt")
+
+    @staticmethod
+    def _acopf_arrays(model):
+        """The arrays of ``asm_acopf_desc`` for one model, branch coefficients ``coef`` [12, nl] included."""
         net = model.net
         i32 = lambda a: np.ascontiguousarray(a, dtype=np.int32)   # noqa: E731
         f64 = lambda a: np.ascontiguousarray(a, dtype=np.float64)  # noqa: E731
-        cf = model._cf
-        keep = dict(
+        return dict(
             f_bus=i32(net.f_bus), t_bus=i32(net.t_bus),
-            coef=f64(np.stack([cf[k] for k in ("a_pf", "b_pf", "c_pf", "a_qf", "b_qf", "c_qf", "a_pt", "b_pt", "c_pt",
-                                               "a_qt", "b_qt", "c_qt")])),
+            coef=f64(np.stack([model._cf[k] for k in SubLp._COEF_KEYS])),
             gs=f64(net.gs), bs=f64(net.bs), cost2=f64(net.cost2), cost1=f64(net.cost1), cost0=f64(net.cost0),
             dc_loss1=f64(net.dc_loss1 if model.nd else np.zeros(1)),
             bal_ptr=i32(np.concatenate([[0], np.cumsum(np.bincount(model._bal_rows - model.r_bal,
                                                                    minlength=2 * model.nb))])),
             bal_col=i32(model._bal_cols), bal_coef=f64(model._bal_coef))
+
+    def attach_acopf(self, model):
+        """Hand the network of an ``examples.acopf.AcopfModel`` to the device so that ``eval_acopf`` /
+        ``acopf_trial`` replace the host callbacks (``src/MOI_wrapper.jl:1047-1069``).
+
+        ``model``: one model, whose network every scenario of the batch shares (loads only enter the row bounds
+        given at construction), or a list of ``batch`` models, one per scenario.  The models of a list must agree in
+        everything the evaluator holds once for the batch (topology, shunts, costs, dc-line losses, reference bus);
+        their branch coefficients may differ (impedance or tap changes, branch outages), and when they do they are
+        uploaded per scenario (``asm_slp_acopf_branch_coef``).  Generator outages, relaxed angle rows and loads reach
+        the device through the per-scenario bounds."""
+        models = list(model) if isinstance(model, (list, tuple)) else [model]
+        if len(models) not in (1, self.batch):
+            raise ValueError(f"attach_acopf: {len(models)} models for a batch of {self.batch}")
+        m0 = models[0]
+        keep = self._acopf_arrays(m0)
+        coefs = [keep["coef"]]
+        for k, mdl in enumerate(models[1:], 1):
+            if (mdl.nb, mdl.ng, mdl.nl, mdl.nd, int(mdl.net.ref_bus)) != (m0.nb, m0.ng, m0.nl, m0.nd, int(m0.net.ref_bus)):
+                raise ValueError(f"attach_acopf: scenario {k} differs from scenario 0 in its sizes or reference bus")
+            arrs = self._acopf_arrays(mdl)
+            for name, a in arrs.items():
+                if name != "coef" and not np.array_equal(a, keep[name], equal_nan=a.dtype == np.float64):
+                    raise ValueError(f"attach_acopf: scenario {k} differs from scenario 0 in {name}")
+            coefs.append(arrs["coef"])
         d = capi.AcopfDesc()
-        d.nb, d.ng, d.nl, d.nd, d.ref_bus = model.nb, model.ng, model.nl, model.nd, int(net.ref_bus)
+        d.nb, d.ng, d.nl, d.nd, d.ref_bus = m0.nb, m0.ng, m0.nl, m0.nd, int(m0.net.ref_bus)
         for k, a in keep.items():
             setattr(d, k, a.ctypes.data_as(capi.c_int32_p if a.dtype == np.int32 else capi.c_double_p))
         capi.check(self._lib.asm_slp_attach_acopf(self._h, C.byref(d)))
+        if any(not np.array_equal(c, coefs[0]) for c in coefs[1:]):
+            capi.check(self._lib.asm_slp_acopf_branch_coef(self._h, capi.dptr(np.ascontiguousarray(np.stack(coefs)))))
 
     def eval_acopf(self, x, delta=1000.0, feasibility=False):
         """``eval_functions!`` (slp.jl:186-191) on the device at ``x`` + the device part of ``update``."""

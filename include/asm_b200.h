@@ -224,7 +224,10 @@ int asm_slp_merit_derivative(asm_slp *h, const double *nu, int32_t feasibility, 
  * (src/algorithms/slp.jl:186-191) for the ACP-polar OPF in the variable / row / Jacobian layout of
  * activesetmethods_b200/examples/acopf.py: variables va[nb] vm[nb] pg[ng] qg[ng] p[2nl] q[2nl] pdc[2nd] qdc[2nd];
  * rows angmax[nl] angmin[nl] ref dc[nd] thermal[2nl] balance[2nb] ohm[4nl]; j_str in the same block order.
- * All scenarios of a batch share the network (loads only enter the row bounds). */
+ * All scenarios of a batch share the topology, shunts, costs, dc-line losses and reference bus.  Loads, generator
+ * outages and relaxed angle rows only enter the bounds; the 12 branch coefficients are shared unless
+ * asm_slp_acopf_branch_coef gives them per scenario (impedance or tap changes, branch outages with zero coefficients
+ * on the fixed pattern: N-1 contingency batches). */
 typedef struct asm_acopf_desc {
     int32_t nb, ng, nl, nd, ref_bus;
     const int32_t *f_bus, *t_bus;         /* [nl] 0-based bus indices                                              */
@@ -237,6 +240,10 @@ typedef struct asm_acopf_desc {
     const double *bal_coef;               /* constant coefficients, NaN at the vm^2 (shunt) slots                  */
 } asm_acopf_desc;
 int asm_slp_attach_acopf(asm_slp *h, const asm_acopf_desc *d);
+/* per-scenario branch coefficients coef[batch][12][nl], each scenario in the order of asm_acopf_desc.coef; finite.
+ * Call after asm_slp_attach_acopf (ASM_E_STATE before); they hold until the next attach, which returns the handle to
+ * the shared coefficients of its description. */
+int asm_slp_acopf_branch_coef(asm_slp *h, const double *coef);
 /* eval_functions! on the device at x[batch][n], then the device part of asm_slp_update */
 int asm_slp_eval_acopf(asm_slp *h, const double *x, const double *delta, int32_t feasibility);
 /* f[batch], df[batch][n], E[batch][m], dE[batch][nnz_coo] of the last evaluation; any pointer may be NULL */
