@@ -116,6 +116,8 @@ SIGNATURES = {
     "asm_slp_timer_stop": (C.c_int, [_VP, c_double_p]),
     "asm_slp_kernel_timing": (C.c_int, [_VP, C.c_int32, c_double_p, c_double_p]),
     "asm_slp_set_active": (C.c_int, [_VP, c_int32_p]),
+    "asm_slp_load_lanes": (C.c_int, [_VP, C.c_int32, c_int32_p, c_double_p, c_double_p, c_double_p, c_double_p]),
+    "asm_slp_acopf_branch_coef_lanes": (C.c_int, [_VP, C.c_int32, c_int32_p, c_double_p]),
     "asm_slp_ipm_info": (C.c_int, [_VP, c_int64_p, c_double_p]),
     "asm_slp_ipm_timing": (C.c_int, [_VP, C.c_int32, c_double_p, c_double_p]),
     "asm_kkt_selftest": (C.c_int, [C.c_int32, C.c_int32, c_int64_p, c_int32_p, c_double_p, c_double_p, c_double_p,

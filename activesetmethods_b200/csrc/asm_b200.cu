@@ -527,12 +527,17 @@ struct SlpHandle {
     DBuf<int> ac_f, ac_t, ac_bal_ptr, ac_bal_col;
     DBuf<double> ac_coef, ac_gs, ac_bs, ac_c2, ac_c1, ac_c0, ac_loss1, ac_bal_coef, ac_ftrial;
     DBuf<double> ac_coef_scen;   // per-scenario branch coefficients [12 nl][B] (asm_slp_acopf_branch_coef)
+    // asm_slp_load_lanes / asm_slp_acopf_branch_coef_lanes: the lane list on the device
+    DBuf<int> d_lanes;
+    cudaEvent_t lanes_ev = nullptr;
+    bool lanes_ev_used = false;
 
     ~SlpHandle() {
         normal.reset();
         fr.reset();
         if (tev0) cudaEventDestroy(tev0);
         if (tev1) cudaEventDestroy(tev1);
+        if (lanes_ev) cudaEventDestroy(lanes_ev);
         if (stream) cudaStreamDestroy(stream);
     }
     LpSolver *cur() { return phase == 1 ? fr.get() : normal.get(); }
@@ -558,6 +563,87 @@ struct SlpHandle {
         v.adj = d_adj.p;
         v.adj_of_row = d_adj_of_row.p;
         return v;
+    }
+
+    // row class of the bounds (l, u) (subproblem.jl:87-112); ASM_E_FREE_ROW when both are infinite
+    static int classify(double l, double u, uint8_t &out) {
+        const bool lf = l > -INFINITY, uf = u < INFINITY;
+        if (!lf && !uf) return ASM_E_FREE_ROW;
+        if (l == u)
+            out = ROW_EQ;
+        else if (lf && uf)
+            out = ROW_RANGE;
+        else if (lf)
+            out = ROW_LOWER;
+        else
+            out = ROW_UPPER;
+        return ASM_OK;
+    }
+
+    // the lane list lanes[k] -> d_lanes through the pinned small buffer (after the area of the reductions and trial
+    // steps); the event keeps the next call from overwriting the pinned copy before its DMA has read it
+    int put_lane_list(const int32_t *lanes, int k) {
+        int32_t *pl = (int32_t *)((double *)pin_small.p + (size_t)B * (R_COUNT + 1));
+        if (lanes_ev_used) ASM_CK(cudaEventSynchronize(lanes_ev));
+        if (!lanes_ev) ASM_CK(cudaEventCreateWithFlags(&lanes_ev, cudaEventDisableTiming));
+        memcpy(pl, lanes, sizeof(int32_t) * k);
+        ASM_CK(cudaMemcpyAsync(d_lanes.p, pl, sizeof(int32_t) * k, cudaMemcpyHostToDevice, stream));
+        ASM_CK(cudaEventRecord(lanes_ev, stream));
+        lanes_ev_used = true;
+        return ASM_OK;
+    }
+    // host [k][len] -> device [len][B] at the lanes of the last put_lane_list, through the pinned ring and `stage`
+    int put_lanes(const double *host, int64_t len, int k, double *dst) {
+        if (len == 0) return ASM_OK;
+        if (stage.n < (size_t)len * k) {
+            ASM_CK(cudaStreamSynchronize(stream));   // earlier layout kernels may still read the old buffer
+            ASM_TRY(stage.alloc((size_t)len * k));
+        }
+        ASM_TRY(ring.h2d(stage.p, host, (size_t)len * k * sizeof(double), stream));
+        dim3 grid((unsigned)((len + 31) / 32), (unsigned)((k + 31) / 32)), block(32, 8);
+        k_lanes_in<<<grid, block, 0, stream>>>(stage.p, dst, d_lanes.p, len, k, B);
+        ++own_launches;
+        ASM_CK(cudaGetLastError());
+        return ASM_OK;
+    }
+    int check_lanes(int k, const int32_t *lanes) {
+        if (k < 0) return fail(ASM_E_INVALID, "negative lane count");
+        if (k > 0 && !lanes) return fail(ASM_E_INVALID, "null lane list");
+        std::vector<char> seen(Buser, 0);
+        for (int j = 0; j < k; ++j) {
+            if (lanes[j] < 0 || lanes[j] >= Buser) return fail(ASM_E_INVALID, "lane out of range");
+            if (seen[lanes[j]]) return fail(ASM_E_INVALID, "lane repeated");
+            seen[lanes[j]] = 1;
+        }
+        return ASM_OK;
+    }
+
+    // replace the scenarios of k lanes: bounds x_L/x_U[k][n], g_L/g_U[k][m] in the order of `lanes`
+    int load_lanes(int k, const int32_t *lanes, const double *hxL, const double *hxU, const double *hgL,
+                   const double *hgU) {
+        ASM_TRY(check_lanes(k, lanes));
+        if (k == 0) return ASM_OK;
+        if (!hxL || !hxU || (m > 0 && (!hgL || !hgU))) return fail(ASM_E_INVALID, "null bound array");
+        if (Bb == 1 && Buser > 1) return fail(ASM_E_STATE, "the handle shares one set of bounds over its batch");
+        for (int j = 0; j < k; ++j)
+            for (int i = 0; i < m; ++i) {
+                uint8_t c = 0;
+                if (classify(hgL[(size_t)j * m + i], hgU[(size_t)j * m + i], c) != ASM_OK)
+                    return fail(ASM_E_FREE_ROW, "row with two infinite bounds (unsupported by the reference builder)");
+                if (c != cls[i]) return fail(ASM_E_INVALID, "row class differs from the handle's");
+            }
+        ASM_CK(cudaSetDevice(device));
+        ASM_TRY(put_lane_list(lanes, k));
+        ASM_TRY(put_lanes(hxL, n, k, xL.p));
+        ASM_TRY(put_lanes(hxU, n, k, xU.p));
+        ASM_TRY(put_lanes(hgL, m, k, gL.p));
+        ASM_TRY(put_lanes(hgU, m, k, gU.p));
+        normal->forget_warm_start(lanes, k);
+        if (fr) fr->forget_warm_start(lanes, k);
+        phase = -1;   // the LP data of the loaded lanes is stale until the next update
+        solved = false;
+        extracted = false;
+        return ASM_OK;
     }
 
     // host [S][len] -> device [len][B]
@@ -617,19 +703,6 @@ struct SlpHandle {
         const int S = per_scen ? batch : 1;
         int col = n;
         for (int i = 0; i < m; ++i) {
-            auto classify = [&](double l, double u, uint8_t &out) -> int {
-                const bool lf = l > -INFINITY, uf = u < INFINITY;
-                if (!lf && !uf) return ASM_E_FREE_ROW;
-                if (l == u)
-                    out = ROW_EQ;
-                else if (lf && uf)
-                    out = ROW_RANGE;
-                else if (lf)
-                    out = ROW_LOWER;
-                else
-                    out = ROW_UPPER;
-                return ASM_OK;
-            };
             uint8_t c0 = 0;
             if (classify(hgL[i], hgU[i], c0) != ASM_OK)
                 return fail(ASM_E_FREE_ROW, "row with two infinite bounds (unsupported by the reference builder)");
@@ -685,6 +758,7 @@ struct SlpHandle {
         ASM_TRY(small_out.alloc((size_t)B * R_COUNT));
         ASM_TRY(partials.alloc((size_t)R_COUNT * kMaxBlocksX * B));
         ASM_TRY(pin_small.reserve(sizeof(double) * (size_t)B * (R_COUNT + 4)));
+        ASM_TRY(d_lanes.alloc(B));
         ASM_TRY(pslack.zero(stream));
         ASM_TRY(lam.zero(stream));
         ASM_TRY(p.zero(stream));
@@ -1172,6 +1246,11 @@ int asm_slp_set_active(asm_slp *h, const int32_t *active) {
         h->h.mask.clear();
     return ASM_OK;
 }
+int asm_slp_load_lanes(asm_slp *h, int32_t k, const int32_t *lanes, const double *x_L, const double *x_U,
+                       const double *g_L, const double *g_U) {
+    if (!h) return fail(ASM_E_INVALID, "null handle");
+    return h->h.load_lanes(k, lanes, x_L, x_U, g_L, g_U);
+}
 int asm_slp_extract(asm_slp *h, double *p, double *lambda, double *mult_x_U, double *mult_x_L, double *p_slack,
                     int32_t *status) {
     if (!h) return fail(ASM_E_INVALID, "null handle");
@@ -1200,6 +1279,7 @@ int asm_slp_sub_optimize(asm_slp *h, const double *x_k, const double *f, const d
 int asm_slp_norm_violations(asm_slp *hh, const double *E, const double *x, int32_t p_norm, double *out) {
     SLP_GUARD();
     if (!out || p_norm < 0 || p_norm > 2) return fail(ASM_E_INVALID, "bad argument");
+    if ((!E || !x) && h.phase < 0) return fail(ASM_E_STATE, "no update yet");
     const double *dEv = h.E.p, *dx = h.xk.p;
     if (E) {
         ASM_TRY(h.put(E, h.m, h.Buser, h.tmp_m.p));
@@ -1265,6 +1345,7 @@ int asm_slp_kt_residuals(asm_slp *hh, const double *df, const double *lambda, co
 int asm_slp_norm_complementarity(asm_slp *hh, const double *E, const double *lambda, double *out) {
     SLP_GUARD();
     if (!out || !lambda) return fail(ASM_E_INVALID, "null argument");
+    if (!E && h.phase < 0) return fail(ASM_E_STATE, "no update yet");
     const double *dEv = h.E.p;
     if (E) {
         ASM_TRY(h.put(E, h.m, h.Buser, h.tmp_m.p));
@@ -1421,6 +1502,35 @@ int asm_slp_acopf_branch_coef(asm_slp *hh, const double *coef) {
     if (h.ac_coef_scen.n < cnt) ASM_TRY(h.ac_coef_scen.alloc(cnt));
     ASM_TRY(h.put(coef, len, h.Buser, h.ac_coef_scen.p));
     ASM_CK(cudaGetLastError());
+    h.acopf.coef = h.ac_coef_scen.p;
+    h.acopf.coef_ld = B;
+    h.acopf.coef_ls = 1;
+    return ASM_OK;
+}
+
+// per-scenario branch coefficients coef[k][12][nl] for the lanes `lanes`; the other lanes keep theirs.  The first call
+// on a handle that still shares its coefficients first broadcasts them into every lane of a per-scenario array.
+int asm_slp_acopf_branch_coef_lanes(asm_slp *hh, int32_t k, const int32_t *lanes, const double *coef) {
+    SLP_GUARD();
+    ASM_TRY(h.check_lanes(k, lanes));
+    if (k == 0) return ASM_OK;
+    if (!coef) return fail(ASM_E_INVALID, "null argument");
+    if (!h.has_acopf) return fail(ASM_E_STATE, "asm_slp_attach_acopf first");
+    const int64_t len = 12 * (int64_t)h.acopf.nl;
+    for (int64_t e = 0; e < len * k; ++e)
+        if (!std::isfinite(coef[e])) return fail(ASM_E_INVALID, "non-finite branch coefficient");
+    if (!h.ac_coef_scen.p) {
+        ASM_TRY(h.ac_coef_scen.alloc((size_t)std::max<int64_t>(len * B, 1)));
+        if (len && B == 1) {
+            ASM_CK(cudaMemcpyAsync(h.ac_coef_scen.p, h.ac_coef.p, len * sizeof(double), cudaMemcpyDeviceToDevice, stream));
+        } else if (len) {
+            dim3 grid((unsigned)((len + 31) / 32), B / 32), block(32, 8);
+            k_layout_in<<<grid, block, 0, stream>>>(h.ac_coef.p, h.ac_coef_scen.p, len, 1, B);
+            ++own_launches;
+        }
+    }
+    ASM_TRY(h.put_lane_list(lanes, k));
+    ASM_TRY(h.put_lanes(coef, len, k, h.ac_coef_scen.p));
     h.acopf.coef = h.ac_coef_scen.p;
     h.acopf.coef_ld = B;
     h.acopf.coef_ls = 1;

@@ -1543,6 +1543,13 @@ class LpSolver {
         return ASM_OK;
     }
 
+    // the scenarios in `lanes` were replaced: their next PDHG solve starts cold (d_prev_ok is built from host_state at
+    // the start of a warm solve).  The barrier engine keeps nothing across solves.
+    void forget_warm_start(const int32_t *lanes, int k) {
+        for (int j = 0; j < k; ++j)
+            if (lanes[j] < (int)host_state.size()) host_state[lanes[j]].status = ASM_LP_SKIPPED;
+    }
+
     // ---- barrier engine: Mehrotra predictor-corrector on the fixed-pattern L D L' (ipm.cuh) ----------------------
     int ensure_ipm() {
         if (ipm) return ASM_OK;

@@ -291,6 +291,28 @@ __global__ void k_layout_out(const double *__restrict__ src, double *__restrict_
     }
 }
 
+// k_layout_in for k lanes of a batch: host [k][len] (entry j in the order of `lanes`) -> device d[i * B + lanes[j]],
+// tiled like k_layout_in so that the staging reads coalesce.  grid (ceil(len/32), ceil(k/32)), block (32, 8).
+// The other lanes are not touched.
+__global__ void k_lanes_in(const double *__restrict__ src, double *__restrict__ dst, const int *__restrict__ lanes,
+                           int64_t len, int k, int B) {
+    __shared__ double tile[32][33];
+    const int64_t i0 = (int64_t)blockIdx.x * 32;
+    const int j0 = blockIdx.y * 32;
+    for (int r = threadIdx.y; r < 32; r += 8) {
+        const int j = j0 + r;
+        const int64_t i = i0 + threadIdx.x;
+        if (i < len && j < k) tile[r][threadIdx.x] = src[(int64_t)j * len + i];
+    }
+    __syncthreads();
+    const int j = j0 + threadIdx.x;
+    const int s = j < k ? lanes[j] : 0;
+    for (int r = threadIdx.y; r < 32; r += 8) {
+        const int64_t i = i0 + r;
+        if (i < len && j < k) dst[i * B + s] = tile[threadIdx.x][r];
+    }
+}
+
 // 1, or a multiple of 32; batches beyond 32 round up to 64 so that the two-scenarios-per-lane kernels apply
 inline int pad_batch(int b) { return b <= 1 ? 1 : (b <= 32 ? 32 : ((b + 63) / 64) * 64); }
 

@@ -135,7 +135,15 @@ class _SlpBatch:
 
     ``record``: optional ``callable(driver, dict)``, called before every sub-LP solve for each scenario solved, with
     that scenario's linearisation (``x, f, df, E, dE, delta, fr``).  ``lp_log[s]`` lists (status, objective,
-    restoration flag, iterations) of every sub-LP solved for scenario ``s``."""
+    restoration flag, iterations) of every sub-LP solved for scenario ``s``.
+
+    ``lanes``: run ``len(problems)`` scenarios through a handle of only ``lanes`` lanes (continuous batching).  Lane
+    ``l`` starts with problem ``l``; a problem whose run ends in a round is retired in that round, and before the next
+    round the next queued problems are loaded into the freed lanes with one ``load_lanes`` call (the handle, its
+    symbolic analysis and its captured graphs stay).  A loaded lane starts exactly like a lane of a fresh batch.
+    During ``run`` the state arrays are indexed by lane; afterwards ``ret``, ``iter``, ``x``, ``obj_val``,
+    ``prim_infeas``, ``dual_infeas``, ``compl``, ``lp_solves`` and ``lp_log`` (and ``delta`` for the trust region) are
+    indexed by problem.  ``None`` (or ``lanes >= len(problems)``): one lane per problem, one batch."""
 
     # Line search: every sub-LP starts from the previous one's (p, lambda) -- the analogue of GLPK keeping its basis
     # (one glp_prob per SLP run, slp.jl:24); it halves the PDHG work (case118: 1.03 M -> 0.51 M iterations for the
@@ -143,8 +151,10 @@ class _SlpBatch:
     # (degenerate) restoration LPs is returned and the runs measured so far ended further from the optimum.
     # ``lp_options={"warm_start": ...}`` overrides either.
     warm_start = 1
+    # per-problem results of a queued run (see ``lanes``)
+    _outputs = ("ret", "iter", "x", "obj_val", "prim_infeas", "dual_infeas", "compl", "lp_solves")
 
-    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
+    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False, lanes=None):
         self.device_evaluator = bool(device_evaluator)
         self.problems = list(problems)
         self.options = parameters if parameters is not None else Parameters()
@@ -153,6 +163,20 @@ class _SlpBatch:
         for pr in self.problems:
             if pr.n != self.n or pr.m != self.m or not np.array_equal(pr.j_str, p0.j_str):
                 raise ValueError("batched scenarios must share the Jacobian pattern")
+        self._queue = None                  # all problems of a queued run; None: one lane per problem
+        if lanes is not None:
+            if int(lanes) < 1:
+                raise ValueError(f"lanes must be at least 1, got {lanes}")
+            ext = self.options.external_optimizer
+            if int(lanes) < self.B:
+                if ext != "B200LP" and not hasattr(ext, "load_lanes"):
+                    raise ValueError("lanes < len(problems) needs an external_optimizer with load_lanes")
+                self._queue = self.problems
+                self.problems = self._queue[:int(lanes)]
+                self.B = int(lanes)
+                self._slot = np.arange(self.B)  # problem held by each lane, -1 once retired with the queue empty
+                self._next = self.B             # next problem to load
+                self.loads = []                 # lanes loaded before each round that loaded any, (round, lanes)
         B, n, m = self.B, self.n, self.m
         self.x = np.array([np.array(pr.x if isinstance(pr, Model) else pr.x0, dtype=float) for pr in self.problems])
         self.f = np.zeros(B)
@@ -193,9 +217,10 @@ class _SlpBatch:
                 # the device evaluator holds one topology, shunts, costs, dc-line losses and reference bus for the
                 # batch; branch data (impedances, taps, shifts, outages) may differ per scenario, and loads, generator
                 # outages and relaxed angle rows only enter the bounds.  A Model hands over the problem it was built from.
-                acopf = [pr.source if isinstance(pr, Model) else pr for pr in prs]
+                acopf = self._acopf(prs)
                 n0 = acopf[0].net
-                for k, pr in enumerate(acopf[1:], 1):
+                # a queued run checks every problem up front, so that a mismatch fails before any solve
+                for k, pr in enumerate(self._acopf(self._queue or prs)[1:], 1):
                     for name in ("f_bus", "t_bus", "gs", "bs", "cost2", "cost1", "cost0", "gen_bus", "dc_loss1"):
                         if not np.array_equal(getattr(pr.net, name), getattr(n0, name)):
                             raise ValueError(f"device_evaluator: scenario {k} differs from scenario 0 in network.{name}")
@@ -208,12 +233,67 @@ class _SlpBatch:
         return o.external_optimizer(self.n, self.m, prs[0].j_str, arr("x_L"), arr("x_U"), arr("g_L"), arr("g_U"),
                                     batch=self.B)
 
+    @staticmethod
+    def _acopf(prs):
+        """The ACOPF models behind ``prs`` (a Model hands over the problem it was built from)."""
+        return [pr.source if isinstance(pr, Model) else pr for pr in prs]
+
     def _clip_starts(self):
-        for s, pr in enumerate(self.problems):                              # slp_line_search.jl:96-105
-            lo = pr.x_L > -INF
-            self.x[s][lo] = np.maximum(self.x[s][lo], pr.x_L[lo])
-            up = pr.x_U > -INF
-            self.x[s][up] = np.minimum(self.x[s][up], pr.x_U[up])
+        for s, pr in enumerate(self.problems):
+            self._clip_start(s, pr)
+
+    def _clip_start(self, s, pr):                                           # slp_line_search.jl:96-105
+        lo = pr.x_L > -INF
+        self.x[s][lo] = np.maximum(self.x[s][lo], pr.x_L[lo])
+        up = pr.x_U > -INF
+        self.x[s][up] = np.minimum(self.x[s][up], pr.x_U[up])
+
+    def _reset_lane(self, s, pr):
+        """Lane ``s`` starts problem ``pr`` exactly like lane ``s`` of a fresh batch."""
+        self.x[s] = np.array(pr.x if isinstance(pr, Model) else pr.x0, dtype=float)
+        self._clip_start(s, pr)
+        for a in (self.f, self.df, self.E, self.dE, self.p, self.lam, self.mult_x_U, self.mult_x_L, self.nu):
+            a[s] = 0.0
+        self.prim_infeas[s] = self.dual_infeas[s] = self.compl[s] = INF
+        self.iter[s] = 1
+        self.ret[s] = -5
+        self.fr[s] = False
+        self.running[s] = True
+        self.lp_solves[s] = 0
+        self.lp_log[s] = []
+
+    def _refill(self):
+        """Continuous batching, at the end of a round: retire the problems whose runs ended in it (their results are
+        stored by problem), then load the next queued problems into the freed lanes with one ``load_lanes`` call."""
+        if not hasattr(self, "_res"):
+            N = len(self._queue)
+            self._res = {name: np.zeros((N,) + getattr(self, name).shape[1:], getattr(self, name).dtype)
+                         for name in self._outputs}
+            self._res_log = [None] * N
+        done = np.nonzero(~self.running & (self._slot >= 0))[0]
+        for s in done:
+            q = self._slot[s]
+            self.obj_val[s] = self.problems[s].eval_f(self.x[s])
+            for name in self._outputs:
+                self._res[name][q] = getattr(self, name)[s]
+            self._res_log[q] = self.lp_log[s]
+            self._slot[s] = -1
+        load = done[:max(0, len(self._queue) - self._next)]
+        if not len(load):
+            return
+        new = self._queue[self._next:self._next + len(load)]
+        for s, pr in zip(load, new):
+            self._slot[s] = self._next
+            self._next += 1
+            self.problems[s] = pr
+            self._reset_lane(s, pr)
+        bounds = [np.array([np.asarray(getattr(pr, name), dtype=float) for pr in new])
+                  for name in ("x_L", "x_U", "g_L", "g_U")]
+        if self.device_evaluator:
+            self.optimizer.load_lanes(load, *bounds, acopf=self._acopf(new))
+        else:
+            self.optimizer.load_lanes(load, *bounds)
+        self.loads.append((self.rounds, load.copy()))
 
     def _eval(self, s):
         pr = self.problems[s]
@@ -257,8 +337,15 @@ class _SlpBatch:
                   f"{self.dual_infeas[s]:.4e}  {self.compl[s]:.4e}  {self.lp_time:7.2f}{extra}")
 
     def _finish(self):
-        for s, pr in enumerate(self.problems):
-            self.obj_val[s] = pr.eval_f(self.x[s])
+        if self._queue is None:
+            for s, pr in enumerate(self.problems):
+                self.obj_val[s] = pr.eval_f(self.x[s])
+            return
+        # every problem was retired by _refill in the round its run ended: publish the results by problem
+        self.problems = self._queue
+        for name in self._outputs:
+            setattr(self, name, self._res[name])
+        self.lp_log = self._res_log
 
 
 class SlpLSBatch(_SlpBatch):
@@ -272,9 +359,13 @@ class SlpLSBatch(_SlpBatch):
     f, g and the Jacobian are evaluated by the device-side ACOPF evaluator (``SubLp.eval_acopf``) and every
     backtracking trial is one ``SubLp.acopf_trial`` call for the whole batch."""
 
-    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
-        super().__init__(problems, parameters, device_evaluator)
+    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False, lanes=None):
+        super().__init__(problems, parameters, device_evaluator, lanes)
         self.alpha = np.zeros(self.B)
+
+    def _reset_lane(self, s, pr):
+        super()._reset_lane(s, pr)
+        self.alpha[s] = 0.0
 
     def run(self):
         o = self.options
@@ -362,6 +453,8 @@ class SlpLSBatch(_SlpBatch):
                     continue
                 self.x[s] = self.x[s] + self.alpha[s] * self.p[s]
                 self.iter[s] += 1
+            if self._queue is not None:
+                self._refill()
         self._finish()
         return self
 
@@ -417,13 +510,18 @@ class SlpTRBatch(_SlpBatch):
     ``device_evaluator=True``: as for ``SlpLSBatch``; ϕ(x + p) is one ``SubLp.acopf_trial`` call for the batch."""
 
     warm_start = 0      # see _SlpBatch.warm_start
+    _outputs = _SlpBatch._outputs + ("delta",)
 
-    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False):
-        super().__init__(problems, parameters, device_evaluator)
+    def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False, lanes=None):
+        super().__init__(problems, parameters, device_evaluator, lanes)
         self.delta = np.full(self.B, float(self.options.tr_size))           # slp_trust_region.jl:62-65
         self.delta_max = 2.0
         self.alpha1 = 0.1
         self.alpha2 = 0.25
+
+    def _reset_lane(self, s, pr):
+        super()._reset_lane(s, pr)
+        self.delta[s] = float(self.options.tr_size)
 
     def run(self):                                                          # :87-206
         self._clip_starts()
@@ -444,6 +542,8 @@ class SlpTRBatch(_SlpBatch):
             for fr in (False, True):
                 if need[fr].any():
                     self._phase(fr, need[fr])
+            if self._queue is not None:
+                self._refill()
         self._finish()
         return self
 

@@ -93,6 +93,7 @@ class SubLp:
         return a[0] if self.batch == 1 and self._squeeze else a
 
     _squeeze = True
+    _acopf_ref = None       # (model, arrays) of scenario 0 of the last attach_acopf
 
     # -- the hot path -----------------------------------------------------------------------------------------
     def update(self, x_k, f, df, E, dE, delta, feasibility=False):
@@ -111,6 +112,31 @@ class SubLp:
         m = np.ascontiguousarray(np.asarray(mask).astype(bool), dtype=np.int32)
         assert m.shape == (self.batch,)
         capi.check(self._lib.asm_slp_set_active(self._h, m.ctypes.data_as(capi.c_int32_p)))
+
+    def load_lanes(self, lanes, x_L, x_U, g_L, g_U, acopf=None):
+        """Replace the scenarios held by the lanes ``lanes`` (distinct, in ``[0, batch)``) with new ones: bounds
+        ``[k, n]`` / ``[k, m]`` in the order of ``lanes``, every row keeping its class.  ``acopf``: with the device
+        evaluator attached, the ``AcopfModel`` of each new scenario; they must agree with the attached network in
+        everything but the branch coefficients, which go up per lane.  The handle needs an ``update`` (or
+        ``eval_acopf``) before the next solve; the loaded lanes start their next PDHG solves cold."""
+        lanes = np.ascontiguousarray(np.asarray(lanes).reshape(-1), dtype=np.int32)
+        k = len(lanes)
+        if k == 0:
+            return
+        coef = None
+        if acopf is not None:
+            acopf = list(acopf)
+            if len(acopf) != k:
+                raise ValueError(f"load_lanes: {len(acopf)} models for {k} lanes")
+            coef = np.ascontiguousarray(np.stack([self._acopf_coef(mdl, f"load_lanes: the model for lane {int(l)}")
+                                                  for l, mdl in zip(lanes, acopf)]))
+        x_L, x_U = capi.as_f64(x_L, (k, self.n)), capi.as_f64(x_U, (k, self.n))
+        g_L, g_U = capi.as_f64(g_L, (k, self.m)), capi.as_f64(g_U, (k, self.m))
+        lp = lanes.ctypes.data_as(capi.c_int32_p)
+        capi.check(self._lib.asm_slp_load_lanes(self._h, k, lp, capi.dptr(x_L), capi.dptr(x_U), capi.dptr(g_L),
+                                                capi.dptr(g_U)))
+        if coef is not None:
+            capi.check(self._lib.asm_slp_acopf_branch_coef_lanes(self._h, k, lp, capi.dptr(coef)))
 
     def solve(self):
         info = (capi.LpInfo * self.batch)()
@@ -278,6 +304,20 @@ class SubLp:
                                                                    minlength=2 * model.nb))])),
             bal_col=i32(model._bal_cols), bal_coef=f64(model._bal_coef))
 
+    def _acopf_coef(self, mdl, who):
+        """The branch coefficients of ``mdl`` after checking that it agrees with the attached network (scenario 0 of
+        the last ``attach_acopf``) in everything the evaluator holds once for the batch."""
+        if self._acopf_ref is None:
+            raise ValueError(f"{who}: no ACOPF network attached (attach_acopf first)")
+        m0, keep = self._acopf_ref
+        if (mdl.nb, mdl.ng, mdl.nl, mdl.nd, int(mdl.net.ref_bus)) != (m0.nb, m0.ng, m0.nl, m0.nd, int(m0.net.ref_bus)):
+            raise ValueError(f"{who} differs from scenario 0 in its sizes or reference bus")
+        arrs = self._acopf_arrays(mdl)
+        for name, a in arrs.items():
+            if name != "coef" and not np.array_equal(a, keep[name], equal_nan=a.dtype == np.float64):
+                raise ValueError(f"{who} differs from scenario 0 in {name}")
+        return arrs["coef"]
+
     def attach_acopf(self, model):
         """Hand the network of an ``examples.acopf.AcopfModel`` to the device so that ``eval_acopf`` /
         ``acopf_trial`` replace the host callbacks (``src/MOI_wrapper.jl:1047-1069``).
@@ -293,15 +333,9 @@ class SubLp:
             raise ValueError(f"attach_acopf: {len(models)} models for a batch of {self.batch}")
         m0 = models[0]
         keep = self._acopf_arrays(m0)
-        coefs = [keep["coef"]]
-        for k, mdl in enumerate(models[1:], 1):
-            if (mdl.nb, mdl.ng, mdl.nl, mdl.nd, int(mdl.net.ref_bus)) != (m0.nb, m0.ng, m0.nl, m0.nd, int(m0.net.ref_bus)):
-                raise ValueError(f"attach_acopf: scenario {k} differs from scenario 0 in its sizes or reference bus")
-            arrs = self._acopf_arrays(mdl)
-            for name, a in arrs.items():
-                if name != "coef" and not np.array_equal(a, keep[name], equal_nan=a.dtype == np.float64):
-                    raise ValueError(f"attach_acopf: scenario {k} differs from scenario 0 in {name}")
-            coefs.append(arrs["coef"])
+        self._acopf_ref = (m0, keep)
+        coefs = [keep["coef"]] + [self._acopf_coef(mdl, f"attach_acopf: scenario {k}") for k, mdl in
+                                  enumerate(models[1:], 1)]
         d = capi.AcopfDesc()
         d.nb, d.ng, d.nl, d.nd, d.ref_bus = m0.nb, m0.ng, m0.nl, m0.nd, int(m0.net.ref_bus)
         for k, a in keep.items():

@@ -304,6 +304,23 @@ int asm_kkt_device_selftest(int32_t n_cols, int32_t n_rows, const int64_t *row_p
  * phase, cost nothing and come back with status ASM_LP_SKIPPED and zeroed outputs. */
 int asm_slp_set_active(asm_slp *h, const int32_t *active);
 
+/* Continuous batching (a queue of scenarios longer than the batch): replace the scenarios held by k lanes of a batch
+ * and keep the handle, its symbolic analysis and its captured graphs.  lanes[k] distinct, in [0, batch);
+ * x_L/x_U[k][n], g_L/g_U[k][m] in the order of `lanes` (Model, model.jl:1-61, of the new scenario).  Every row keeps
+ * its class (equality / range / lower / upper, subproblem.jl:87-112: the restoration LP's layout is built from them):
+ * ASM_E_INVALID when one differs, ASM_E_FREE_ROW for a row with both bounds infinite, ASM_E_STATE on a handle created
+ * with shared bounds and batch > 1.  k = 0 is a no-op; padding lanes and the asm_slp_set_active mask are kept.
+ * The loaded lanes' next PDHG solves start cold in both phases.  Afterwards the handle is back in its state before an
+ * update: solve, extract, the reductions and asm_slp_get_lp answer ASM_E_STATE until the next asm_slp_update or
+ * asm_slp_eval_acopf. */
+int asm_slp_load_lanes(asm_slp *h, int32_t k, const int32_t *lanes, const double *x_L, const double *x_U,
+                       const double *g_L, const double *g_U);
+/* per-lane branch coefficients coef[k][12][nl] (asm_acopf_desc.coef order, finite) for the lanes `lanes` (as in
+ * asm_slp_load_lanes); the other lanes keep theirs.  Call after asm_slp_attach_acopf (ASM_E_STATE before).  On a
+ * handle that still shares its coefficients the first call broadcasts them into every lane first; the next attach
+ * returns the handle to shared coefficients. */
+int asm_slp_acopf_branch_coef_lanes(asm_slp *h, int32_t k, const int32_t *lanes, const double *coef);
+
 /* which engine the last asm_slp_solve used (1 streaming, 2 group, 3 both, 4 barrier), blocks per LP and LPs resident at once */
 int asm_slp_engine_info(asm_slp *h, int32_t *engine, int32_t *group_size, int32_t *groups);
 
