@@ -86,62 +86,49 @@ __global__ void __launch_bounds__(kThreads) k_aty(LpView v, const double *__rest
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < v.n; j += (int64_t)gridDim.x * blockDim.x)
         t[j] = spmv_row(v.AT, v.row_idx, w, v.col_ptr[j], v.col_ptr[j + 1], 1, 0);
 }
-// primal half with the completed K'y in `aty` (same arithmetic as k_primal)
+// primal half with the completed K'y in `aty`
 template <bool CHECK>
 __global__ void __launch_bounds__(kThreads) k_primal_t(LpView v, const double *__restrict__ aty, int jit) {
     const ScenState *st = v.state;
     const double tau = st->eta / st->omega;
-    const int kk = st->k0 + jit + 1;
-    const double w = (double)kk / ((double)kk + 1.0);
+    const double w = pdhg_halpern_weight(st->k0 + jit + 1);
     double acc[3] = {0.0, 0.0, 0.0};
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < v.n; j += (int64_t)gridDim.x * blockDim.x) {
         const double cj = v.cs[j], g = cj - aty[j], xv = v.x[j];
-        const double xpv = fmin(fmax(xv - tau * g, v.lbs[j]), v.ubs[j]);
-        const double xb = 2.0 * xpv - xv;
+        const double xpv = pdhg_primal_step(xv, g, tau, v.lbs[j], v.ubs[j]);
+        const double xb = pdhg_reflect(xpv, xv);
         v.xbar[j] = xb;
         if (CHECK) {
             v.xp[j] = xpv;
-            const double dx = xpv - xv, da = xpv - v.xa[j];
-            acc[0] += dx * dx;
-            acc[1] += da * da;
-            acc[2] += cj * xpv;
+            pdhg_col_terms(xpv, xv, v.xa[j], cj, acc[0], acc[1], acc[2]);
         } else {
-            v.x[j] = w * xb + (1.0 - w) * v.xa[j];
+            v.x[j] = pdhg_halpern(w, xb, v.xa[j]);
         }
     }
     if (CHECK) block_reduce_store<false, 3>(acc, 0u, v.partials, Q_DX2, 1);
 }
-// reduced costs from the completed K'yp (same arithmetic as k_dual_resid)
+// reduced costs from the completed K'yp
 __global__ void __launch_bounds__(kThreads) k_dual_resid_t(LpView v, const double *__restrict__ atyp) {
     const double inv_sc = 1.0 / v.state->sc;
     double acc[2] = {0.0, 0.0};
     for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < v.n; j += (int64_t)gridDim.x * blockDim.x) {
         const double rc = v.cs[j] - atyp[j];
         v.gyp[j] = rc;
-        const double xpv = v.xp[j], l = v.lbs[j], u = v.ubs[j];
-        const double rpos = (isfinite(l) && xpv <= l) ? fmax(rc, 0.0) : 0.0;
-        const double rneg = (isfinite(u) && xpv >= u) ? fmin(rc, 0.0) : 0.0;
-        const double res = (rc - rpos - rneg) * inv_sc / v.dc[j];
-        acc[0] += res * res;
-        acc[1] += (rpos > 0.0 ? l * rpos : 0.0) + (rneg < 0.0 ? u * rneg : 0.0);
+        pdhg_rc_terms(rc, v.xp[j], v.lbs[j], v.ubs[j], inv_sc, v.dc[j], acc[0], acc[1]);
     }
     block_reduce_store<false, 2>(acc, 0u, v.partials, Q_DRES2, 1);
 }
 __global__ void __launch_bounds__(kThreads) k_ray_cols_t(LpView v, const double *__restrict__ atr) {
     double acc[2] = {0.0, 0.0};
-    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < v.n; j += (int64_t)gridDim.x * blockDim.x) {
-        const double a = atr[j], t = -a;
-        acc[0] += t > 0.0 ? t * v.lbs[j] : (t < 0.0 ? t * v.ubs[j] : 0.0);
-        acc[1] = fmax(acc[1], fabs(a / v.dc[j]));
-    }
+    for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < v.n; j += (int64_t)gridDim.x * blockDim.x)
+        pdhg_ray_col_terms(atr[j], v.lbs[j], v.ubs[j], v.dc[j], acc[0], acc[1]);
     block_reduce_store<false, 2>(acc, 2u, v.partials, Q_RAY_COL, 1);
 }
 // second stage of the check reductions into qsum[Q_COUNT] / qmax[2]; column-side sums are replicated on every
 // rank, so only rank 0 contributes them to the all-reduce
 __global__ void __launch_bounds__(kFinalThreads) k_reduce_q(LpView v, int rank, double *qsum, double *qmax) {
     for (int i = 0; i < Q_COUNT; ++i) {
-        const bool rows = (i >= Q_DY2 && i <= Q_DOBJ_ROW) || i == Q_RAY_ROW || i == Q_RAY_MAX;
-        const bool is_max = (i == Q_RAY_MAX || i == Q_KTY_MAX);
+        const bool rows = (kQRows >> i) & 1u, is_max = (kQMax >> i) & 1u;
         const double q = final_reduce(v.partials, i, rows ? v.nbx_rows : v.nbx_cols, 1, 0, is_max);
         if (threadIdx.x == 0) {
             if (is_max) {
@@ -157,14 +144,14 @@ __global__ void k_merge_q(double *qsum, const double *qmax) {
     qsum[Q_RAY_MAX] = qmax[0];
     qsum[Q_KTY_MAX] = qmax[1];
 }
-// k_decide on completed sums (single LP)
+// the check decision on the completed sums (single LP)
 __global__ void k_decide_q(LpView v, const double *q, int jit, int steps) {
     ScenState st = *v.state;
     if (st.status >= 0) return;
-    group_decide(st, *v.prm, q, jit, steps, 0);
+    pdhg_decide(st, *v.prm, q, jit, steps, "pdhg-rows");
     *v.state = st;
 }
-// norms for k_init_state: psum = {c2, cun2 (replicated), q2, qun2 (local)}
+// norms for k_start_q: psum = {c2, cun2 (replicated), q2, qun2 (local)}
 __global__ void __launch_bounds__(kFinalThreads) k_reduce_prep(LpView v, int rank, double *psum) {
     const double c2 = final_reduce(v.partials, P_C2, v.nbx_cols, 1, 0, false);
     const double cun2 = final_reduce(v.partials, P_CUN2, v.nbx_cols, 1, 0, false);
@@ -177,30 +164,7 @@ __global__ void __launch_bounds__(kFinalThreads) k_reduce_prep(LpView v, int ran
         psum[3] = qun2;
     }
 }
-__global__ void k_init_state_q(LpView v, const double *psum) {
-    const double c2 = psum[0], cun2 = psum[1], q2 = psum[2], qun2 = psum[3];
-    ScenState st;
-    st.sb = 1.0 / (sqrt(q2) + 1.0);
-    st.sc = 1.0 / (sqrt(c2) + 1.0);
-    const double nc = sqrt(c2) * st.sc, nq = sqrt(q2) * st.sb;
-    st.omega = (nc > 0.0 && nq > 0.0) ? nc / nq : 1.0;
-    st.omega0 = st.omega;
-    st.eta = 0.998;
-    st.nq_un = sqrt(qun2);
-    st.nc_un = sqrt(cun2);
-    st.r0 = 0.0;
-    st.r_prev = INFINITY;
-    st.e_sum = 0.0;
-    st.e_prev = 0.0;
-    st.pobj = st.dobj = 0.0;
-    st.pres = st.dres = st.gap = INFINITY;
-    st.total = 0;
-    st.k0 = 0;
-    st.restarts = 0;
-    st.status = -1;
-    st.restart_flag = 0;
-    *v.state = st;
-}
+__global__ void k_start_q(LpView v, const double *psum) { *v.state = pdhg_start(psum[0], psum[1], psum[2], psum[3]); }
 
 // ---- host ------------------------------------------------------------------------------------------------------
 class DistLp {
@@ -280,7 +244,7 @@ class DistLp {
         ASM_KL(k_prepare_rows<false><<<gr.grid, gr.block, 0, stream>>>(v));
         ASM_KL(k_reduce_prep<<<1, kFinalThreads, 0, stream>>>(v, rank, psum.p));
         ASM_TRY(allreduce(psum.p, psum.p, 4, NcclApi::kSum));
-        ASM_KL(k_init_state_q<<<1, 1, 0, stream>>>(v, psum.p));
+        ASM_KL(k_start_q<<<1, 1, 0, stream>>>(v, psum.p));
         ASM_KL(k_prepare_finish<false><<<gm.grid, gm.block, 0, stream>>>(v, warm, (const int *)nullptr));
         ASM_CK(cudaGetLastError());
         return ASM_OK;
@@ -300,16 +264,7 @@ class DistLp {
         cudaStream_t stream = L.stream;
         int64_t &launches = L.launches;
         ASM_CK(cudaSetDevice(device));
-        DevParams dp;
-        dp.eps_rel = P.eps_rel;
-        dp.eps_infeas = P.eps_infeas;
-        dp.b_suf = P.restart_sufficient;
-        dp.b_nec = P.restart_necessary;
-        dp.b_art = P.restart_artificial;
-        dp.kp = P.pid_kp;
-        dp.ki = P.pid_ki;
-        dp.kd = P.pid_kd;
-        dp.balance = P.weight_balance;
+        DevParams dp = dev_params(P);
         dp.verbose = P.verbose && rank == 0;
         ASM_CK(cudaMemcpyAsync(L.prm.p, &dp, sizeof dp, cudaMemcpyHostToDevice, stream));
         ASM_CK(cudaStreamSynchronize(stream));
@@ -366,16 +321,7 @@ class DistLp {
         if (hs.status < 0) hs.status = ASM_LP_ITERATION_LIMIT;
         L.last_iters = hs.total;
         L.host_state[0] = hs;
-        if (info) {
-            info->status = hs.status;
-            info->restarts = hs.restarts;
-            info->iterations = hs.total;
-            info->objective = hs.pobj + hc0;
-            info->dual_objective = hs.dobj + hc0;
-            info->primal_residual = hs.pres;
-            info->dual_residual = hs.dres;
-            info->gap = hs.gap;
-        }
+        if (info) lp_info(hs, hc0, *info);
         L.has_solution = true;
         return ASM_OK;
     }

@@ -11,7 +11,8 @@
 //   k_dual<CHECK>     CSR pass  A xbar fused with the dual prox and Halpern step
 //   k_dual_resid      CSC pass  A'y+ for reduced costs / dual residual / dual objective   (check only)
 //   k_ray_rows/cols   Farkas certificate pieces                                          (check only)
-//   k_decide          one block per LP: deterministic second-stage reductions, termination, restart, PID
+//   k_decide          one block per LP: deterministic second-stage reductions, then pdhg_decide (pdhg.cuh):
+//                     termination, restart, PID
 //   k_apply           restart or Halpern update after a check
 //   k_ruiz_* / k_build_scaled / k_prepare_* / k_finalize   preconditioning and (un)scaling
 // A solve launches a CUDA graph of `check_every` iterations per host round trip; the only host<->device
@@ -22,48 +23,10 @@
 #include <map>
 #include <memory>
 
-#include "util.cuh"
+#include "pdhg.cuh"
 
 namespace asmb {
 
-struct ScenState {
-    double omega, omega0, eta, sb, sc;
-    double nq_un, nc_un;
-    double r0, r_prev, e_sum, e_prev;
-    double pobj, dobj, pres, dres, gap;
-    long long total;
-    int k0;
-    int restarts;
-    int status;        // -1 while running, else ASM_LP_*
-    int restart_flag;  // set by k_decide, consumed by k_apply
-};
-
-struct DevParams {
-    double eps_rel, eps_infeas;
-    double b_suf, b_nec, b_art;
-    double kp, ki, kd;
-    double balance;
-    int verbose;
-};
-
-// reduction slots
-enum {
-    Q_DX2 = 0,   // sum (xp - x)^2
-    Q_DXA2,      // sum (xp - xa)^2
-    Q_POBJ,      // sum cs * xp
-    Q_DY2,       // sum (yp - y)^2
-    Q_DYADX,     // sum dy * A dx
-    Q_DYA2,      // sum (yp - ya)^2
-    Q_PRES2,     // unscaled primal residual^2
-    Q_DOBJ_ROW,  // row part of the dual objective (scaled units)
-    Q_DRES2,     // unscaled dual residual^2
-    Q_DOBJ_COL,  // column part of the dual objective (scaled units)
-    Q_RAY_ROW,   // Farkas: sum rl*ray+ + ru*ray-   (scaled units)
-    Q_RAY_MAX,   // max |ray * dr|
-    Q_RAY_COL,   // Farkas: box support of -(A'ray)
-    Q_KTY_MAX,   // max |(A'ray)_j / dc_j|
-    Q_COUNT
-};
 constexpr int kPartialSlots = 16;  // rows of the partial buffer: Q_COUNT here, I_COUNT in ipm.cuh
 // preparation slots (reuse the same partial buffer)
 enum { P_C2 = 0, P_CUN2, P_Q2, P_QUN2, P_COUNT };
@@ -221,29 +184,7 @@ __global__ void __launch_bounds__(kFinalThreads) k_init_state(LpView v) {
     double cun2 = final_reduce(v.partials, P_CUN2, v.nbx_cols, B, s, false);
     double q2 = final_reduce(v.partials, P_Q2, v.nbx_rows, B, s, false);
     double qun2 = final_reduce(v.partials, P_QUN2, v.nbx_rows, B, s, false);
-    if (threadIdx.x == 0) {
-        ScenState st;
-        st.sb = 1.0 / (sqrt(q2) + 1.0);
-        st.sc = 1.0 / (sqrt(c2) + 1.0);
-        const double nc = sqrt(c2) * st.sc, nq = sqrt(q2) * st.sb;
-        st.omega = (nc > 0.0 && nq > 0.0) ? nc / nq : 1.0;
-        st.omega0 = st.omega;
-        st.eta = 0.998;  // ||A||_2 <= 1 after Pock-Chambolle (alpha = 1) scaling
-        st.nq_un = sqrt(qun2);
-        st.nc_un = sqrt(cun2);
-        st.r0 = 0.0;
-        st.r_prev = INFINITY;
-        st.e_sum = 0.0;
-        st.e_prev = 0.0;
-        st.pobj = st.dobj = 0.0;
-        st.pres = st.dres = st.gap = INFINITY;
-        st.total = 0;
-        st.k0 = 0;
-        st.restarts = 0;
-        st.status = -1;
-        st.restart_flag = 0;
-        v.state[s] = st;
-    }
+    if (threadIdx.x == 0) v.state[s] = pdhg_start(c2, cun2, q2, qun2);
 }
 // second pass: bound/objective rescaling and the starting point (x0, y0 are unscaled warm starts or 0)
 template <bool BATCH>
@@ -316,8 +257,7 @@ __global__ void __launch_bounds__(kThreads) k_primal(LpView v, int jit) {
     const ScenState *st = v.state + mp.s;
     const bool live = st->status < 0;
     const double tau = live ? st->eta / st->omega : 0.0;
-    const int kk = st->k0 + jit + 1;
-    const double w = (double)kk / ((double)kk + 1.0);
+    const double w = pdhg_halpern_weight(st->k0 + jit + 1);
     double acc[3] = {0.0, 0.0, 0.0};
     if (live) {
         for (int64_t j = mp.first; j < v.n; j += mp.stride) {
@@ -330,18 +270,15 @@ __global__ void __launch_bounds__(kThreads) k_primal(LpView v, int jit) {
             const double xav = CHECK ? 0.0 : v.xa[e];
             const double a = spmv_row(v.AT, v.row_idx, v.y, k, k1, B, mp.s);
             const double g = cj - a;
-            const double xpv = fmin(fmax(xv - tau * g, lo), up);
-            const double xb = 2.0 * xpv - xv;
+            const double xpv = pdhg_primal_step(xv, g, tau, lo, up);
+            const double xb = pdhg_reflect(xpv, xv);
             v.xbar[e] = xb;
             if (CHECK) {
                 v.xp[e] = xpv;
                 v.gy[e] = g;
-                const double dx = xpv - xv, da = xpv - v.xa[e];
-                acc[0] += dx * dx;
-                acc[1] += da * da;
-                acc[2] += cj * xpv;
+                pdhg_col_terms(xpv, xv, v.xa[e], cj, acc[0], acc[1], acc[2]);
             } else {
-                v.x[e] = w * xb + (1.0 - w) * xav;
+                v.x[e] = pdhg_halpern(w, xb, xav);
             }
         }
     }
@@ -357,8 +294,7 @@ __global__ void __launch_bounds__(kThreads) k_dual(LpView v, int jit) {
     const bool live = st->status < 0;
     const double sigma = live ? st->eta * st->omega : 1.0;
     const double isig = 1.0 / sigma;
-    const int kk = st->k0 + jit + 1;
-    const double w = (double)kk / ((double)kk + 1.0);
+    const double w = pdhg_halpern_weight(st->k0 + jit + 1);
     double acc[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
     if (live) {
         const double inv_sb = 1.0 / st->sb;
@@ -379,22 +315,12 @@ __global__ void __launch_bounds__(kThreads) k_dual(LpView v, int jit) {
             } else {
                 a = spmv_row(v.A, v.col_idx, v.xbar, k0, k1, B, mp.s);
             }
-            const double t = a - yv * isig;
-            const double ypv = t < l ? sigma * (l - t) : (t > u ? sigma * (u - t) : 0.0);
+            const double ypv = pdhg_dual_step(a, yv, sigma, isig, l, u);
             if (CHECK) {
                 v.yp[e] = ypv;
-                const double dy = ypv - yv, da = ypv - v.ya[e];
-                const double adx = 0.5 * (a - ax);  // A (xp - x)
-                const double axp = 0.5 * (a + ax);  // A xp
-                acc[0] += dy * dy;
-                acc[1] += dy * adx;
-                acc[2] += da * da;
-                const double viol = (axp < l ? l - axp : (axp > u ? axp - u : 0.0)) * inv_sb / v.dr[e];
-                acc[3] += viol * viol;
-                // dual objective: rl y+ + ru y- (scaled units; unused side may be infinite -> guard)
-                acc[4] += ypv > 0.0 ? l * ypv : (ypv < 0.0 ? u * ypv : 0.0);
+                pdhg_row_terms(ypv, yv, v.ya[e], a, ax, l, u, inv_sb, v.dr[e], acc[0], acc[1], acc[2], acc[3], acc[4]);
             } else {
-                v.y[e] = w * (2.0 * ypv - yv) + (1.0 - w) * yav;
+                v.y[e] = pdhg_halpern(w, pdhg_reflect(ypv, yv), yav);
             }
         }
     }
@@ -453,19 +379,18 @@ __global__ void __launch_bounds__(kThreads) k_primal2(LpView v, int jit) {
     const ScenState *sa = v.state + s0, *sb = sa + 1;
     const bool la = sa->status < 0, lb = sb->status < 0;
     const double ta = sa->eta / sa->omega, tb = sb->eta / sb->omega;
-    const int ka = sa->k0 + jit + 1, kb = sb->k0 + jit + 1;
-    const double wa = (double)ka / ((double)ka + 1.0), wb = (double)kb / ((double)kb + 1.0);
+    const double wa = pdhg_halpern_weight(sa->k0 + jit + 1), wb = pdhg_halpern_weight(sb->k0 + jit + 1);
     if (!__any_sync(0xffffffffu, la || lb)) return;
     for (int64_t j = mp.first; j < v.n; j += mp.stride) {
         const int k0 = v.col_ptr[j], k1 = v.col_ptr[j + 1];
         const double2 c = ld2(v.cs, j, B, s0), x = ld2(v.x, j, B, s0), lo = ld2(v.lbs, j, B, s0),
                       up = ld2(v.ubs, j, B, s0), xa = ld2(v.xa, j, B, s0);
         const double2 a = spmv_row2(v.AT, v.row_idx, v.y, k0, k1, B, s0);
-        const double pa = fmin(fmax(x.x - ta * (c.x - a.x), lo.x), up.x);
-        const double pb = fmin(fmax(x.y - tb * (c.y - a.y), lo.y), up.y);
-        const double ba = 2.0 * pa - x.x, bb = 2.0 * pb - x.y;
+        const double pa = pdhg_primal_step(x.x, c.x - a.x, ta, lo.x, up.x);
+        const double pb = pdhg_primal_step(x.y, c.y - a.y, tb, lo.y, up.y);
+        const double ba = pdhg_reflect(pa, x.x), bb = pdhg_reflect(pb, x.y);
         st2(v.xbar, j, B, s0, ba, bb, la, lb);
-        st2(v.x, j, B, s0, wa * ba + (1.0 - wa) * xa.x, wb * bb + (1.0 - wb) * xa.y, la, lb);
+        st2(v.x, j, B, s0, pdhg_halpern(wa, ba, xa.x), pdhg_halpern(wb, bb, xa.y), la, lb);
     }
 }
 __global__ void __launch_bounds__(kThreads) k_dual2(LpView v, int jit) {
@@ -475,18 +400,17 @@ __global__ void __launch_bounds__(kThreads) k_dual2(LpView v, int jit) {
     const bool la = sa->status < 0, lb = sb->status < 0;
     const double ga = la ? sa->eta * sa->omega : 1.0, gb = lb ? sb->eta * sb->omega : 1.0;
     const double ia = 1.0 / ga, ib = 1.0 / gb;
-    const int ka = sa->k0 + jit + 1, kb = sb->k0 + jit + 1;
-    const double wa = (double)ka / ((double)ka + 1.0), wb = (double)kb / ((double)kb + 1.0);
+    const double wa = pdhg_halpern_weight(sa->k0 + jit + 1), wb = pdhg_halpern_weight(sb->k0 + jit + 1);
     if (!__any_sync(0xffffffffu, la || lb)) return;
     for (int64_t i = mp.first; i < v.m; i += mp.stride) {
         const int k0 = v.row_ptr[i], k1 = v.row_ptr[i + 1];
         const double2 y = ld2(v.y, i, B, s0), l = ld2(v.rls, i, B, s0), u = ld2(v.rus, i, B, s0),
                       ya = ld2(v.ya, i, B, s0);
         const double2 a = spmv_row2(v.A, v.col_idx, v.xbar, k0, k1, B, s0);
-        const double t0 = a.x - y.x * ia, t1 = a.y - y.y * ib;
-        const double pa = t0 < l.x ? ga * (l.x - t0) : (t0 > u.x ? ga * (u.x - t0) : 0.0);
-        const double pb = t1 < l.y ? gb * (l.y - t1) : (t1 > u.y ? gb * (u.y - t1) : 0.0);
-        st2(v.y, i, B, s0, wa * (2.0 * pa - y.x) + (1.0 - wa) * ya.x, wb * (2.0 * pb - y.y) + (1.0 - wb) * ya.y, la, lb);
+        const double pa = pdhg_dual_step(a.x, y.x, ga, ia, l.x, u.x);
+        const double pb = pdhg_dual_step(a.y, y.y, gb, ib, l.y, u.y);
+        st2(v.y, i, B, s0, pdhg_halpern(wa, pdhg_reflect(pa, y.x), ya.x), pdhg_halpern(wb, pdhg_reflect(pb, y.y), ya.y),
+            la, lb);
     }
 }
 
@@ -508,13 +432,7 @@ __global__ void __launch_bounds__(kThreads) k_dual_resid(LpView v) {
                 a += v.AT[(int64_t)k * B + mp.s] * v.yp[(int64_t)v.row_idx[k] * B + mp.s];
             const double rc = v.cs[e] - a;
             v.gyp[e] = rc;
-            const double xpv = v.xp[e], l = v.lbs[e], u = v.ubs[e];
-            // reduced costs count as multipliers only where the iterate sits on a finite bound
-            const double rpos = (isfinite(l) && xpv <= l) ? fmax(rc, 0.0) : 0.0;
-            const double rneg = (isfinite(u) && xpv >= u) ? fmin(rc, 0.0) : 0.0;
-            const double res = (rc - rpos - rneg) * inv_sc / v.dc[e];
-            acc[0] += res * res;
-            acc[1] += (rpos > 0.0 ? l * rpos : 0.0) + (rneg < 0.0 ? u * rneg : 0.0);
+            pdhg_rc_terms(rc, v.xp[e], v.lbs[e], v.ubs[e], inv_sc, v.dc[e], acc[0], acc[1]);
         }
     }
     block_reduce_store<BATCH, 2>(acc, 0u, v.partials, Q_DRES2, B);
@@ -530,13 +448,10 @@ __global__ void __launch_bounds__(kThreads) k_ray_rows(LpView v) {
     if (live) {
         for (int64_t i = mp.first; i < v.m; i += mp.stride) {
             const int64_t e = i * B + mp.s;
-            double d = v.yp[e] - v.y[e];
             const double l = v.rls[e], u = v.rus[e];
-            if (!isfinite(l)) d = fmin(d, 0.0);
-            if (!isfinite(u)) d = fmax(d, 0.0);
+            const double d = pdhg_ray(v.yp[e] - v.y[e], l, u);
             v.ray[e] = d;
-            acc[0] += d > 0.0 ? l * d : (d < 0.0 ? u * d : 0.0);
-            acc[1] = fmax(acc[1], fabs(d * v.dr[e]));
+            pdhg_ray_row_terms(d, l, u, v.dr[e], acc[0], acc[1]);
         }
     }
     block_reduce_store<BATCH, 2>(acc, 2u, v.partials, Q_RAY_ROW, B);
@@ -554,10 +469,7 @@ __global__ void __launch_bounds__(kThreads) k_ray_cols(LpView v) {
             const int k1 = v.col_ptr[j + 1];
             for (int k = v.col_ptr[j]; k < k1; ++k)
                 a += v.AT[(int64_t)k * B + mp.s] * v.ray[(int64_t)v.row_idx[k] * B + mp.s];
-            // support of the box in direction -(A'ray): min over [lb, ub] of -(a) x
-            const double t = -a;
-            acc[0] += t > 0.0 ? t * v.lbs[e] : (t < 0.0 ? t * v.ubs[e] : 0.0);
-            acc[1] = fmax(acc[1], fabs(a / v.dc[e]));
+            pdhg_ray_col_terms(a, v.lbs[e], v.ubs[e], v.dc[e], acc[0], acc[1]);
         }
     }
     block_reduce_store<BATCH, 2>(acc, 2u, v.partials, Q_RAY_COL, B);
@@ -569,97 +481,13 @@ __global__ void __launch_bounds__(kFinalThreads) k_decide(LpView v, int jit, int
     ScenState *sp = v.state + s;
     if (sp->status >= 0) return;  // uniform per block
     double q[Q_COUNT];
-    for (int i = 0; i < Q_COUNT; ++i) {
-        const bool rows = (i >= Q_DY2 && i <= Q_DOBJ_ROW) || i == Q_RAY_ROW || i == Q_RAY_MAX;
-        const bool is_max = (i == Q_RAY_MAX || i == Q_KTY_MAX);
-        q[i] = final_reduce(v.partials, i, rows ? v.nbx_rows : v.nbx_cols, B, s, is_max);
-    }
+    for (int i = 0; i < Q_COUNT; ++i)
+        q[i] = final_reduce(v.partials, i, ((kQRows >> i) & 1u) ? v.nbx_rows : v.nbx_cols, B, s, (kQMax >> i) & 1u);
     if (threadIdx.x != 0) return;
     ScenState st = *sp;
     const DevParams P = *v.prm;
-    const double tau = st.eta / st.omega, sigma = st.eta * st.omega;
-    const int k = st.k0 + jit + 1;
-    const long long total = st.total + jit + 1;
-    double r2 = q[Q_DX2] / tau - 2.0 * q[Q_DYADX] + q[Q_DY2] / sigma;
-    const double r = sqrt(fmax(r2, 0.0));
-    const double unit = 1.0 / (st.sb * st.sc);
-    const double pobj = q[Q_POBJ] * unit;
-    const double dobj = (q[Q_DOBJ_ROW] + q[Q_DOBJ_COL]) * unit;
-    const double pres = sqrt(q[Q_PRES2]), dres = sqrt(q[Q_DRES2]);
-    const double gap = fabs(pobj - dobj);
-    st.pobj = pobj;
-    st.dobj = dobj;
-    st.pres = pres;
-    st.dres = dres;
-    st.gap = gap;
-    int status = -1;
-    if (pres <= P.eps_rel * (1.0 + st.nq_un) && dres <= P.eps_rel * (1.0 + st.nc_un) &&
-        gap <= P.eps_rel * (1.0 + fabs(pobj) + fabs(dobj)))
-        status = ASM_LP_OPTIMAL;
-    if (status < 0) {
-        // Farkas certificate: ray'rl+ + ray'ru- - max_box (K'ray)'x > 0  (all terms carry 1/(sb sc);
-        // normalise by ||ray||_inf in unscaled units = Q_RAY_MAX / sc)
-        const double nr = q[Q_RAY_MAX] / st.sc;
-        if (nr > 0.0) {
-            const double robj = (q[Q_RAY_ROW] + q[Q_RAY_COL]) * unit / nr;
-            const double kty = q[Q_KTY_MAX] / st.sc / nr;
-            if (robj > P.eps_infeas * fmax(1.0, kty)) status = ASM_LP_INFEASIBLE;
-        }
-    }
-    if (!(r == r) || !(pobj == pobj)) status = ASM_LP_NUMERICAL_ERROR;
-    int restart = 0;
-    if (status < 0) {
-        if (k == 1) {
-            st.r0 = r;
-        } else if (jit + 1 == steps_in_graph) {
-            if (r <= P.b_suf * st.r0)
-                restart = 1;
-            else if (r <= P.b_nec * st.r0 && r > st.r_prev)
-                restart = 1;
-            else if ((double)k >= P.b_art * (double)total)
-                restart = 1;
-        }
-        st.r_prev = r;
-        if (restart) {
-            // primal weight: PID controller on log(omega * |dx| / |dy|); the default gains (0.5, 0, 0) are the
-            // PDLP rule omega <- sqrt(omega * |dy| / |dx|).  Degenerate moves or a runaway weight fall back to
-            // the initial one.
-            const double ddx = sqrt(q[Q_DXA2]), ddy = sqrt(q[Q_DYA2]);
-            const double rp = pres / (1.0 + st.nq_un), rd = dres / (1.0 + st.nc_un);
-            if (P.balance > 0.0) {
-                // residual balancing: a larger weight shortens the primal step and lengthens the dual one, which
-                // drives the primal residual down faster -- move the weight towards equal relative residuals
-                if (rp > 0.0 && rd > 0.0) st.omega = exp(log(st.omega) + P.balance * log(rp / rd));
-            } else if (ddx > 1e-16 && ddy > 1e-16) {
-                const double e = log(st.omega * ddx / ddy);
-                st.e_sum += e;
-                const double dlog = -(P.kp * e + P.ki * st.e_sum + P.kd * (e - st.e_prev));
-                st.omega = exp(log(st.omega) + dlog);
-                st.e_prev = e;
-            }
-            if (!(st.omega > st.omega0 * 1e-16 && st.omega < st.omega0 * 1e16)) {
-                st.omega = st.omega0;
-                st.e_sum = 0.0;
-                st.e_prev = 0.0;
-            }
-            st.restarts += 1;
-            st.r_prev = INFINITY;
-        }
-    }
-    if (P.verbose && s == 0)
-        printf("[pdhg] it %lld k %d pres %.3e dres %.3e gap %.3e pobj %.10e r %.3e w %.3e restarts %d%s\n", total, k,
-               pres, dres, gap, pobj, r, st.omega, st.restarts, restart ? " R" : "");
-    st.restart_flag = restart;
-    if (jit + 1 == steps_in_graph) {
-        st.total += steps_in_graph;
-        st.k0 = restart ? 0 : st.k0 + steps_in_graph;
-    }
-    if (status >= 0) {
-        st.total = total;
-        st.status = status;
-        st.restart_flag = 2;  // k_apply: freeze at (xp, yp)
-        atomicSub(v.n_active, 1);
-    }
+    pdhg_decide(st, P, q, jit, steps_in_graph, s == 0 ? "pdhg" : nullptr);
+    if (st.status >= 0) atomicSub(v.n_active, 1);
     *sp = st;
 }
 
@@ -672,8 +500,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(LpView v, const int *__restr
     const ScenState *st = v.state + mp.s;
     const int flag = st->restart_flag;
     if (st->status >= 0 && flag != 2) return;
-    const int kk = kstep[mp.s];
-    const double w = (double)kk / ((double)kk + 1.0);
+    const double w = pdhg_halpern_weight(kstep[mp.s]);
     for (int64_t j = mp.first; j < v.n; j += mp.stride) {
         const int64_t e = j * B + mp.s;
         if (flag) {
@@ -681,7 +508,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(LpView v, const int *__restr
             v.x[e] = t;
             v.xa[e] = t;
         } else {
-            v.x[e] = w * v.xbar[e] + (1.0 - w) * v.xa[e];
+            v.x[e] = pdhg_halpern(w, v.xbar[e], v.xa[e]);
         }
     }
     for (int64_t i = mp.first; i < v.m; i += mp.stride) {
@@ -691,7 +518,7 @@ __global__ void __launch_bounds__(kThreads) k_apply(LpView v, const int *__restr
             v.y[e] = t;
             v.ya[e] = t;
         } else {
-            v.y[e] = w * (2.0 * v.yp[e] - v.y[e]) + (1.0 - w) * v.ya[e];
+            v.y[e] = pdhg_halpern(w, pdhg_reflect(v.yp[e], v.y[e]), v.ya[e]);
         }
     }
 }
@@ -1759,17 +1586,7 @@ class LpSolver {
                 graph_exec = nullptr;
             }
         }
-        DevParams dp;
-        dp.eps_rel = P.eps_rel;
-        dp.eps_infeas = P.eps_infeas;
-        dp.b_suf = P.restart_sufficient;
-        dp.b_nec = P.restart_necessary;
-        dp.b_art = P.restart_artificial;
-        dp.kp = P.pid_kp;
-        dp.ki = P.pid_ki;
-        dp.kd = P.pid_kd;
-        dp.balance = P.weight_balance;
-        dp.verbose = P.verbose;
+        const DevParams dp = dev_params(P);
         int *flag = (int *)pin_flag.p;
         DevParams *pdp = (DevParams *)((char *)pin_flag.p + 16);
         static_assert(sizeof(DevParams) + 16 <= 128, "pinned flag area too small");  // 9 doubles + int
@@ -1921,16 +1738,7 @@ class LpSolver {
             ScenState &st = host_state[s];
             if (st.status < 0) st.status = ASM_LP_ITERATION_LIMIT;
             last_iters = std::max<int64_t>(last_iters, st.total);
-            if (info) {
-                info[s].status = st.status;
-                info[s].restarts = st.restarts;
-                info[s].iterations = st.total;
-                info[s].objective = st.pobj + hc0[s];
-                info[s].dual_objective = st.dobj + hc0[s];
-                info[s].primal_residual = st.pres;
-                info[s].dual_residual = st.dres;
-                info[s].gap = st.gap;
-            }
+            if (info) lp_info(st, hc0[s], info[s]);
         }
         has_solution = true;
         return ASM_OK;

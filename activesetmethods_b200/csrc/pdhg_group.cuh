@@ -18,12 +18,13 @@
 //                           through distributed shared memory, and the cluster barrier publishes the stores
 //   GRID mode     G  > 16 : cooperative launch, barrier = one global counter per group
 // Groups pull LPs of the batch from an atomic queue, so every LP stops at its own convergence.
-// The KKT / restart / primal-weight logic is the one of lp_solver.cuh (k_decide), evaluated redundantly and
-// bit-identically by every block of the group from the same ordered partial sums.
+// The iteration's arithmetic and the check decision (KKT, restart, primal weight: pdhg_decide) are the ones of
+// pdhg.cuh; every block of the group takes the decision redundantly and bit-identically from the same ordered
+// partial sums.
 #pragma once
 #include <cooperative_groups.h>
 
-#include "util.cuh"
+#include "pdhg.cuh"
 
 namespace asmb {
 
@@ -268,93 +269,6 @@ __device__ __forceinline__ void block_reduce(double (&acc)[NQ], unsigned maxmask
     __syncthreads();
 }
 
-// the scalar decisions of one check (same logic as k_decide in lp_solver.cuh); returns the status (>= 0: done)
-__device__ inline void group_decide(ScenState &st, const DevParams &P, const double *q, int jit, int steps, int s) {
-    const double tau = st.eta / st.omega, sigma = st.eta * st.omega;
-    const int k = st.k0 + jit + 1;
-    const long long total = st.total + jit + 1;
-    const double r2 = q[Q_DX2] / tau - 2.0 * q[Q_DYADX] + q[Q_DY2] / sigma;
-    const double r = sqrt(fmax(r2, 0.0));
-    const double unit = 1.0 / (st.sb * st.sc);
-    const double pobj = q[Q_POBJ] * unit;
-    const double dobj = (q[Q_DOBJ_ROW] + q[Q_DOBJ_COL]) * unit;
-    const double pres = sqrt(q[Q_PRES2]), dres = sqrt(q[Q_DRES2]);
-    const double gap = fabs(pobj - dobj);
-    st.pobj = pobj;
-    st.dobj = dobj;
-    st.pres = pres;
-    st.dres = dres;
-    st.gap = gap;
-    int status = -1;
-    if (pres <= P.eps_rel * (1.0 + st.nq_un) && dres <= P.eps_rel * (1.0 + st.nc_un) &&
-        gap <= P.eps_rel * (1.0 + fabs(pobj) + fabs(dobj)))
-        status = ASM_LP_OPTIMAL;
-    double dbg_robj = 0.0, dbg_kty = 0.0, dbg_nr = 0.0;
-    if (status < 0) {
-        const double nr = q[Q_RAY_MAX] / st.sc;
-        if (nr > 0.0) {
-            const double robj = (q[Q_RAY_ROW] + q[Q_RAY_COL]) * unit / nr;
-            const double kty = q[Q_KTY_MAX] / st.sc / nr;
-            dbg_robj = robj;
-            dbg_kty = kty;
-            dbg_nr = nr;
-            if (robj > P.eps_infeas * fmax(1.0, kty)) status = ASM_LP_INFEASIBLE;
-        }
-    }
-    if (!(r == r) || !(pobj == pobj)) status = ASM_LP_NUMERICAL_ERROR;
-    int restart = 0;
-    if (status < 0) {
-        if (k == 1) {
-            st.r0 = r;
-        } else if (jit + 1 == steps) {
-            if (r <= P.b_suf * st.r0)
-                restart = 1;
-            else if (r <= P.b_nec * st.r0 && r > st.r_prev)
-                restart = 1;
-            else if ((double)k >= P.b_art * (double)total)
-                restart = 1;
-        }
-        st.r_prev = r;
-        if (restart) {
-            const double ddx = sqrt(q[Q_DXA2]), ddy = sqrt(q[Q_DYA2]);
-            const double rp = pres / (1.0 + st.nq_un), rd = dres / (1.0 + st.nc_un);
-            if (P.balance > 0.0) {
-                // residual balancing: a larger weight shortens the primal step and lengthens the dual one, which
-                // drives the primal residual down faster -- move the weight towards equal relative residuals
-                if (rp > 0.0 && rd > 0.0) st.omega = exp(log(st.omega) + P.balance * log(rp / rd));
-            } else if (ddx > 1e-16 && ddy > 1e-16) {
-                const double e = log(st.omega * ddx / ddy);
-                st.e_sum += e;
-                const double dlog = -(P.kp * e + P.ki * st.e_sum + P.kd * (e - st.e_prev));
-                st.omega = exp(log(st.omega) + dlog);
-                st.e_prev = e;
-            }
-            if (!(st.omega > st.omega0 * 1e-16 && st.omega < st.omega0 * 1e16)) {
-                st.omega = st.omega0;
-                st.e_sum = 0.0;
-                st.e_prev = 0.0;
-            }
-            st.restarts += 1;
-            st.r_prev = INFINITY;
-        }
-    }
-    if (P.verbose && s == 0 && blockIdx.x == 0)
-        printf("[pdhg-g] it %lld k %d pres %.3e dres %.3e gap %.3e pobj %.10e r %.3e w %.3e restarts %d%s | ray: obj %.3e "
-               "(row %.3e col %.3e) kty %.3e norm %.3e\n", total, k, pres, dres, gap, pobj, r, st.omega, st.restarts,
-               restart ? " R" : "", dbg_robj, q[Q_RAY_ROW] * unit, q[Q_RAY_COL] * unit, dbg_kty, dbg_nr);
-    st.restart_flag = restart;
-    if (jit + 1 == steps) {
-        st.total += steps;
-        st.k0 = restart ? 0 : st.k0 + steps;
-    }
-    if (status >= 0) {
-        st.total = total;
-        st.status = status;
-        st.restart_flag = 2;
-    }
-}
-
-
 // halo copy: shared[t] = vec[list[t]] (list sorted => neighbouring lanes hit neighbouring sectors)
 __device__ __forceinline__ void halo_fetch(double *__restrict__ dst, const double *__restrict__ vec,
                                            const int *__restrict__ list, int cnt) {
@@ -562,8 +476,7 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
             // step sizes and Halpern weights of this block of iterations (they only change at its last check)
             const double tau = st.eta / st.omega, sigma = st.eta * st.omega, isig = 1.0 / sigma;
             if (tid < a.steps) {
-                const int kk = st.k0 + tid + 1;
-                wtab[tid] = (double)kk / ((double)kk + 1.0);
+                wtab[tid] = pdhg_halpern_weight(st.k0 + tid + 1);
             }
             __syncthreads();
             for (int j = 0; j < a.steps && !done; ++j) {
@@ -579,15 +492,15 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                         const double acc = sell_dot<MATS>(t_val, gAT, t_idx, hy, p0, len, tl, __any_sync(0xffffffffu, tl));
                         const int gj = cmap[sl];
                         const double xv = sx[sl];
-                        const double xpv = fmin(fmax(xv - tau * (scc[sl] - acc), slb[sl]), sub[sl]);
-                        const double xb = 2.0 * xpv - xv;
+                        const double xpv = pdhg_primal_step(xv, scc[sl] - acc, tau, slb[sl], sub[sl]);
+                        const double xb = pdhg_reflect(xpv, xv);
                         if (gj >= 0) {
                             if (PUSH)
                                 push_halo(hx, spushC_ptr, spushC_dst, sl, xb, G == 1 ? -1 : rank);
                             else
                                 gx[gj] = xb;
                         }
-                        sx[sl] = w * xb + (1.0 - w) * sxa[sl];
+                        sx[sl] = pdhg_halpern(w, xb, sxa[sl]);
                     }
                     if (PUSH)
                         cluster_sync_dsm(G);
@@ -602,10 +515,8 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                         const double acc = sell_dot<MATS>(a_val, gA, a_idx, hx, p0, len, tl, __any_sync(0xffffffffu, tl));
                         const int gi = rmap[sl];
                         const double yv = sy[sl];
-                        const double t = acc - yv * isig;
-                        const double l = srl[sl], u = sru[sl];
-                        const double ypv = t < l ? sigma * (l - t) : (t > u ? sigma * (u - t) : 0.0);
-                        const double yn = w * (2.0 * ypv - yv) + (1.0 - w) * sya[sl];
+                        const double ypv = pdhg_dual_step(acc, yv, sigma, isig, srl[sl], sru[sl]);
+                        const double yn = pdhg_halpern(w, pdhg_reflect(ypv, yv), sya[sl]);
                         sy[sl] = yn;
                         if (gi >= 0) {
                             if (PUSH)
@@ -634,15 +545,13 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                     const int gj = cmap[sl];
                     if (gj < 0) continue;
                     const double cj = scc[sl], xv = sx[sl];
-                    const double xpv = fmin(fmax(xv - tau * (cj - s1), slb[sl]), sub[sl]);
-                    gx[gj] = 2.0 * xpv - xv;
-                    if (PUSH) push_halo(hx, spushC_ptr, spushC_dst, sl, 2.0 * xpv - xv, G == 1 ? -1 : rank);
+                    const double xpv = pdhg_primal_step(xv, cj - s1, tau, slb[sl], sub[sl]);
+                    const double xb = pdhg_reflect(xpv, xv);
+                    gx[gj] = xb;
+                    if (PUSH) push_halo(hx, spushC_ptr, spushC_dst, sl, xb, G == 1 ? -1 : rank);
                     gx2[gj] = xv;
                     gxp[gj] = xpv;
-                    const double dx = xpv - xv, da = xpv - sxa[sl];
-                    acc[Q_DX2] += dx * dx;
-                    acc[Q_DXA2] += da * da;
-                    acc[Q_POBJ] += cj * xpv;
+                    pdhg_col_terms(xpv, xv, sxa[sl], cj, acc[Q_DX2], acc[Q_DXA2], acc[Q_POBJ]);
                 }
                 group_sync<CLUSTER>(bar, epoch, G);
                 if (PUSH) cluster_sync_dsm(G);
@@ -663,25 +572,15 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                     const int gi = rmap[sl];
                     if (gi < 0) continue;
                     const double yv = sy[sl];
-                    const double t = s1 - yv * isig;
                     const double l = srl[sl], u = sru[sl];
-                    const double ypv = t < l ? sigma * (l - t) : (t > u ? sigma * (u - t) : 0.0);
+                    const double ypv = pdhg_dual_step(s1, yv, sigma, isig, l, u);
                     gyp[gi] = ypv;
-                    const double dy = ypv - yv, da = ypv - sya[sl];
-                    const double adx = 0.5 * (s1 - s2), axp = 0.5 * (s1 + s2);
-                    acc[Q_DY2] += dy * dy;
-                    acc[Q_DYADX] += dy * adx;
-                    acc[Q_DYA2] += da * da;
                     const double dri = v.dr[(size_t)gi * B + s];
-                    const double viol = (axp < l ? l - axp : (axp > u ? axp - u : 0.0)) * inv_sb / dri;
-                    acc[Q_PRES2] += viol * viol;
-                    acc[Q_DOBJ_ROW] += ypv > 0.0 ? l * ypv : (ypv < 0.0 ? u * ypv : 0.0);
-                    double dd = dy;
-                    if (!isfinite(l)) dd = fmin(dd, 0.0);
-                    if (!isfinite(u)) dd = fmax(dd, 0.0);
+                    pdhg_row_terms(ypv, yv, sya[sl], s1, s2, l, u, inv_sb, dri, acc[Q_DY2], acc[Q_DYADX], acc[Q_DYA2],
+                                   acc[Q_PRES2], acc[Q_DOBJ_ROW]);
+                    const double dd = pdhg_ray(ypv - yv, l, u);
                     gray[gi] = dd;
-                    acc[Q_RAY_ROW] += dd > 0.0 ? l * dd : (dd < 0.0 ? u * dd : 0.0);
-                    acc[Q_RAY_MAX] = fmax(acc[Q_RAY_MAX], fabs(dd * dri));
+                    pdhg_ray_row_terms(dd, l, u, dri, acc[Q_RAY_ROW], acc[Q_RAY_MAX]);
                 }
                 group_sync<CLUSTER>(bar, epoch, G);
                 halo_fetch(hy, gyp, listC, d.haloC_cnt);
@@ -703,19 +602,13 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                     grc[gj] = rc;
                     const double xpv = gxp[gj], l = slb[sl], u = sub[sl];
                     const double dcj = v.dc[(size_t)gj * B + s];
-                    const double rpos = (isfinite(l) && xpv <= l) ? fmax(rc, 0.0) : 0.0;
-                    const double rneg = (isfinite(u) && xpv >= u) ? fmin(rc, 0.0) : 0.0;
-                    const double res = (rc - rpos - rneg) * inv_sc / dcj;
-                    acc[Q_DRES2] += res * res;
-                    acc[Q_DOBJ_COL] += (rpos > 0.0 ? l * rpos : 0.0) + (rneg < 0.0 ? u * rneg : 0.0);
-                    const double t = -s2;
-                    acc[Q_RAY_COL] += t > 0.0 ? t * l : (t < 0.0 ? t * u : 0.0);
-                    acc[Q_KTY_MAX] = fmax(acc[Q_KTY_MAX], fabs(s2 / dcj));
+                    pdhg_rc_terms(rc, xpv, l, u, inv_sc, dcj, acc[Q_DRES2], acc[Q_DOBJ_COL]);
+                    pdhg_ray_col_terms(s2, l, u, dcj, acc[Q_RAY_COL], acc[Q_KTY_MAX]);
                 }
-                block_reduce<Q_COUNT>(acc, (1u << Q_RAY_MAX) | (1u << Q_KTY_MAX), scratch, part + (size_t)rank * Q_COUNT);
+                block_reduce<Q_COUNT>(acc, kQMax, scratch, part + (size_t)rank * Q_COUNT);
                 group_sync<CLUSTER>(bar, epoch, G);
                 if (tid < Q_COUNT) {
-                    const bool is_max = (tid == Q_RAY_MAX || tid == Q_KTY_MAX);
+                    const bool is_max = (kQMax >> tid) & 1u;
                     double t = __ldcg(part + tid);
                     for (int r = 1; r < G; ++r) {
                         const double u = __ldcg(part + (size_t)r * Q_COUNT + tid);
@@ -724,7 +617,7 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                     qred[tid] = t;
                 }
                 __syncthreads();
-                if (tid == 0) group_decide(st, P, qred, j, a.steps, s);
+                if (tid == 0) pdhg_decide(st, P, qred, j, a.steps, s == 0 && blockIdx.x == 0 ? "pdhg-g" : nullptr);
                 __syncthreads();
                 const int flag = st.restart_flag;
                 // ------------------------------ apply: restart / freeze, or finish the Halpern step
@@ -736,7 +629,7 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                         sx[sl] = xpv;
                         sxa[sl] = xpv;
                     } else {
-                        sx[sl] = w * (2.0 * xpv - sx[sl]) + (1.0 - w) * sxa[sl];
+                        sx[sl] = pdhg_halpern(w, pdhg_reflect(xpv, sx[sl]), sxa[sl]);
                     }
                 }
                 for (int sl = tid; sl < d.nSR * 32; sl += kGThreads) {
@@ -748,7 +641,7 @@ __global__ void __launch_bounds__(kGThreads, 1) k_pdhg_group(const GroupArgs a) 
                         yn = ypv;
                         sya[sl] = ypv;
                     } else {
-                        yn = w * (2.0 * ypv - sy[sl]) + (1.0 - w) * sya[sl];
+                        yn = pdhg_halpern(w, pdhg_reflect(ypv, sy[sl]), sya[sl]);
                     }
                     sy[sl] = yn;
                     gy[gi] = yn;
