@@ -1105,10 +1105,14 @@ int asm_lp_get_col_dual(asm_lp *h, double *dual_lb, double *dual_ub) {
 int asm_lp_set_start(asm_lp *h, const double *x, const double *y) {
     if (!h) return fail(ASM_E_INVALID, "null argument");
     ASM_CK(cudaSetDevice(h->device));
+    // a NULL side starts cold: zero is the cold start of both sides (k_prepare_finish), and whatever the last
+    // solve left there (a Farkas direction, an unconverged point) must not ride along with the caller's other side
     if (x) ASM_TRY(h->put(x, h->s.n, h->s.Buser, h->s.xo.p));
+    else ASM_TRY(h->s.xo.zero(h->s.stream));
     if (y) ASM_TRY(h->put(y, h->s.m, h->s.Buser, h->s.yo.p));
+    else if (h->s.m) ASM_TRY(h->s.yo.zero(h->s.stream));
     ASM_CK(cudaStreamSynchronize(h->s.stream));
-    h->s.has_solution = true;
+    h->s.accept_start();
     return ASM_OK;
 }
 

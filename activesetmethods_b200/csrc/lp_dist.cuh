@@ -245,7 +245,7 @@ class DistLp {
         ASM_KL(k_reduce_prep<<<1, kFinalThreads, 0, stream>>>(v, rank, psum.p));
         ASM_TRY(allreduce(psum.p, psum.p, 4, NcclApi::kSum));
         ASM_KL(k_start_q<<<1, 1, 0, stream>>>(v, psum.p));
-        ASM_KL(k_prepare_finish<false><<<gm.grid, gm.block, 0, stream>>>(v, warm, (const int *)nullptr));
+        ASM_KL(k_prepare_finish<false><<<gm.grid, gm.block, 0, stream>>>(v, warm, (const int *)(warm ? L.d_prev_ok.p : nullptr)));
         ASM_CK(cudaGetLastError());
         return ASM_OK;
     }
@@ -269,7 +269,9 @@ class DistLp {
         ASM_CK(cudaMemcpyAsync(L.prm.p, &dp, sizeof dp, cudaMemcpyHostToDevice, stream));
         ASM_CK(cudaStreamSynchronize(stream));
         L.tiny_rel = P.tiny_rel > 0.0 ? P.tiny_rel : kTinyRel;
-        ASM_TRY(precondition(P.ruiz_iters, (P.warm_start && L.has_solution) ? (int)P.warm_start : 0));
+        const int warm = (P.warm_start && L.has_solution) ? (int)P.warm_start : 0;
+        if (warm) ASM_TRY(L.upload_start_ok());   // the single-GPU rule: every rank holds the same decision
+        ASM_TRY(precondition(P.ruiz_iters, warm));
         const int steps = std::max(2, (int)P.check_every);
         LpView v = L.view();
         const int n = L.n, m = L.m;
@@ -321,6 +323,7 @@ class DistLp {
         if (hs.status < 0) hs.status = ASM_LP_ITERATION_LIMIT;
         L.last_iters = hs.total;
         L.host_state[0] = hs;
+        L.start_ok[0] = hs.status == ASM_LP_OPTIMAL;
         if (info) lp_info(hs, hc0, *info);
         L.has_solution = true;
         return ASM_OK;

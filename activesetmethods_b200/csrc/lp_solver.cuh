@@ -191,8 +191,8 @@ template <bool BATCH>
 __global__ void __launch_bounds__(kThreads) k_prepare_finish(LpView v, int warm_all, const int *__restrict__ prev_ok) {
     Map<BATCH> mp;
     const int B = v.B;
-    // a scenario is warm-started only from an OPTIMAL previous solve: after INFEASIBLE the stored duals are a growing
-    // Farkas direction, after an iteration limit an unconverged point
+    // a scenario is warm-started only from an OPTIMAL previous solve or a start the caller set (LpSolver::start_ok):
+    // after INFEASIBLE the stored duals are a growing Farkas direction, after an iteration limit an unconverged point
     const int warm = (warm_all && (!prev_ok || prev_ok[mp.s])) ? warm_all : 0;
     const double sb = v.state[mp.s].sb, sc = v.state[mp.s].sc;
     for (int64_t j = mp.first; j < v.n; j += mp.stride) {
@@ -657,7 +657,10 @@ class LpSolver {
     int homeB = 0, homeBuser = 0;
     int compactions = 0;
     int last_engine = 0, last_G = 0, last_groups = 0;
-    DBuf<int> d_prev_ok;              // per scenario: the previous solve ended OPTIMAL (gates the PDHG warm start)
+    // per scenario: xo / yo hold a start the next warm PDHG solve may use -- set by asm_lp_set_start and by an OPTIMAL
+    // solve, cleared by any other outcome (a Farkas direction or an unconverged point) and by forget_warm_start
+    std::vector<int> start_ok;
+    DBuf<int> d_prev_ok;              // start_ok on the device (gates k_prepare_finish)
     DBuf<int> d_active;               // asm_slp_set_active: mask of the scenarios the next solves work on
     int n_masked = -1;                // number of active scenarios of the mask; -1 = no mask
     std::unique_ptr<IpmEngine> ipm;   // barrier engine (ipm.cuh), built at the first solve that uses it
@@ -762,6 +765,7 @@ class LpSolver {
         ASM_TRY(kstep.alloc(B));
         ASM_TRY(pin_flag.reserve(64));
         host_state.resize(B);
+        start_ok.assign(B, 0);
         ASM_TRY(c0.zero(stream));
         ASM_TRY(xo.zero(stream));
         ASM_TRY(yo.zero(stream));
@@ -967,10 +971,11 @@ class LpSolver {
                 ASM_KB(k_dual_resid, gc, v);
                 ASM_KB(k_ray_rows, gr, v);
                 ASM_KB(k_ray_cols, gc, v);
-                ASM_KL(k_store_kstep<<<(B + 127) / 128, 128, 0, stream>>>(state.p, kstep.p, j, B));
+                // v.state: after a compaction the running LPs' states live in the working set, not in `state`
+                ASM_KL(k_store_kstep<<<(B + 127) / 128, 128, 0, stream>>>(v.state, kstep.p, j, B));
                 ASM_KL(k_decide<<<B, kFinalThreads, 0, stream>>>(v, j, steps));
                 ASM_KB(k_apply, gm, v, kstep.p);
-                ASM_KL(k_after_apply<<<(B + 127) / 128, 128, 0, stream>>>(state.p, B));
+                ASM_KL(k_after_apply<<<(B + 127) / 128, 128, 0, stream>>>(v.state, B));
             } else if (B % 64 == 0) {
                 Geo g2c = gc, g2r = gr;
                 g2c.grid.y = g2r.grid.y = B / 64;
@@ -1370,11 +1375,27 @@ class LpSolver {
         return ASM_OK;
     }
 
-    // the scenarios in `lanes` were replaced: their next PDHG solve starts cold (d_prev_ok is built from host_state at
-    // the start of a warm solve).  The barrier engine keeps nothing across solves.
+    // the scenarios in `lanes` were replaced: their next PDHG solve starts cold.  The barrier engine keeps nothing
+    // across solves.
     void forget_warm_start(const int32_t *lanes, int k) {
         for (int j = 0; j < k; ++j)
-            if (lanes[j] < (int)host_state.size()) host_state[lanes[j]].status = ASM_LP_SKIPPED;
+            if (lanes[j] >= 0 && lanes[j] < (int)start_ok.size()) start_ok[lanes[j]] = 0;
+    }
+
+    // the caller's start (asm_lp_set_start) is used by the next warm solve of every scenario, whatever ended the last
+    void accept_start() {
+        std::fill(start_ok.begin(), start_ok.end(), 1);
+        has_solution = true;
+    }
+
+    // start_ok -> d_prev_ok for the warm solve about to be preconditioned
+    int upload_start_ok() {
+        if (d_prev_ok.n < (size_t)B) ASM_TRY(d_prev_ok.alloc(B));
+        std::vector<int> ok(B, 0);
+        for (int s = 0; s < Buser; ++s) ok[s] = start_ok[s];
+        ASM_CK(cudaMemcpyAsync(d_prev_ok.p, ok.data(), sizeof(int) * B, cudaMemcpyHostToDevice, stream));
+        ASM_CK(cudaStreamSynchronize(stream));
+        return ASM_OK;
     }
 
     // ---- barrier engine: Mehrotra predictor-corrector on the fixed-pattern L D L' (ipm.cuh) ----------------------
@@ -1605,13 +1626,7 @@ class LpSolver {
             use_ipm = false;
         }
         const int warm = (!use_ipm && P.warm_start && has_solution) ? (int)P.warm_start : 0;
-        if (warm) {
-            if (d_prev_ok.n < (size_t)B) ASM_TRY(d_prev_ok.alloc(B));
-            std::vector<int> ok(B, 0);
-            for (int s = 0; s < Buser; ++s) ok[s] = host_state[s].status == ASM_LP_OPTIMAL;
-            ASM_CK(cudaMemcpyAsync(d_prev_ok.p, ok.data(), sizeof(int) * B, cudaMemcpyHostToDevice, stream));
-            ASM_CK(cudaStreamSynchronize(stream));
-        }
+        if (warm) ASM_TRY(upload_start_ok());
         ASM_TRY(precondition(P.ruiz_iters, warm));
         if (n_masked >= 0) {
             ASM_KL(k_apply_mask<<<(Buser + 127) / 128, 128, 0, stream>>>(state.p, d_active.p, Buser));
@@ -1737,6 +1752,7 @@ class LpSolver {
         for (int s = 0; s < Buser; ++s) {
             ScenState &st = host_state[s];
             if (st.status < 0) st.status = ASM_LP_ITERATION_LIMIT;
+            start_ok[s] = st.status == ASM_LP_OPTIMAL;
             last_iters = std::max<int64_t>(last_iters, st.total);
             if (info) lp_info(st, hc0[s], info[s]);
         }

@@ -128,7 +128,11 @@ int asm_lp_get_row_dual(asm_lp *h, double *y);
 /* MOI.get(ConstraintDual) on the two bound constraints of every column (subproblem.jl:519-520):
  * dual_lb >= 0 (GreaterThan), dual_ub <= 0 (LessThan); either pointer may be NULL */
 int asm_lp_get_col_dual(asm_lp *h, double *dual_lb, double *dual_ub);
-/* warm start for the next solve (used when params.warm_start = 1); either pointer may be NULL */
+/* warm start for the next solve (used when params.warm_start = 1, y also with 2); either pointer may be NULL: that
+ * side then starts cold (x = 0 clipped to the bounds, y = 0), never from what the previous solve left.  A warm solve starts an LP from the handle's stored (x, y) only when that
+ * start is sound: after asm_lp_set_start (whatever ended the previous solve) or after a solve that ended
+ * ASM_LP_OPTIMAL.  After any other outcome (a Farkas direction, an unconverged point) the LP starts cold until the
+ * next set_start.  x is clipped to the column bounds, y projected onto the sign cone of the infinite row sides. */
 int asm_lp_set_start(asm_lp *h, const double *x, const double *y);
 
 /* ---- row-partitioned single LP (SURVEY.md 8(e): one very large instance over several GPUs) -----------------
