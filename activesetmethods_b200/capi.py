@@ -51,6 +51,19 @@ class AcopfDesc(C.Structure):
     ]
 
 
+class QcqpDesc(C.Structure):
+    _fields_ = [
+        ("n", C.c_int32), ("m", C.c_int32), ("nnz_coo", C.c_int64), ("c0", C.c_double),
+        ("n_obj_aff", C.c_int32), ("n_obj_quad", C.c_int32),
+        ("obj_aff_col", c_int32_p), ("obj_aff_coef", c_double_p),
+        ("obj_quad_i", c_int32_p), ("obj_quad_j", c_int32_p), ("obj_quad_coef", c_double_p),
+        ("n_aff", C.c_int64), ("n_quad", C.c_int64),
+        ("aff_row", c_int32_p), ("aff_col", c_int32_p), ("aff_coef", c_double_p), ("aff_pos", c_int64_p),
+        ("quad_row", c_int32_p), ("quad_i", c_int32_p), ("quad_j", c_int32_p), ("quad_coef", c_double_p),
+        ("quad_pos", c_int64_p),
+    ]
+
+
 class AsmError(RuntimeError):
     def __init__(self, code, msg):
         super().__init__(f"asm_b200 error {code}: {msg}")
@@ -105,6 +118,9 @@ SIGNATURES = {
     "asm_slp_eval_acopf": (C.c_int, [_VP, c_double_p, c_double_p, C.c_int32]),
     "asm_slp_get_eval": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, c_double_p]),
     "asm_slp_acopf_trial": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, C.c_int32, c_double_p]),
+    "asm_slp_attach_qcqp": (C.c_int, [_VP, C.POINTER(QcqpDesc)]),
+    "asm_slp_eval_qcqp": (C.c_int, [_VP, c_double_p, c_double_p, C.c_int32]),
+    "asm_slp_qcqp_trial": (C.c_int, [_VP, c_double_p, c_double_p, c_double_p, C.c_int32, c_double_p]),
     "asm_slp_launch_count": (C.c_int64, [_VP]),
     "asm_slp_last_solve_timing": (C.c_int, [_VP, c_double_p, c_int64_p]),
     "asm_plan_check": (C.c_int, [C.c_int32, C.c_int32, c_int64_p, c_int32_p, C.c_int32, c_int64_p, c_int32_p,

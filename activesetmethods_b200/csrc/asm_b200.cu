@@ -449,6 +449,93 @@ __global__ void k_acopf_misc(AcopfDev a, AcopfIo io, int n) {
     }
 }
 
+// =================================== device-side QCQP evaluator =================================================
+// The evaluator of the ACOPF section above for any model whose objective and rows are affine or quadratic
+// (asm_qcqp_desc).  Attach turns the term lists into three owner-computes layouts, so that every output has exactly
+// one writer and no atomics are needed:
+//   rows:     per row, its terms (affine, then quadratic, in term order) and its j_str positions in ascending order,
+//             each with the list of derivative contributions it receives (affine first, then quadratic, term order);
+//   columns:  per column, the contributions of the objective terms to its gradient entry (same order);
+//   f:        the objective terms, reduced per scenario in a fixed order.
+// A term or contribution is (c, i, j) with j = -1 for c * x_i and, in the contribution lists, i = -1 for the
+// constant c.  Products and sums are rounded one operation at a time (no FMA contraction): every output is the plain
+// left-to-right sum of its terms, whose error the tests bound a priori, and two calls agree bit for bit.
+struct QcqpDev {
+    int n = 0, m = 0, n_obj = 0;
+    double c0 = 0.0;
+    const int64_t *row_ptr, *pos_ptr, *con_ptr, *col_ptr;   // [m+1], [m+1], [nnz_coo+1], [n+1]
+    const int *term_i, *term_j, *pos, *con_i, *grad_i, *obj_i, *obj_j;
+    const double *term_c, *con_c, *grad_c, *obj_c;
+};
+__device__ __forceinline__ double qcqp_term(double c, double xi, double xj, bool quad) {
+    const double cx = __dmul_rn(c, xi);
+    return quad ? __dmul_rn(cx, xj) : cx;
+}
+// one row per item: E and the row's own Jacobian positions (derivatives skipped when TRIAL)
+template <bool BATCH, bool TRIAL>
+__global__ void __launch_bounds__(kThreads) k_qcqp_rows(QcqpDev q, AcopfIo io) {
+    Map<BATCH> mp;
+    const int B = io.B, s = mp.s;
+    for (int64_t r = mp.first; r < q.m; r += mp.stride) {
+        double acc = 0.0;
+        for (int64_t t = q.row_ptr[r]; t < q.row_ptr[r + 1]; ++t) {
+            const int j = q.term_j[t];
+            const double xi = acopf_x<TRIAL>(io, q.term_i[t], s);
+            const double xj = j >= 0 ? acopf_x<TRIAL>(io, j, s) : 0.0;
+            acc = __dadd_rn(acc, qcqp_term(q.term_c[t], xi, xj, j >= 0));
+        }
+        io.E[r * B + s] = acc;
+        if (!TRIAL) {
+            for (int64_t k = q.pos_ptr[r]; k < q.pos_ptr[r + 1]; ++k) {
+                double d = 0.0;
+                for (int64_t c = q.con_ptr[k]; c < q.con_ptr[k + 1]; ++c) {
+                    const int v = q.con_i[c];
+                    d = __dadd_rn(d, v >= 0 ? __dmul_rn(q.con_c[c], acopf_x<false>(io, v, s)) : q.con_c[c]);
+                }
+                io.dE[(int64_t)q.pos[k] * B + s] = d;
+            }
+        }
+    }
+}
+// one column per item: the gradient entry from the column's objective contributions
+template <bool BATCH>
+__global__ void __launch_bounds__(kThreads) k_qcqp_grad(QcqpDev q, AcopfIo io) {
+    Map<BATCH> mp;
+    const int B = io.B, s = mp.s;
+    for (int64_t j = mp.first; j < q.n; j += mp.stride) {
+        double d = 0.0;
+        for (int64_t c = q.col_ptr[j]; c < q.col_ptr[j + 1]; ++c) {
+            const int v = q.grad_i[c];
+            d = __dadd_rn(d, v >= 0 ? __dmul_rn(q.grad_c[c], acopf_x<false>(io, v, s)) : q.grad_c[c]);
+        }
+        io.df[j * B + s] = d;
+    }
+}
+// f per scenario: one block of kThreads per 32 scenarios (B > 1), one block of kWarps threads (B = 1).  Part t of a
+// scenario (a warp's lane, or a thread) sums the terms t, t + T, ... (T = kWarps parts), then the T partial sums are
+// added in part order, then c0: a fixed order that depends neither on the other lanes nor on the batch width.
+template <bool BATCH, bool TRIAL>
+__global__ void __launch_bounds__(kThreads) k_qcqp_obj(QcqpDev q, AcopfIo io) {
+    constexpr int T = kWarps;
+    __shared__ double sm[T][BATCH ? 32 : 1];
+    const int lane = BATCH ? (threadIdx.x & 31) : 0, t = BATCH ? (threadIdx.x >> 5) : threadIdx.x;
+    const int s = BATCH ? blockIdx.y * 32 + lane : 0;
+    double acc = 0.0;
+    for (int k = t; k < q.n_obj; k += T) {
+        const int j = q.obj_j[k];
+        const double xi = acopf_x<TRIAL>(io, q.obj_i[k], s);
+        const double xj = j >= 0 ? acopf_x<TRIAL>(io, j, s) : 0.0;
+        acc = __dadd_rn(acc, qcqp_term(q.obj_c[k], xi, xj, j >= 0));
+    }
+    sm[t][lane] = acc;
+    __syncthreads();
+    if (t == 0) {
+        double f = sm[0][lane];
+        for (int w = 1; w < T; ++w) f = __dadd_rn(f, sm[w][lane]);
+        io.f[s] = __dadd_rn(q.c0, f);
+    }
+}
+
 // =================================== host side: pattern analysis ================================================
 struct Pattern {
     int n = 0, m = 0;
@@ -527,6 +614,12 @@ struct SlpHandle {
     DBuf<int> ac_f, ac_t, ac_bal_ptr, ac_bal_col;
     DBuf<double> ac_coef, ac_gs, ac_bs, ac_c2, ac_c1, ac_c0, ac_loss1, ac_bal_coef, ac_ftrial;
     DBuf<double> ac_coef_scen;   // per-scenario branch coefficients [12 nl][B] (asm_slp_acopf_branch_coef)
+    // device-side QCQP evaluator (optional; a handle holds it or the ACOPF one)
+    bool has_qcqp = false;
+    QcqpDev qcqp;
+    DBuf<int64_t> qc_row_ptr, qc_pos_ptr, qc_con_ptr, qc_col_ptr;
+    DBuf<int> qc_term_i, qc_term_j, qc_pos, qc_con_i, qc_grad_i, qc_obj_i, qc_obj_j;
+    DBuf<double> qc_term_c, qc_con_c, qc_grad_c, qc_obj_c, qc_ftrial;
     // asm_slp_load_lanes / asm_slp_acopf_branch_coef_lanes: the lane list on the device
     DBuf<int> d_lanes;
     cudaEvent_t lanes_ev = nullptr;
@@ -923,6 +1016,59 @@ struct SlpHandle {
         }
         if (hstatus) ASM_CK(cudaMemcpyAsync(hstatus, d_status.p, Buser * sizeof(int), cudaMemcpyDeviceToHost, stream));
         ASM_CK(cudaStreamSynchronize(stream));
+        return ASM_OK;
+    }
+
+    // host part of a device-side evaluation (both evaluators): x[Buser][n] and delta[Buser] to the device
+    int eval_inputs(const double *hx, const double *hdelta) {
+        ASM_TRY(put(hx, n, Buser, xk.p));
+        double *ps = (double *)pin_small.p;
+        for (int s = 0; s < B; ++s) ps[s] = hdelta[s < Buser ? s : 0];
+        ASM_CK(cudaMemcpyAsync(delta.p, ps, B * sizeof(double), cudaMemcpyHostToDevice, stream));
+        return ASM_OK;
+    }
+    // host part of a trial evaluation (both evaluators) before its kernels: the step of the last solve, nu, alpha
+    int trial_inputs(const double *halpha, const double *hnu) {
+        ASM_TRY(extract_device());
+        ASM_TRY(put(hnu, m, Buser, tmp_m2.p));
+        double *ps = (double *)pin_small.p + (size_t)B * R_COUNT;
+        for (int s = 0; s < B; ++s) ps[s] = halpha[s < Buser ? s : 0];
+        ASM_CK(cudaMemcpyAsync(d_alpha.p, ps, sizeof(double) * B, cudaMemcpyHostToDevice, stream));
+        return ASM_OK;
+    }
+    // after a trial evaluation wrote g(x + alpha p) to tmp_m and f(x + alpha p) to ftrial: compute_phi through k_merit
+    int trial_merit(const double *halpha, const double *hbase, int feas, const double *ftrial, double *out) {
+        SlpView sv = view();
+        const Geo g = geo_for(m, B);
+        SLP_KB(k_merit, g, sv, (const double *)tmp_m.p, tmp_m2.p, pslack.p, (const double *)d_alpha.p, feas,
+               partials.p);
+        std::vector<double> r;
+        ASM_TRY(finish_reduce(g.grid.x, 0u, r));
+        std::vector<double> ft(B, 0.0);
+        ASM_CK(cudaMemcpyAsync(ft.data(), ftrial, sizeof(double) * B, cudaMemcpyDeviceToHost, stream));
+        ASM_CK(cudaStreamSynchronize(stream));
+        for (int s = 0; s < Buser; ++s) {
+            const double b0 = feas ? hbase[s] + halpha[s] * r[s * R_COUNT + R_B] : ft[s];
+            out[s] = b0 + r[s * R_COUNT + R_A];
+        }
+        return ASM_OK;
+    }
+    // the QCQP evaluator's kernels at xk (+ alpha p when TRIAL), outputs as in io
+    template <bool TRIAL>
+    int qcqp_launch(const AcopfIo &io) {
+        const Geo gr = geo_for(std::max(m, 1), B), gc = geo_for(n, B);
+        const dim3 go(1, B > 1 ? B / 32 : 1);
+        if (B > 1) {
+            k_qcqp_rows<true, TRIAL><<<gr.grid, gr.block, 0, stream>>>(qcqp, io);
+            if (!TRIAL) k_qcqp_grad<true><<<gc.grid, gc.block, 0, stream>>>(qcqp, io);
+            k_qcqp_obj<true, TRIAL><<<go, kThreads, 0, stream>>>(qcqp, io);
+        } else {
+            k_qcqp_rows<false, TRIAL><<<gr.grid, gr.block, 0, stream>>>(qcqp, io);
+            if (!TRIAL) k_qcqp_grad<false><<<gc.grid, gc.block, 0, stream>>>(qcqp, io);
+            k_qcqp_obj<false, TRIAL><<<go, kWarps, 0, stream>>>(qcqp, io);
+        }
+        own_launches += TRIAL ? 2 : 3;
+        ASM_CK(cudaGetLastError());
         return ASM_OK;
     }
 
@@ -1490,6 +1636,7 @@ int asm_slp_attach_acopf(asm_slp *hh, const asm_acopf_desc *d) {
     h.ac_coef_scen.release();   // back to the shared coefficients
     h.acopf = a;
     h.has_acopf = true;
+    h.has_qcqp = false;   // one evaluator per handle
     return ASM_OK;
 }
 
@@ -1546,10 +1693,7 @@ int asm_slp_eval_acopf(asm_slp *hh, const double *x, const double *delta, int32_
     SLP_GUARD();
     if (!h.has_acopf) return fail(ASM_E_STATE, "asm_slp_attach_acopf first");
     if (!x || !delta) return fail(ASM_E_INVALID, "null argument");
-    ASM_TRY(h.put(x, h.n, h.Buser, h.xk.p));
-    double *ps = (double *)h.pin_small.p;
-    for (int s = 0; s < B; ++s) ps[s] = delta[s < h.Buser ? s : 0];
-    ASM_CK(cudaMemcpyAsync(h.delta.p, ps, B * sizeof(double), cudaMemcpyHostToDevice, stream));
+    ASM_TRY(h.eval_inputs(x, delta));
     ASM_TRY(h.df.zero(stream));
     AcopfIo io;
     io.xk = h.xk.p; io.p = nullptr; io.alpha = nullptr;
@@ -1590,11 +1734,7 @@ int asm_slp_acopf_trial(asm_slp *hh, const double *alpha, const double *nu, cons
     if (!h.has_acopf) return fail(ASM_E_STATE, "asm_slp_attach_acopf first");
     if (!alpha || !nu || !out || (feasibility && !base)) return fail(ASM_E_INVALID, "null argument");
     if (h.phase < 0 || !h.solved) return fail(ASM_E_STATE, "no solved sub-LP yet");
-    ASM_TRY(h.extract_device());
-    ASM_TRY(h.put(nu, h.m, h.Buser, h.tmp_m2.p));
-    double *ps = (double *)h.pin_small.p + (size_t)B * R_COUNT;
-    for (int s = 0; s < B; ++s) ps[s] = alpha[s < h.Buser ? s : 0];
-    ASM_CK(cudaMemcpyAsync(h.d_alpha.p, ps, sizeof(double) * B, cudaMemcpyHostToDevice, stream));
+    ASM_TRY(h.trial_inputs(alpha, nu));
     AcopfIo io;
     io.xk = h.xk.p; io.p = h.p.p; io.alpha = h.d_alpha.p;
     io.f = h.ac_ftrial.p; io.df = nullptr; io.E = h.tmp_m.p; io.dE = nullptr; io.B = B;
@@ -1608,20 +1748,230 @@ int asm_slp_acopf_trial(asm_slp *hh, const double *alpha, const double *nu, cons
     }
     k_acopf_misc<true><<<(B + 127) / 128, 128, 0, stream>>>(h.acopf, io, h.n);
     own_launches += 3;
-    SlpView sv = h.view();
-    const Geo g = geo_for(h.m, B);
-    SLP_KB(k_merit, g, sv, (const double *)h.tmp_m.p, h.tmp_m2.p, h.pslack.p, (const double *)h.d_alpha.p, (int)feasibility,
-           h.partials.p);
-    std::vector<double> r;
-    ASM_TRY(h.finish_reduce(g.grid.x, 0u, r));
-    std::vector<double> ft(B, 0.0);
-    ASM_CK(cudaMemcpyAsync(ft.data(), h.ac_ftrial.p, sizeof(double) * B, cudaMemcpyDeviceToHost, stream));
-    ASM_CK(cudaStreamSynchronize(stream));
-    for (int s = 0; s < h.Buser; ++s) {
-        const double b0 = feasibility ? base[s] + alpha[s] * r[s * R_COUNT + R_B] : ft[s];
-        out[s] = b0 + r[s * R_COUNT + R_A];
+    return h.trial_merit(alpha, base, feasibility, h.ac_ftrial.p, out);
+}
+
+// ---- device-side QCQP evaluator -------------------------------------------------------------------------------
+int asm_slp_attach_qcqp(asm_slp *hh, const asm_qcqp_desc *d) {
+    SLP_GUARD();
+    (void)B;
+    if (!d) return fail(ASM_E_INVALID, "null QCQP description");
+    const int n = h.n, m = h.m;
+    const int64_t nnz = h.pat.nnz_coo;
+    if (d->n != n || d->m != m || d->nnz_coo != nnz)
+        return fail(ASM_E_INVALID, "QCQP description does not match the handle's n, m, nnz");
+    if (d->n_obj_aff < 0 || d->n_obj_quad < 0 || d->n_aff < 0 || d->n_quad < 0)
+        return fail(ASM_E_INVALID, "negative term count in the QCQP description");
+    if ((d->n_obj_aff && (!d->obj_aff_col || !d->obj_aff_coef)) ||
+        (d->n_obj_quad && (!d->obj_quad_i || !d->obj_quad_j || !d->obj_quad_coef)) ||
+        (d->n_aff && (!d->aff_row || !d->aff_col || !d->aff_coef || !d->aff_pos)) ||
+        (d->n_quad && (!d->quad_row || !d->quad_i || !d->quad_j || !d->quad_coef || !d->quad_pos)))
+        return fail(ASM_E_INVALID, "null array in the QCQP description");
+    if (d->n_aff + d->n_quad > 0x7fffffffLL || (int64_t)d->n_obj_aff + d->n_obj_quad > 0x7fffffffLL)
+        return fail(ASM_E_INVALID, "too many terms in the QCQP description");
+    if (!std::isfinite(d->c0)) return fail(ASM_E_INVALID, "non-finite objective constant");
+    auto col_ok = [&](int32_t j) { return j >= 0 && j < n; };
+    auto row_ok = [&](int32_t r) { return r >= 0 && r < m; };
+    for (int k = 0; k < d->n_obj_aff; ++k) {
+        if (!col_ok(d->obj_aff_col[k])) return fail(ASM_E_INVALID, "objective affine column out of range");
+        if (!std::isfinite(d->obj_aff_coef[k])) return fail(ASM_E_INVALID, "non-finite objective coefficient");
     }
+    for (int k = 0; k < d->n_obj_quad; ++k) {
+        if (!col_ok(d->obj_quad_i[k]) || !col_ok(d->obj_quad_j[k]))
+            return fail(ASM_E_INVALID, "objective quadratic variable out of range");
+        if (!std::isfinite(d->obj_quad_coef[k])) return fail(ASM_E_INVALID, "non-finite objective coefficient");
+    }
+    // (row, col) of every j_str entry, from the handle's analysis of the original pattern
+    std::vector<int> coo_row(nnz), coo_col(nnz);
+    {
+        std::vector<int> slot_row(h.pat.nnz);
+        for (int r = 0; r < m; ++r)
+            for (int64_t k = h.pat.row_ptr[r]; k < h.pat.row_ptr[r + 1]; ++k) slot_row[k] = r;
+        for (int64_t k = 0; k < nnz; ++k) {
+            coo_row[k] = slot_row[h.pat.slot_of_coo[k]];
+            coo_col[k] = h.pat.col_idx[h.pat.slot_of_coo[k]];
+        }
+    }
+    auto pos_ok = [&](int64_t p, int r, int v) { return p >= 0 && p < nnz && coo_row[p] == r && coo_col[p] == v; };
+    for (int64_t k = 0; k < d->n_aff; ++k) {
+        if (!row_ok(d->aff_row[k]) || !col_ok(d->aff_col[k])) return fail(ASM_E_INVALID, "affine term index out of range");
+        if (!std::isfinite(d->aff_coef[k])) return fail(ASM_E_INVALID, "non-finite affine coefficient");
+        if (!pos_ok(d->aff_pos[k], d->aff_row[k], d->aff_col[k]))
+            return fail(ASM_E_INVALID, "affine term position out of range or not at its (row, col) in j_str");
+    }
+    for (int64_t k = 0; k < d->n_quad; ++k) {
+        const int r = d->quad_row[k], i = d->quad_i[k], j = d->quad_j[k];
+        if (!row_ok(r) || !col_ok(i) || !col_ok(j)) return fail(ASM_E_INVALID, "quadratic term index out of range");
+        if (!std::isfinite(d->quad_coef[k])) return fail(ASM_E_INVALID, "non-finite quadratic coefficient");
+        const int64_t p0 = d->quad_pos[2 * k], p1 = d->quad_pos[2 * k + 1];
+        if (i == j) {
+            if (p1 != -1) return fail(ASM_E_INVALID, "quad_pos[2k + 1] must be -1 for a term with i == j");
+            if (!pos_ok(p0, r, i))
+                return fail(ASM_E_INVALID, "quadratic term position out of range or not at its (row, col) in j_str");
+        } else if (!pos_ok(p0, r, i) || !pos_ok(p1, r, j)) {
+            return fail(ASM_E_INVALID, "quadratic term position out of range or not at its (row, col) in j_str");
+        }
+    }
+    // rows: terms (affine, then quadratic, each in term order)
+    std::vector<int64_t> row_ptr(m + 1, 0), pos_ptr(m + 1, 0), con_ptr(nnz + 1, 0), col_ptr(n + 1, 0);
+    for (int64_t k = 0; k < d->n_aff; ++k) row_ptr[d->aff_row[k] + 1]++;
+    for (int64_t k = 0; k < d->n_quad; ++k) row_ptr[d->quad_row[k] + 1]++;
+    for (int r = 0; r < m; ++r) row_ptr[r + 1] += row_ptr[r];
+    const int64_t nt = row_ptr[m];
+    std::vector<int> term_i(nt), term_j(nt);
+    std::vector<double> term_c(nt);
+    {
+        std::vector<int64_t> fill(row_ptr.begin(), row_ptr.end() - 1);
+        for (int64_t k = 0; k < d->n_aff; ++k) {
+            const int64_t t = fill[d->aff_row[k]]++;
+            term_i[t] = d->aff_col[k]; term_j[t] = -1; term_c[t] = d->aff_coef[k];
+        }
+        for (int64_t k = 0; k < d->n_quad; ++k) {
+            const int64_t t = fill[d->quad_row[k]]++;
+            term_i[t] = d->quad_i[k]; term_j[t] = d->quad_j[k]; term_c[t] = d->quad_coef[k];
+        }
+    }
+    // rows: their j_str positions in ascending order; each position's derivative contributions
+    std::vector<int> pos(nnz), slot(nnz);   // slot: index of j_str entry p in `pos`
+    for (int64_t p = 0; p < nnz; ++p) pos_ptr[coo_row[p] + 1]++;
+    for (int r = 0; r < m; ++r) pos_ptr[r + 1] += pos_ptr[r];
+    {
+        std::vector<int64_t> fill(pos_ptr.begin(), pos_ptr.end() - 1);
+        for (int64_t p = 0; p < nnz; ++p) {
+            const int64_t t = fill[coo_row[p]]++;
+            pos[t] = (int)p;
+            slot[p] = (int)t;
+        }
+    }
+    for (int64_t k = 0; k < d->n_aff; ++k) con_ptr[slot[d->aff_pos[k]] + 1]++;
+    for (int64_t k = 0; k < d->n_quad; ++k) {
+        con_ptr[slot[d->quad_pos[2 * k]] + 1]++;
+        if (d->quad_i[k] != d->quad_j[k]) con_ptr[slot[d->quad_pos[2 * k + 1]] + 1]++;
+    }
+    for (int64_t t = 0; t < nnz; ++t) con_ptr[t + 1] += con_ptr[t];
+    const int64_t nc = con_ptr[nnz];
+    std::vector<int> con_i(nc);
+    std::vector<double> con_c(nc);
+    {
+        std::vector<int64_t> fill(con_ptr.begin(), con_ptr.end() - 1);
+        auto push = [&](int64_t p, double c, int v) {
+            const int64_t e = fill[slot[p]]++;
+            con_c[e] = c;
+            con_i[e] = v;
+        };
+        for (int64_t k = 0; k < d->n_aff; ++k) push(d->aff_pos[k], d->aff_coef[k], -1);
+        for (int64_t k = 0; k < d->n_quad; ++k) {
+            const int i = d->quad_i[k], j = d->quad_j[k];
+            const double q = d->quad_coef[k];
+            if (i == j) {
+                push(d->quad_pos[2 * k], 2.0 * q, i);
+            } else {
+                push(d->quad_pos[2 * k], q, j);
+                push(d->quad_pos[2 * k + 1], q, i);
+            }
+        }
+    }
+    // columns: the objective's gradient contributions (affine, then quadratic, term order)
+    for (int k = 0; k < d->n_obj_aff; ++k) col_ptr[d->obj_aff_col[k] + 1]++;
+    for (int k = 0; k < d->n_obj_quad; ++k) {
+        col_ptr[d->obj_quad_i[k] + 1]++;
+        if (d->obj_quad_i[k] != d->obj_quad_j[k]) col_ptr[d->obj_quad_j[k] + 1]++;
+    }
+    for (int j = 0; j < n; ++j) col_ptr[j + 1] += col_ptr[j];
+    const int64_t ng = col_ptr[n];
+    std::vector<int> grad_i(ng);
+    std::vector<double> grad_c(ng);
+    {
+        std::vector<int64_t> fill(col_ptr.begin(), col_ptr.end() - 1);
+        auto push = [&](int col, double c, int v) {
+            const int64_t e = fill[col]++;
+            grad_c[e] = c;
+            grad_i[e] = v;
+        };
+        for (int k = 0; k < d->n_obj_aff; ++k) push(d->obj_aff_col[k], d->obj_aff_coef[k], -1);
+        for (int k = 0; k < d->n_obj_quad; ++k) {
+            const int i = d->obj_quad_i[k], j = d->obj_quad_j[k];
+            const double q = d->obj_quad_coef[k];
+            if (i == j) {
+                push(i, 2.0 * q, i);
+            } else {
+                push(i, q, j);
+                push(j, q, i);
+            }
+        }
+    }
+    // objective terms (affine, then quadratic)
+    const int no = d->n_obj_aff + d->n_obj_quad;
+    std::vector<int> obj_i(no), obj_j(no);
+    std::vector<double> obj_c(no);
+    for (int k = 0; k < d->n_obj_aff; ++k) {
+        obj_i[k] = d->obj_aff_col[k]; obj_j[k] = -1; obj_c[k] = d->obj_aff_coef[k];
+    }
+    for (int k = 0; k < d->n_obj_quad; ++k) {
+        const int e = d->n_obj_aff + k;
+        obj_i[e] = d->obj_quad_i[k]; obj_j[e] = d->obj_quad_j[k]; obj_c[e] = d->obj_quad_coef[k];
+    }
+    auto up = [&](auto &b, const auto &v) -> int {
+        ASM_TRY(b.alloc(std::max<size_t>(v.size(), 1)));
+        if (!v.empty()) ASM_CK(cudaMemcpy(b.p, v.data(), v.size() * sizeof(v[0]), cudaMemcpyHostToDevice));
+        return ASM_OK;
+    };
+    ASM_TRY(up(h.qc_row_ptr, row_ptr));
+    ASM_TRY(up(h.qc_pos_ptr, pos_ptr));
+    ASM_TRY(up(h.qc_con_ptr, con_ptr));
+    ASM_TRY(up(h.qc_col_ptr, col_ptr));
+    ASM_TRY(up(h.qc_term_i, term_i));
+    ASM_TRY(up(h.qc_term_j, term_j));
+    ASM_TRY(up(h.qc_term_c, term_c));
+    ASM_TRY(up(h.qc_pos, pos));
+    ASM_TRY(up(h.qc_con_i, con_i));
+    ASM_TRY(up(h.qc_con_c, con_c));
+    ASM_TRY(up(h.qc_grad_i, grad_i));
+    ASM_TRY(up(h.qc_grad_c, grad_c));
+    ASM_TRY(up(h.qc_obj_i, obj_i));
+    ASM_TRY(up(h.qc_obj_j, obj_j));
+    ASM_TRY(up(h.qc_obj_c, obj_c));
+    ASM_TRY(h.qc_ftrial.alloc(h.B));
+    QcqpDev q;
+    q.n = n; q.m = m; q.n_obj = no; q.c0 = d->c0;
+    q.row_ptr = h.qc_row_ptr.p; q.pos_ptr = h.qc_pos_ptr.p; q.con_ptr = h.qc_con_ptr.p; q.col_ptr = h.qc_col_ptr.p;
+    q.term_i = h.qc_term_i.p; q.term_j = h.qc_term_j.p; q.term_c = h.qc_term_c.p; q.pos = h.qc_pos.p;
+    q.con_i = h.qc_con_i.p; q.con_c = h.qc_con_c.p; q.grad_i = h.qc_grad_i.p; q.grad_c = h.qc_grad_c.p;
+    q.obj_i = h.qc_obj_i.p; q.obj_j = h.qc_obj_j.p; q.obj_c = h.qc_obj_c.p;
+    h.qcqp = q;
+    h.has_qcqp = true;
+    h.has_acopf = false;   // one evaluator per handle
     return ASM_OK;
+}
+
+// eval_functions! of the attached QCQP on the device, then the device part of asm_slp_update
+int asm_slp_eval_qcqp(asm_slp *hh, const double *x, const double *delta, int32_t feasibility) {
+    SLP_GUARD();
+    (void)B;
+    if (!h.has_qcqp) return fail(ASM_E_STATE, "asm_slp_attach_qcqp first");
+    if (!x || !delta) return fail(ASM_E_INVALID, "null argument");
+    ASM_TRY(h.eval_inputs(x, delta));
+    AcopfIo io;
+    io.xk = h.xk.p; io.p = nullptr; io.alpha = nullptr;
+    io.f = h.fval.p; io.df = h.df.p; io.E = h.E.p; io.dE = h.dE.p; io.B = h.B;
+    ASM_TRY(h.qcqp_launch<false>(io));
+    return h.update_device(feasibility);
+}
+
+// compute_phi(x + alpha p) with f and g of the attached QCQP evaluated on the device at the trial point
+int asm_slp_qcqp_trial(asm_slp *hh, const double *alpha, const double *nu, const double *base, int32_t feasibility,
+                       double *out) {
+    SLP_GUARD();
+    (void)B;
+    if (!h.has_qcqp) return fail(ASM_E_STATE, "asm_slp_attach_qcqp first");
+    if (!alpha || !nu || !out || (feasibility && !base)) return fail(ASM_E_INVALID, "null argument");
+    if (h.phase < 0 || !h.solved) return fail(ASM_E_STATE, "no solved sub-LP yet");
+    ASM_TRY(h.trial_inputs(alpha, nu));
+    AcopfIo io;
+    io.xk = h.xk.p; io.p = h.p.p; io.alpha = h.d_alpha.p;
+    io.f = h.qc_ftrial.p; io.df = nullptr; io.E = h.tmp_m.p; io.dE = nullptr; io.B = h.B;
+    ASM_TRY(h.qcqp_launch<true>(io));
+    return h.trial_merit(alpha, base, feasibility, h.qc_ftrial.p, out);
 }
 
 int64_t asm_slp_launch_count(asm_slp *h) {

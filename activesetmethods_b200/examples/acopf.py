@@ -737,3 +737,134 @@ class AcopfModel:
         v[k:k + 20 * nl] = J.ravel(); k += 20 * nl
         assert k == self.nnz
         return values
+
+
+class AcrModel:
+    """The same OPF in rectangular voltage coordinates ("ACR", PowerModels' ``ACRPowerModel``, one of the formulations
+    the reference's example builds: ``examples/acopf/opf.jl:18-21``).  Every row and the objective are affine or
+    quadratic in (vr, vi), so the model is a ``qcqp.QcqpModel`` and runs on the device-side QCQP evaluator with no
+    formulation-specific kernel.  Built by ``AcrModel(net)``, which returns the ``QcqpModel``.
+
+    Variables: vr[nb], vi[nb] (bounds +-vmax) in the slots of AcopfModel's va, vm; then pg, qg, p, q, p_dc, q_dc with
+    AcopfModel's order, bounds and costs.
+    Row order (attributes ``r_*`` of the returned model):
+      angmax[nl]   (vi_f vr_t - vr_f vi_t) - tan(angmax) (vr_f vr_t + vi_f vi_t) <= 0
+      angmin[nl]   (vi_f vr_t - vr_f vi_t) - tan(angmin) (vr_f vr_t + vi_f vi_t) >= 0
+                   (exact: the reader keeps every limit inside (-90, 90) degrees)
+      ref          vi_ref = 0
+      dc[nd]       (1 - loss1) p_dc_f + p_dc_t = loss0
+      vm[nb]       vmin^2 <= vr^2 + vi^2 <= vmax^2
+      thermal[2nl] p^2 + q^2 <= rate^2 per branch, from then to
+      balance[2nb] P, Q per bus: AcopfModel's affine terms, shunt gs (vr^2 + vi^2), -bs (vr^2 + vi^2)
+      ohm[4nl]     p_fr, q_fr, p_to, q_to per branch: the arc flow minus AcopfModel's expression with the same 12
+                   coefficients, vm_f vm_t cos(va_f - va_t) -> vr_f vr_t + vi_f vi_t and
+                   vm_f vm_t sin(va_f - va_t) -> vi_f vr_t - vr_f vi_t.
+    Start: vr at the midpoint of [vmin, vmax] and vi = 0 (AcopfModel's start as a physical point; the midpoint of the
+    +-vmax box would be the all-zero voltage, where every Ohm row's Jacobian vanishes); the rest as AcopfModel.
+    Out-of-service generators enter through the bounds; an out-of-service branch raises ValueError (its zero
+    coefficients would change the term lists, which the device evaluator shares over a batch)."""
+
+    def __new__(cls, net: Network):
+        from .qcqp import QcqpModel
+        if np.any(net.br_status == 0):
+            raise ValueError("AcrModel: out-of-service branches are not supported (the term lists are shared by a batch)")
+        P = AcopfModel(net)
+        nb, ng, nl, nd = P.nb, P.ng, P.nl, P.nd
+        cf = P._cf
+        o_vr, o_vi = 0, nb
+        f, t = np.asarray(net.f_bus, dtype=np.int64), np.asarray(net.t_bus, dtype=np.int64)
+        br = np.arange(nl)
+        x_L, x_U = P.x_L.copy(), P.x_U.copy()
+        x_L[:2 * nb] = -np.tile(net.vmax, 2)
+        x_U[:2 * nb] = np.tile(net.vmax, 2)
+        x0 = P.x0.copy()
+        x0[:nb] = 0.5 * (net.vmin + net.vmax)
+        x0[nb:2 * nb] = 0.0
+        inf = np.inf
+        r = 0
+        r_angmax = r; r += nl
+        r_angmin = r; r += nl
+        r_ref = r; r += 1
+        r_dc = r; r += nd
+        r_vm = r; r += nb
+        r_thermal = r; r += 2 * nl
+        r_bal = r; r += 2 * nb
+        r_ohm = r; r += 4 * nl
+        m = r
+        gl, gu = np.full(m, -inf), np.full(m, inf)
+        gu[r_angmax:r_angmax + nl] = 0.0
+        gl[r_angmin:r_angmin + nl] = 0.0
+        gl[r_ref] = gu[r_ref] = 0.0
+        if nd:
+            gl[r_dc:r_dc + nd] = gu[r_dc:r_dc + nd] = net.dc_loss0
+        gl[r_vm:r_vm + nb] = net.vmin ** 2
+        gu[r_vm:r_vm + nb] = net.vmax ** 2
+        gu[r_thermal:r_thermal + 2 * nl] = np.repeat(net.rate_a ** 2, 2)
+        gl[r_bal:r_bal + 2 * nb:2] = gu[r_bal:r_bal + 2 * nb:2] = -net.pd
+        gl[r_bal + 1:r_bal + 2 * nb:2] = gu[r_bal + 1:r_bal + 2 * nb:2] = -net.qd
+        gl[r_ohm:] = gu[r_ohm:] = 0.0
+
+        A = ([], [], [])          # affine terms: row, col, coef
+        Q = ([], [], [], [])      # quadratic terms: row, i, j, coef
+
+        def aff(row, col, coef):
+            for lst, v in zip(A, (row, col, coef)):
+                lst.append(np.asarray(v).reshape(-1))
+
+        def quad(row, i, j, coef):
+            for lst, v in zip(Q, (row, i, j, coef)):
+                lst.append(np.asarray(v).reshape(-1))
+
+        vrf, vrt, vif, vit = o_vr + f, o_vr + t, o_vi + f, o_vi + t
+
+        def cols(*a):             # per-branch columns interleaved term by term
+            return np.stack(a, 1)
+        for r0, lim in ((r_angmax, net.angmax), (r_angmin, net.angmin)):
+            ta = np.tan(lim)
+            rows = np.repeat(r0 + br, 4)
+            quad(rows, cols(vif, vrf, vrf, vif), cols(vrt, vit, vrt, vit),
+                 cols(np.ones(nl), -np.ones(nl), -ta, -ta))
+        aff([r_ref], [o_vi + net.ref_bus], [1.0])
+        if nd:
+            d = np.arange(nd)
+            aff(np.repeat(r_dc + d, 2), cols(P.o_pdc + d, P.o_pdc + nd + d), cols(1.0 - net.dc_loss1, np.ones(nd)))
+        bus = np.arange(nb)
+        quad(np.repeat(r_vm + bus, 2), cols(o_vr + bus, o_vi + bus), cols(o_vr + bus, o_vi + bus), np.ones(2 * nb))
+        rt = np.stack([r_thermal + 2 * br, r_thermal + 2 * br + 1], 1)
+        quad(np.repeat(rt.reshape(-1), 2),
+             cols(P.o_p + br, P.o_q + br, P.o_p + nl + br, P.o_q + nl + br).reshape(nl, 2, 2),
+             cols(P.o_p + br, P.o_q + br, P.o_p + nl + br, P.o_q + nl + br).reshape(nl, 2, 2), np.ones(4 * nl))
+        # balances: AcopfModel's affine terms in its order, the shunt on vr^2 + vi^2
+        lin = ~np.isnan(P._bal_coef)
+        aff(P._bal_rows[lin] - P.r_bal + r_bal, P._bal_cols[lin], P._bal_coef[lin])
+        for i in range(nb):
+            for is_q, sh in ((0, net.gs[i]), (1, -net.bs[i])):
+                if sh != 0.0:
+                    quad([r_bal + 2 * i + is_q] * 2, [o_vr + i, o_vi + i], [o_vr + i, o_vi + i], [sh, sh])
+        # Ohm rows: arc - (a v_own^2 + b (vr_f vr_t + vi_f vi_t) + sg c (vi_f vr_t - vr_f vi_t))
+        for k, (key, arc, own_f, sg) in enumerate((("pf", P.o_p + br, True, 1.0), ("qf", P.o_q + br, True, 1.0),
+                                                   ("pt", P.o_p + nl + br, False, -1.0),
+                                                   ("qt", P.o_q + nl + br, False, -1.0))):
+            a, b, c = cf["a_" + key], cf["b_" + key], cf["c_" + key]
+            row = r_ohm + 4 * br + k
+            own_r, own_i = (vrf, vif) if own_f else (vrt, vit)
+            aff(row, arc, np.ones(nl))
+            quad(np.repeat(row, 6), cols(own_r, own_i, vrf, vif, vif, vrf), cols(own_r, own_i, vrt, vit, vrt, vit),
+                 cols(-a, -a, -b, -b, -sg * c, sg * c))
+        cat = lambda lst, dt: np.concatenate(lst).astype(dt) if lst else np.zeros(0, dt)   # noqa: E731
+        a_row, a_col, a_coef = cat(A[0], np.int64), cat(A[1], np.int64), cat(A[2], float)
+        q_row, q_i, q_j, q_coef = cat(Q[0], np.int64), cat(Q[1], np.int64), cat(Q[2], np.int64), cat(Q[3], float)
+        # terms of one row must stay together in the order listed above: sort rows stably
+        oa, oq = np.argsort(a_row, kind="stable"), np.argsort(q_row, kind="stable")
+        pg = P.o_pg + np.arange(ng)
+        mdl = QcqpModel(P.n, x_L, x_U, gl, gu, x0, obj_const=float(np.sum(net.cost0)),
+                        obj_aff=(pg, net.cost1), obj_quad=(pg, pg, net.cost2),
+                        aff=(a_row[oa], a_col[oa], a_coef[oa]), quad=(q_row[oq], q_i[oq], q_j[oq], q_coef[oq]))
+        mdl.net = net
+        mdl.nb, mdl.ng, mdl.nl, mdl.nd = nb, ng, nl, nd
+        mdl.o_vr, mdl.o_vi = o_vr, o_vi
+        for name in ("o_pg", "o_qg", "o_p", "o_q", "o_pdc", "o_qdc"):
+            setattr(mdl, name, getattr(P, name))
+        mdl.r_angmax, mdl.r_angmin, mdl.r_ref, mdl.r_dc, mdl.r_vm = r_angmax, r_angmin, r_ref, r_dc, r_vm
+        mdl.r_thermal, mdl.r_bal, mdl.r_ohm = r_thermal, r_bal, r_ohm
+        return mdl

@@ -15,8 +15,9 @@ here                              reference (relative to /root/reference)
 
 Each algorithm has one driver, the lock-step batch (``SlpLSBatch``, ``SlpTRBatch``); a single solve is its
 one-scenario case.  The NLP callbacks (``eval_f``, ``eval_grad_f``, ``eval_g``, ``eval_jac_g``) stay on the host
-exactly like the JuMP ``NLPEvaluator`` of the reference (``src/MOI_wrapper.jl:1047-1069``), unless the device-side
-ACOPF evaluator replaces them.  Per round the driver hands ``x, f, df, E, dE`` to ``SubLp.update`` (one H2D
+exactly like the JuMP ``NLPEvaluator`` of the reference (``src/MOI_wrapper.jl:1047-1069``), unless a device-side
+evaluator replaces them: the ACOPF one for ``examples.acopf.AcopfModel``, the QCQP one for
+``examples.qcqp.QcqpModel`` (affine and quadratic models such as ``examples.acopf.AcrModel``).  Per round the driver hands ``x, f, df, E, dE`` to ``SubLp.update`` (one H2D
 hand-over, assembly + bounds on the device), solves the sub-LPs with ``solve_extract`` and asks the device for the
 merit / KKT reductions.
 """
@@ -70,9 +71,9 @@ class Parameters:
     # engine options forwarded to asm_lp_params (not in the reference)
     lp_options: dict = field(default_factory=dict)
     device: int = 0
-    # either algorithm on an examples.acopf.AcopfModel with the B200 engine: evaluate f, g, the Jacobian and the
-    # merit at trial points (backtracking / step quality) with the device-side ACOPF evaluator instead of the host
-    # callbacks (SURVEY.md 8(f)-1)
+    # either algorithm on an examples.acopf.AcopfModel or an examples.qcqp.QcqpModel with the B200 engine: evaluate
+    # f, g, the Jacobian and the merit at trial points (backtracking / step quality) with the device-side ACOPF or QCQP
+    # evaluator instead of the host callbacks (SURVEY.md 8(f)-1)
     device_evaluator: bool = False
 
 
@@ -151,6 +152,7 @@ class _SlpBatch:
     # (degenerate) restoration LPs is returned and the runs measured so far ended further from the optimum.
     # ``lp_options={"warm_start": ...}`` overrides either.
     warm_start = 1
+    _dev = "acopf"          # the device-side evaluator attached by _instantiate: "acopf" or "qcqp"
     # per-problem results of a queued run (see ``lanes``)
     _outputs = ("ret", "iter", "x", "obj_val", "prim_infeas", "dual_infeas", "compl", "lp_solves")
 
@@ -210,10 +212,24 @@ class _SlpBatch:
         prs = self.problems
         arr = lambda name: np.array([np.asarray(getattr(pr, name), dtype=float) for pr in prs])  # noqa: E731
         if o.external_optimizer == "B200LP":
+            qcqp = self.device_evaluator and self._is_qcqp(prs[0])
+            if qcqp:
+                # the QCQP evaluator holds one set of term lists for the batch: scenarios differ in bounds and start
+                # only.  A queued run checks every problem up front, so that a mismatch fails before any solve.
+                models = self._acopf(self._queue or prs)
+                for k, pr in enumerate(models[1:], 1):
+                    if not self._is_qcqp(pr):
+                        raise ValueError(f"device_evaluator: scenario {k} is not a QcqpModel like scenario 0")
+                    diff = models[0].same_terms(pr)
+                    if diff is not None:
+                        raise ValueError(f"device_evaluator: scenario {k} differs from scenario 0 in its terms ({diff})")
             opt = SubLp(self.n, self.m, prs[0].j_str, arr("x_L"), arr("x_U"), arr("g_L"), arr("g_U"), batch=self.B,
                         device=o.device, **{"warm_start": self.warm_start, **o.lp_options})
             opt._squeeze = False
-            if self.device_evaluator:
+            if qcqp:
+                opt.attach_qcqp(models[0])
+                self._dev = "qcqp"
+            elif self.device_evaluator:
                 # the device evaluator holds one topology, shunts, costs, dc-line losses and reference bus for the
                 # batch; branch data (impedances, taps, shifts, outages) may differ per scenario, and loads, generator
                 # outages and relaxed angle rows only enter the bounds.  A Model hands over the problem it was built from.
@@ -227,11 +243,28 @@ class _SlpBatch:
                     if pr.net.ref_bus != n0.ref_bus:
                         raise ValueError(f"device_evaluator: scenario {k} has another reference bus")
                 opt.attach_acopf(acopf)
+                self._dev = "acopf"
             return opt
         if self.device_evaluator:
             raise ValueError("device_evaluator needs the B200 engine")
         return o.external_optimizer(self.n, self.m, prs[0].j_str, arr("x_L"), arr("x_U"), arr("g_L"), arr("g_U"),
                                     batch=self.B)
+
+    @staticmethod
+    def _is_qcqp(pr):
+        return hasattr(pr.source if isinstance(pr, Model) else pr, "qcqp_desc")
+
+    def _dev_eval(self, delta, feasibility):
+        """The device-side evaluation at ``self.x`` + the device part of ``update``, with the attached evaluator."""
+        if self._dev == "qcqp":
+            self.optimizer.eval_qcqp(self.x, delta, feasibility)
+        else:
+            self.optimizer.eval_acopf(self.x, delta, feasibility)
+
+    def _dev_trial(self, alpha, fr):
+        """compute_phi(x + alpha p) for the batch with the attached device-side evaluator."""
+        trial = self.optimizer.qcqp_trial if self._dev == "qcqp" else self.optimizer.acopf_trial
+        return np.atleast_1d(trial(alpha, self.nu, self.prim_infeas if fr else None, fr))
 
     @staticmethod
     def _acopf(prs):
@@ -289,7 +322,7 @@ class _SlpBatch:
             self._reset_lane(s, pr)
         bounds = [np.array([np.asarray(getattr(pr, name), dtype=float) for pr in new])
                   for name in ("x_L", "x_U", "g_L", "g_U")]
-        if self.device_evaluator:
+        if self.device_evaluator and self._dev == "acopf":
             self.optimizer.load_lanes(load, *bounds, acopf=self._acopf(new))
         else:
             self.optimizer.load_lanes(load, *bounds)
@@ -310,7 +343,7 @@ class _SlpBatch:
         if hasattr(opt, "set_active"):
             opt.set_active(sel)
         if fr and self.device_evaluator:
-            opt.eval_acopf(self.x, delta, True)
+            self._dev_eval(delta, True)
         elif fr:                    # the normal-phase data push was done at the start of this round
             opt.update(self.x, self.f, self.df, self.E, self.dE, delta, True)
         idx = np.nonzero(sel)[0]
@@ -355,9 +388,10 @@ class SlpLSBatch(_SlpBatch):
     (``slp_line_search.jl:78-215``) — a scenario that terminates simply stops moving while the others go on.  A
     single solve (``SlpLS``) is the one-scenario batch.
 
-    ``device_evaluator=True`` (ACOPF scenarios of one network, B200 engine): the NLP callbacks are not called at all —
-    f, g and the Jacobian are evaluated by the device-side ACOPF evaluator (``SubLp.eval_acopf``) and every
-    backtracking trial is one ``SubLp.acopf_trial`` call for the whole batch."""
+    ``device_evaluator=True`` (ACOPF scenarios of one network, or QCQP scenarios that share their terms; B200
+    engine): the NLP callbacks are not called at all — f, g and the Jacobian are evaluated by the device-side evaluator
+    (``SubLp.eval_acopf`` / ``SubLp.eval_qcqp``) and every backtracking trial is one ``SubLp.acopf_trial`` /
+    ``SubLp.qcqp_trial`` call for the whole batch."""
 
     def __init__(self, problems, parameters: Parameters | None = None, device_evaluator: bool = False, lanes=None):
         super().__init__(problems, parameters, device_evaluator, lanes)
@@ -379,7 +413,7 @@ class SlpLSBatch(_SlpBatch):
             run = np.nonzero(self.running)[0]
             # KKT metrics with last round's multipliers on this round's Jacobian (App. C-7)
             if self.device_evaluator:
-                opt.eval_acopf(self.x, 1000.0, False)
+                self._dev_eval(1000.0, False)
                 self.f[:] = opt.get_eval_f()
             else:
                 for s in run:
@@ -475,7 +509,7 @@ class SlpLSBatch(_SlpBatch):
         while searching.any():
             act = np.nonzero(searching)[0]
             if self.device_evaluator:
-                phi = np.atleast_1d(self.optimizer.acopf_trial(self.alpha, self.nu, self.prim_infeas if fr else None, fr))
+                phi = self._dev_trial(self.alpha, fr)
             else:
                 for s in act:
                     pr = self.problems[s]
@@ -507,7 +541,8 @@ class SlpTRBatch(_SlpBatch):
     ``step_quality``.  All of a phase runs before the next phase's push, which overwrites the step and slacks on the
     device that the merit calls read.
 
-    ``device_evaluator=True``: as for ``SlpLSBatch``; ϕ(x + p) is one ``SubLp.acopf_trial`` call for the batch."""
+    ``device_evaluator=True``: as for ``SlpLSBatch``; ϕ(x + p) is one ``SubLp.acopf_trial`` / ``SubLp.qcqp_trial``
+    call for the batch."""
 
     warm_start = 0      # see _SlpBatch.warm_start
     _outputs = _SlpBatch._outputs + ("delta",)
@@ -531,7 +566,7 @@ class SlpTRBatch(_SlpBatch):
         while self.running.any():
             self.rounds += 1
             if self.device_evaluator:
-                opt.eval_acopf(self.x, self.delta, False)
+                self._dev_eval(self.delta, False)
                 self.f[:] = opt.get_eval_f()
             else:
                 for s in np.nonzero(self.running)[0]:
@@ -623,7 +658,7 @@ class SlpTRBatch(_SlpBatch):
         B = self.B
         base = self.prim_infeas if fr else self.f
         if self.device_evaluator:
-            phi1 = np.atleast_1d(opt.acopf_trial(np.ones(B), self.nu, self.prim_infeas if fr else None, fr))
+            phi1 = self._dev_trial(np.ones(B), fr)
         else:
             base1 = base.copy()
             Et = self.E.copy()

@@ -379,6 +379,38 @@ class SubLp:
             capi.dptr(None if base is None else self._scal(base)), 1 if feasibility else 0, capi.dptr(out)))
         return self._ret(out) if self._squeeze else out
 
+    # -- device-side evaluator for affine and quadratic models ---------------------------------------------------
+    def attach_qcqp(self, model):
+        """Hand the term lists of an ``examples.qcqp.QcqpModel`` (or anything with its ``qcqp_desc()``) to the device so
+        that ``eval_qcqp`` / ``qcqp_trial`` replace the host callbacks.  Every scenario of the batch shares the terms;
+        scenarios differ in bounds and start points only.  Detaches the ACOPF evaluator."""
+        arrs = model.qcqp_desc()
+        d = capi.QcqpDesc()
+        d.n, d.m, d.nnz_coo, d.c0 = int(arrs["n"]), int(arrs["m"]), int(arrs["nnz_coo"]), float(arrs["c0"])
+        d.n_obj_aff, d.n_obj_quad = len(arrs["obj_aff_col"]), len(arrs["obj_quad_i"])
+        d.n_aff, d.n_quad = len(arrs["aff_row"]), len(arrs["quad_row"])
+        ptr = {np.dtype(np.int32): capi.c_int32_p, np.dtype(np.int64): capi.c_int64_p,
+               np.dtype(np.float64): capi.c_double_p}
+        for k, a in arrs.items():
+            if isinstance(a, np.ndarray):
+                setattr(d, k, a.ctypes.data_as(ptr[a.dtype]) if len(a) else None)
+        capi.check(self._lib.asm_slp_attach_qcqp(self._h, C.byref(d)))
+        self._acopf_ref = None
+
+    def eval_qcqp(self, x, delta=1000.0, feasibility=False):
+        """``eval_functions!`` (slp.jl:186-191) of the attached QCQP on the device at ``x`` + the device part of
+        ``update``; ``get_eval`` reads the evaluation back."""
+        capi.check(self._lib.asm_slp_eval_qcqp(self._h, capi.dptr(self._vec(x, self.n)), capi.dptr(self._scal(delta)),
+                                               1 if feasibility else 0))
+
+    def qcqp_trial(self, alpha, nu, base=None, feasibility=False):
+        """``compute_phi(x + alpha p)`` (slp.jl:79-115) with f and g of the attached QCQP evaluated on the device."""
+        out = np.empty(self.batch)
+        capi.check(self._lib.asm_slp_qcqp_trial(
+            self._h, capi.dptr(self._scal(alpha)), capi.dptr(self._vec(nu, self.m)),
+            capi.dptr(None if base is None else self._scal(base)), 1 if feasibility else 0, capi.dptr(out)))
+        return self._ret(out) if self._squeeze else out
+
     # -- instrumentation ----------------------------------------------------------------------------------------
     def launch_count(self) -> int:
         return int(self._lib.asm_slp_launch_count(self._h))

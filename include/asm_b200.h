@@ -257,6 +257,48 @@ int asm_slp_get_eval(asm_slp *h, double *f, double *df, double *E, double *dE);
 int asm_slp_acopf_trial(asm_slp *h, const double *alpha, const double *nu, const double *base, int32_t feasibility,
                         double *out);
 
+/* ---- device-side evaluator for affine and quadratic models (QCQP) -------------------------------------------
+ * The same role as the ACOPF evaluator above for any model whose objective and rows are all affine or quadratic
+ * (the rows the reference's MOI wrapper evaluates inline, src/MOI_wrapper.jl:889-918): f, grad f, g and the Jacobian
+ * are sums over fixed term lists.  Conventions:
+ *   - 0-based indices; a quadratic term is q * x_i * x_j (no 1/2 convention; i == j allowed);
+ *   - row r is g_r(x) = sum of its affine terms, then of its quadratic terms, each in the given term order; the
+ *     objective is c0 + its affine terms + its quadratic terms in the same way;
+ *   - positions index j_str (0-based).  The derivative a of an affine term goes to aff_pos[k]; for a quadratic term
+ *     k with i != j, q x_j goes to quad_pos[2k] and q x_i to quad_pos[2k + 1]; with i == j, 2q x_i goes to
+ *     quad_pos[2k] and quad_pos[2k + 1] must be -1.  An entry several derivatives target gets their sum (affine
+ *     first, then quadratic, each in term order); an entry no term targets is written 0 at every evaluation;
+ *   - coefficients are shared by the whole batch: scenarios differ in bounds (and start points) only, so
+ *     asm_slp_set_active and asm_slp_load_lanes work unchanged.
+ * asm_slp_attach_qcqp returns ASM_E_INVALID (message in asm_last_error) for sizes that differ from the handle's, an
+ * index out of range, a non-finite coefficient, a position whose j_str (row, col) is not the (row, variable) of the
+ * derivative it receives, or a bad quad_pos for i == j.  A handle holds one evaluator at a time: attaching the QCQP
+ * evaluator detaches the ACOPF one and vice versa (the detached evaluator's calls then return ASM_E_STATE). */
+typedef struct asm_qcqp_desc {
+    int32_t n, m;
+    int64_t nnz_coo;                      /* must equal the handle's                                               */
+    double c0;                            /* objective constant                                                    */
+    int32_t n_obj_aff, n_obj_quad;
+    const int32_t *obj_aff_col;           /* [n_obj_aff]                                                           */
+    const double *obj_aff_coef;
+    const int32_t *obj_quad_i, *obj_quad_j; /* [n_obj_quad]: q * x_i * x_j                                         */
+    const double *obj_quad_coef;
+    int64_t n_aff, n_quad;
+    const int32_t *aff_row, *aff_col;     /* [n_aff]                                                               */
+    const double *aff_coef;
+    const int64_t *aff_pos;               /* [n_aff]: j_str entry of the derivative                                */
+    const int32_t *quad_row, *quad_i, *quad_j; /* [n_quad]                                                         */
+    const double *quad_coef;
+    const int64_t *quad_pos;              /* [2 n_quad]: j_str entry of d/dx_i, of d/dx_j (-1 when i == j)          */
+} asm_qcqp_desc;
+int asm_slp_attach_qcqp(asm_slp *h, const asm_qcqp_desc *d);
+/* as asm_slp_eval_acopf: the model's f, grad f, g, Jacobian at x[batch][n] on the device, then the device part of
+ * asm_slp_update; asm_slp_get_eval reads the evaluation back */
+int asm_slp_eval_qcqp(asm_slp *h, const double *x, const double *delta, int32_t feasibility);
+/* as asm_slp_acopf_trial: compute_phi(x + alpha p) with f and g of the model evaluated on the device */
+int asm_slp_qcqp_trial(asm_slp *h, const double *alpha, const double *nu, const double *base, int32_t feasibility,
+                       double *out);
+
 /* ---- instrumentation --------------------------------------------------------------------------------- */
 /* kernels launched by this handle's solver since creation (all of them this library's own) */
 int64_t asm_slp_launch_count(asm_slp *h);
